@@ -4,7 +4,7 @@ bench.py — policy-evaluation throughput (Bellman state-backups/s) on the
 reference's largest configuration: Double CartPole swing-up, 6-D, --bins 20
 (64 M states, 9 actions; BASELINE.json configs[4], SURVEY.md §8 K5).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
 
 A *step* is one sync interval of the reference's policy_evaluation loop
 (src/cuda_policy_iteration.py:300-336): 25 Jacobi sweeps over the whole grid
@@ -18,9 +18,10 @@ events on the engine's stream (max over ranks).  Rank 0 prints ONE JSON line.
   roofline     HBM roofline of the evaluation-sweep kernel (algorithmic bytes =
                compact row + V read + V write per backup; DESIGN.md §4)
   cpu_baseline the CPU restatement (oracle/pi_oracle.c, OpenMP) on a bounded slab
-  --impl reference   the reference's OWN kernels (oracle/_ref cubins compiled from
-               /root/reference by NVRTC) driven by the reference's host loop on one
+  --impl reference   the reference's OWN kernels (oracle/_ref cubins compiled by
+               oracle/build_ref.py with NVRTC) driven by the reference's host loop on one
                B200 — the reference has no CPU policy-iteration path (SURVEY §8c)
+  --dump-outputs DIR   after the timed steps, what the last one computed (see dump_outputs)
 """
 from __future__ import annotations
 
@@ -63,6 +64,23 @@ def v_checksum(t) -> int:
     import torch
 
     return int((t.contiguous().view(torch.int32).to(torch.int64) & 0xFFFFFFFF).sum().item())
+
+
+DUMP_SAMPLE = 1 << 22   # states of V written by --dump-outputs: 16 MB of values + 32 MB of indices
+
+
+def dump_outputs(out_dir: str, values: np.ndarray, residual: float) -> None:
+    """What a caller of the timed path receives after its last step: V in reference order (every state up to
+    DUMP_SAMPLE states, else a fixed sample drawn with seed 0, sorted) with the flat state index of each value, and
+    the residual max|V_new - V_old| of the step's last sweep.  The inputs are the same in every run with the same
+    arguments, so two builds can be compared file by file."""
+    d = Path(out_dir)
+    d.mkdir(parents=True, exist_ok=True)
+    n = values.size
+    idx = np.arange(n) if n <= DUMP_SAMPLE else np.sort(np.random.default_rng(0).choice(n, DUMP_SAMPLE, replace=False))
+    np.save(d / "value_function.npy", values[idx].astype(np.float32))
+    np.save(d / "value_function_index.npy", idx.astype(np.float64))
+    np.save(d / "residual.npy", np.array([residual], dtype=np.float32))
 
 
 def _quiet_logs() -> None:
@@ -187,7 +205,7 @@ def run_ours(args) -> dict:
     t0 = time.perf_counter()
     dev_ms = 0.0
     for _ in range(args.steps):
-        _, ms = eng.sweeps(SWEEPS_PER_STEP)
+        residual, ms = eng.sweeps(SWEEPS_PER_STEP)
         dev_ms += ms
     barrier()
     wall_s = time.perf_counter() - t0
@@ -207,6 +225,11 @@ def run_ours(args) -> dict:
     csum = int(csum.item())
     n_sweeps_at_checksum = 2 * SWEEPS_PER_STEP + (max(args.warmup, 3) + args.steps) * SWEEPS_PER_STEP
     kinfo = eng.eval_kernel_info()   # which sweep kernel the engine runs for THIS policy (scalar gather / x-line)
+    if args.dump_outputs:
+        values, _ = eng.download()   # every rank: the whole V is gathered when sharded
+        if rank == 0:
+            dump_outputs(args.dump_outputs, values, residual)
+        del values
 
     # ---- end-to-end arm: host buffers in, host buffers out ---------------------
     n_local = hi - lo
@@ -509,7 +532,7 @@ def run_reference(args) -> dict | None:
                      "converged": bool(ref12.converged)}
         kind = {"value": value, "unit": UNIT, "cores": 0, "kind": "reference",
                 "sample": "the reference's own eval kernel + max|x-y| reduction (oracle/_ref cubin, NVRTC-compiled "
-                          "from /root/reference) on one B200, full grid; the reference has no CPU path"}
+                          "from the original project's sources) on one B200, full grid; the reference has no CPU path"}
     else:
         cb = cpu_baseline(args.bins, budget_s=30.0)
         value = cb["value"]
@@ -545,7 +568,12 @@ def main() -> int:
     ap.add_argument("--no-converge", action="store_true")
     ap.add_argument("--no-stable", action="store_true", help="skip the K5 run to a stable policy")
     ap.add_argument("--no-extras", action="store_true", help="skip the per-configuration stage table (K1-K4) and the --bins 12 runs")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write V and the residual after the last timed step to DIR/*.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs is only available with --impl ours")
     _quiet_logs()
     # stdout carries exactly ONE JSON line: while the benchmark runs, file descriptor 1 points at stderr, so
     # anything a library prints there (torch's "NCCL version ..." banner under torchrun) cannot precede it

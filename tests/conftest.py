@@ -45,11 +45,54 @@ def golden_dir() -> Path:
     return ROOT / "tests" / "golden"
 
 
-@pytest.fixture(scope="session")
-def ref_runner():
-    """The reference's own kernels (oracle/_ref cubins).  Parity tests need them:
-    a missing oracle is a failure, not a skip."""
-    from oracle import ref_runner as rr
+REFERENCE_GOLDEN = ROOT / "tests" / "golden" / "reference_parity.json"
 
-    assert rr.available(), "oracle/_ref/ is missing: run `python oracle/build_ref.py` where /root/reference exists"
-    return rr
+
+class ReferenceGolden:
+    """What the reference's own kernels computed for one test case, stored in tests/golden/reference_parity.json
+    (its "source" entry says how it was produced): per array its dtype, shape, the SHA-256 of its bytes and the values
+    at a few flat positions (`at`, `sample`) for the failure message; scalars as they are.  `check` is bit-exact, as
+    a comparison with the reference's arrays themselves would be.
+
+    The file is data, not output of this suite: nothing here writes it.  A new or changed case must be recorded from
+    the reference's kernels (oracle/_ref, oracle/ref_runner.py), never from the engine under test."""
+
+    def __init__(self, case: str, stored: dict | None) -> None:
+        self.case, self.stored = case, stored
+
+    def _expected(self, label: str):
+        assert self.stored is not None and label in self.stored, f"no stored reference result for {self.case} / {label}"
+        return self.stored[label]
+
+    def check(self, label: str, a) -> None:
+        import hashlib
+
+        import numpy as np
+
+        exp = self._expected(label)
+        a = np.ascontiguousarray(a)
+        assert [str(a.dtype), list(a.shape)] == [exp["dtype"], exp["shape"]], (label, a.dtype, a.shape, exp)
+        sample = a.reshape(-1)[exp["at"]]
+        ref_sample = np.asarray(exp["sample"], dtype=a.dtype)
+        assert sample.tobytes() == ref_sample.tobytes(), f"{label}: values {sample} at {exp['at']} != reference {ref_sample}"
+        assert hashlib.sha256(a.tobytes()).hexdigest() == exp["sha256"], f"{label}: bits differ from the reference's"
+
+    def check_value(self, label: str, v) -> None:
+        assert v == self._expected(label), (label, v, self._expected(label))
+
+    def check_run(self, eng, prefix: str = "") -> None:
+        """A finished run(): PI iterations, evaluation sweeps, policy and value-function bits."""
+        self.check_value(prefix + "pi_iterations", eng.pi_iterations)
+        self.check_value(prefix + "total_sweeps", eng.total_eval_sweeps)
+        self.check(prefix + "policy", eng.policy)
+        self.check(prefix + "value_function", eng.value_function)
+
+
+@pytest.fixture()
+def reference(request):
+    """The reference's results for this test case (see ReferenceGolden)."""
+    import json
+
+    case = f"{Path(str(request.node.fspath)).name}::{request.node.nodeid.split('::', 1)[1]}"
+    assert REFERENCE_GOLDEN.exists(), f"{REFERENCE_GOLDEN} is missing"
+    return ReferenceGolden(case, json.loads(REFERENCE_GOLDEN.read_text())["cases"].get(case))

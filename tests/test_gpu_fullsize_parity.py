@@ -1,4 +1,4 @@
-"""Bit-for-bit parity with the reference's own kernels (oracle/_ref cubins) AT BASELINE.json's sizes:
+"""Bit-for-bit parity with what the reference's own kernels compute (tests/golden/reference_parity.json) AT BASELINE.json's sizes:
 K2 (Continuous Mountain Car --bins 400, also with a 201-action grid) and K3 (CartPole --bins 30) complete run()s;
 K4 (Double Pendulum swing-up --bins 50) and K5 (Double CartPole swing-up --bins 20, 64 M states) one improvement
 pass and one evaluation sweep under the mixed policy of PI iteration 1 with the DEFAULT-selected sweep kernel
@@ -13,45 +13,32 @@ from dynamicprogramming_b200 import envs
 pytestmark = pytest.mark.gpu
 
 
-def bits(a):
-    return np.ascontiguousarray(a).view(np.uint32)
-
-
 @pytest.mark.parametrize("env,bins,n_actions", [("continuous_mountain_car", 400, None), ("continuous_mountain_car", 400, 201),
                                                 ("cartpole", 30, None)])
-def test_complete_run_at_baseline_size_matches_the_reference(env, bins, n_actions, ref_runner):
+def test_complete_run_at_baseline_size_matches_the_reference(env, bins, n_actions, reference):
     spec = envs.REGISTRY[env]
     actions = None
     if n_actions is not None:
         actions = np.linspace(float(spec.actions.min()), float(spec.actions.max()), n_actions).astype(np.float32)
     eng = spec.make(bins=bins, actions=actions)
-    ref = ref_runner.from_engine_env(env, bins=bins, actions=actions)
     eng.run()
-    ref.run()
-    assert eng.pi_iterations == ref.pi_iterations and eng.total_eval_sweeps == ref.total_sweeps
-    np.testing.assert_array_equal(eng.policy, ref.policy)
-    np.testing.assert_array_equal(bits(eng.value_function), bits(ref.value_function))
+    reference.check_run(eng)
 
 
-def _mixed_policy_pair(env, bins, ref_runner, sweeps=50):
-    """Engine and reference object after `sweeps` sweeps of the initial policy and one improvement pass."""
+def _mixed_policy(env, bins, sweeps=50):
+    """Engine after `sweeps` sweeps of the initial policy and one improvement pass."""
     eng = envs.make(env, bins=bins)
     eng.build_table()
     eng.sweeps(sweeps)
     eng.policy_improvement()
-    ref = ref_runner.from_engine_env(env, bins=bins)
-    for _ in range(sweeps):
-        ref.eval_launch()
-        ref.d_value_function, ref.d_new_value_function = ref.d_new_value_function, ref.d_value_function
-    ref.improve_launch()
-    return eng, ref
+    return eng
 
 
 @pytest.mark.parametrize("env,bins,kernels", [("double_pendulum_swingup", 50, "default"), ("double_pendulum_swingup", 50, "gather"),
                                               ("double_pendulum_swingup", 50, "aot"), ("double_cartpole_swingup", 20, "default"),
                                               ("double_cartpole_swingup", 20, "gather"), ("double_cartpole_swingup", 20, "plane"),
                                               ("double_cartpole_swingup", 20, "plane_one"), ("double_cartpole_swingup", 20, "aot")])
-def test_improvement_and_sweep_at_baseline_size_match_the_reference(env, bins, kernels, ref_runner, monkeypatch):
+def test_improvement_and_sweep_at_baseline_size_match_the_reference(env, bins, kernels, reference, monkeypatch):
     """K4 / K5: the improvement pass (policy bits) and one sweep under the resulting mixed policy (V bits), with the
     kernel the engine selects by default — the one bench.py times — and with each sweep family pinned."""
     if kernels == "gather":
@@ -65,7 +52,7 @@ def test_improvement_and_sweep_at_baseline_size_match_the_reference(env, bins, k
         monkeypatch.setenv("DPB200_PLANE", "off")
         monkeypatch.setenv("DPB200_XLINE", "off")
         monkeypatch.setenv("DPB200_PAIR", "off")
-    eng, ref = _mixed_policy_pair(env, bins, ref_runner)
+    eng = _mixed_policy(env, bins)
     info = eng.eval_kernel_info()
     if kernels == "default" and env == "double_cartpole_swingup":
         assert "ps_sweep" in info["kernel"] or "gp_sweep" in info["kernel"], info     # the JIT sweeps bench.py times
@@ -74,49 +61,43 @@ def test_improvement_and_sweep_at_baseline_size_match_the_reference(env, bins, k
     if kernels == "aot":
         assert "eval_sweep_kernel" in info["kernel"], info
     _, pol = eng.download()
-    np.testing.assert_array_equal(pol, ref.d_policy.cpu().numpy())
+    reference.check("improved policy", pol)
     v0, _ = eng.download()
-    np.testing.assert_array_equal(bits(v0), bits(ref.d_value_function.cpu().numpy()))
+    reference.check("value_function before the sweep", v0)
     delta, _ = eng.sweeps(1)
     v1, _ = eng.download()
-    vr = ref.sweep_once()
-    np.testing.assert_array_equal(bits(v1), bits(vr))
-    assert delta == float(np.max(np.abs(vr - v0)))
+    reference.check("value_function after the sweep", v1)
+    assert delta == float(np.max(np.abs(v1 - v0)))
     eng.close()
 
 
-def test_k5_transition_rows_match_the_reference_slab_wise(ref_runner):
+def test_k5_transition_rows_match_the_reference_slab_wise(reference):
     """64 M x 9 rows cannot be expanded at once (2 x 16 GB per action): compare slabs spread over the grid."""
     env, bins = "double_cartpole_swingup", 20
     eng = envs.make(env, bins=bins)
     eng.build_table()
-    ref = ref_runner.from_engine_env(env, bins=bins)
     n = 160_000
     compared = 0
     for a, s0 in ((0, 0), (1, 3_200_000), (4, 13_333_337), (8, 31_999_999), (2, 50_000_000), (6, 60_500_000),
                   (7, 64_000_000 - n)):
         idx, w, r, t = eng.expand_rows(a, s0, n)
-        ridx, rw, rr, rt, _ = ref.probe_rows(a, s0, n)
-        own = t != 2                      # states in the terminal mask have no row (new_V := V, :1053); the probe ignores the mask
-        live = own & (rt == 0)
-        np.testing.assert_array_equal((t == 1)[own], (rt != 0)[own])
-        np.testing.assert_array_equal(idx[live], ridx[live])
-        np.testing.assert_array_equal(bits(w[live]), bits(rw[live]))
-        np.testing.assert_array_equal(bits(r[own]), bits(rr[own]))
+        own = t != 2                      # states in the terminal mask have no row (new_V := V, :1053)
+        live = own & (t != 1)
+        slab = f"action {a} states {s0}+{n}"
+        reference.check(f"{slab} terminated", (t == 1)[own])
+        reference.check(f"{slab} idx", idx[live])
+        reference.check(f"{slab} w", w[live])
+        reference.check(f"{slab} reward", r[own])
         compared += int(own.sum())
     assert compared >= 4 * n          # the first and the last slab (and the end of the sixth) lie in the terminal mask |x| > 2.4
     eng.close()
 
 
 @pytest.mark.timeout(900)
-def test_k5_bins12_runs_to_the_same_stable_policy_as_the_reference(ref_runner):
+def test_k5_bins12_runs_to_the_same_stable_policy_as_the_reference(reference):
     """The autoresearch trial workload (--bins 12, 2 985 984 states) with the reference's own config, to the end."""
     env, bins = "double_cartpole_swingup", 12
     eng = envs.make(env, bins=bins)
-    ref = ref_runner.from_engine_env(env, bins=bins)
     eng.run()
-    ref.run()
-    assert eng.pi_iterations == ref.pi_iterations and eng.total_eval_sweeps == ref.total_sweeps
-    assert eng.converged and ref.converged
-    np.testing.assert_array_equal(eng.policy, ref.policy)
-    np.testing.assert_array_equal(bits(eng.value_function), bits(ref.value_function))
+    assert eng.converged
+    reference.check_run(eng)

@@ -1,10 +1,9 @@
-"""Parity tests proper: the CUDA engine (through the C ABI) against the
-reference's own kernels (oracle/_ref cubins) on the same GPU — bit-exact for
+"""Parity tests proper: the CUDA engine (through the C ABI) against what the
+reference's own kernels compute (tests/golden/reference_parity.json) — bit-exact for
 transition indices, weights, rewards, value functions, policies, sweep counts —
 and against the reference's golden files and the CPU oracle at tolerance."""
 import numpy as np
 import pytest
-import torch
 
 from dynamicprogramming_b200 import envs
 
@@ -14,34 +13,27 @@ SMALL = {"pendulum": 41, "mountain_car": 50, "continuous_mountain_car": 50, "car
          "double_pendulum_swingup": 9, "overhead_crane": 9, "double_cartpole": 5, "double_cartpole_swingup": 6}
 
 
-def bits(a):
-    return np.ascontiguousarray(a).view(np.uint32)
-
-
 @pytest.mark.parametrize("env", sorted(SMALL))
-def test_transition_rows_are_bit_exact(env, ref_runner):
+def test_transition_rows_are_bit_exact(env, reference):
     """Indices, weights, reward and `terminated` of every (state, action) row
     equal what the reference's step_dynamics + get_barycentric_Nd produce."""
     eng = envs.make(env, bins=SMALL[env])
-    ref = ref_runner.from_engine_env(env, bins=SMALL[env])
     term = eng._terminal_mask_host.astype(bool)
     live = ~term
     for a in range(eng.n_actions):
         idx, w, r, t = eng.expand_rows(a)
-        ridx, rw, rr, rt, _ = ref.probe_rows(a)
         assert (t[term] == 2).all()                                  # absorbing rows are flagged
-        np.testing.assert_array_equal((t[live] == 1), (rt[live] == 1))
-        ok = live & (rt == 0)
-        np.testing.assert_array_equal(idx[ok], ridx[ok])
-        np.testing.assert_array_equal(bits(w[ok]), bits(rw[ok]))
-        np.testing.assert_array_equal(bits(r[live]), bits(rr[live]))
+        reference.check(f"action {a} terminated", t[live] == 1)
+        ok = live & (t != 1)
+        reference.check(f"action {a} idx", idx[ok])
+        reference.check(f"action {a} w", w[ok])
+        reference.check(f"action {a} reward", r[live])
     eng.close()
 
 
 @pytest.mark.parametrize("env", sorted(SMALL))
-def test_single_sweep_and_improvement_are_bit_exact(env, ref_runner):
+def test_single_sweep_and_improvement_are_bit_exact(env, reference):
     eng = envs.make(env, bins=SMALL[env])
-    ref = ref_runner.from_engine_env(env, bins=SMALL[env])
     N, A = eng.n_states, eng.n_actions
     rng = np.random.default_rng(3)
     V0 = (rng.standard_normal(N) * 10).astype(np.float32)
@@ -51,32 +43,23 @@ def test_single_sweep_and_improvement_are_bit_exact(env, ref_runner):
         eng.upload_values(V0)
         delta, _ = eng.sweeps(1)
         v_mine, _ = eng.download()
-        ref.d_policy.copy_(torch.from_numpy(pol).cuda())
-        ref.d_value_function.copy_(torch.from_numpy(V0).cuda())
-        v_ref = ref.sweep_once()
-        np.testing.assert_array_equal(bits(v_mine), bits(v_ref))
-        assert np.float32(delta) == np.abs(v_ref - V0).max()          # fused residual == max|new_V - V|
+        reference.check(f"sweep under policy {a}", v_mine)
+        assert np.float32(delta) == np.abs(v_mine - V0).max()         # fused residual == max|new_V - V|
     # mixed policy
     pol = rng.integers(0, A, N).astype(np.int32)
     eng.upload_policy(pol)
     eng.upload_values(V0)
     eng.sweeps(1)
     v_mine, _ = eng.download()
-    ref.d_policy.copy_(torch.from_numpy(pol).cuda())
-    ref.d_value_function.copy_(torch.from_numpy(V0).cuda())
-    np.testing.assert_array_equal(bits(v_mine), bits(ref.sweep_once()))
+    reference.check("sweep under the mixed policy", v_mine)
     # improvement from the same V
     eng.upload_policy(np.zeros(N, dtype=np.int32))
     eng.upload_values(V0)
     stable = eng.policy_improvement()
     _, p_mine = eng.download()
-    ref.d_policy.zero_()
-    ref.d_value_function.copy_(torch.from_numpy(V0).cuda())
-    ref.improve_launch()
-    p_ref = ref.d_policy.cpu().numpy()
-    np.testing.assert_array_equal(p_mine, p_ref)
-    assert stable == bool((p_ref == 0).all())
-    assert eng.last_changed == int((p_ref != 0).sum())
+    reference.check("improved policy", p_mine)
+    assert stable == bool((p_mine == 0).all())
+    assert eng.last_changed == int((p_mine != 0).sum())
     eng.close()
 
 
@@ -86,7 +69,7 @@ RUNS = [("mountain_car", 200, None), ("continuous_mountain_car", 200, None), ("p
 
 
 @pytest.mark.parametrize("env,bins,max_pi", RUNS)
-def test_full_policy_iteration_is_bit_identical_to_the_reference(env, bins, max_pi, ref_runner):
+def test_full_policy_iteration_is_bit_identical_to_the_reference(env, bins, max_pi, reference):
     """run(): same number of PI iterations and sweeps, identical policy, identical V bits."""
     spec = envs.REGISTRY[env]
     cfg = spec.config()
@@ -94,12 +77,7 @@ def test_full_policy_iteration_is_bit_identical_to_the_reference(env, bins, max_
         cfg.max_pi_iter = max_pi
     eng = spec.make(bins=bins, config=cfg)
     eng.run()
-    ref = ref_runner.from_engine_env(env, bins=bins, config=cfg)
-    ref.run()
-    assert eng.pi_iterations == ref.pi_iterations
-    assert eng.total_eval_sweeps == ref.total_sweeps
-    np.testing.assert_array_equal(eng.policy, ref.policy)
-    np.testing.assert_array_equal(bits(eng.value_function), bits(ref.value_function))
+    reference.check_run(eng)
     assert eng.value_function.dtype == np.float32 and eng.policy.dtype == np.int32
     assert not hasattr(eng, "d_value_function")                       # VRAM released like the reference
 

@@ -75,7 +75,7 @@ def test_plane_sweep_without_plane_structure_falls_back_correctly(env, bins, lay
 
 
 @pytest.mark.parametrize("env,bins", [("double_cartpole_swingup", 8), ("cartpole", 12), ("double_cartpole", 10)])
-def test_full_policy_iteration_with_the_plane_sweep_matches_the_reference(env, bins, monkeypatch, ref_runner):
+def test_full_policy_iteration_with_the_plane_sweep_matches_the_reference(env, bins, monkeypatch, reference):
     """Complete run() with the plane-staged sweep forced on: PI iterations, sweep counts, policy and V bits
     equal the reference's own kernels."""
     monkeypatch.setenv("DPB200_PLANE", "force")
@@ -86,12 +86,8 @@ def test_full_policy_iteration_with_the_plane_sweep_matches_the_reference(env, b
     eng.build_table()
     info = eng.eval_kernel_info()
     assert info["plane"] and "ps_sweep" in info["kernel"], info
-    ref = ref_runner.from_engine_env(env, bins=bins, config=c)
     eng.run()
-    ref.run()
-    assert eng.total_eval_sweeps == ref.total_sweeps and eng.pi_iterations == ref.pi_iterations
-    np.testing.assert_array_equal(eng.policy, ref.policy)
-    np.testing.assert_array_equal(bits(eng.value_function), bits(ref.value_function))
+    reference.check_run(eng)
 
 
 def test_plane_autotune_never_changes_results(monkeypatch):

@@ -50,7 +50,7 @@ def test_xline_sweep_is_bit_identical_to_the_scalar_sweep(env, bins, cfg, monkey
 @pytest.mark.parametrize("env,bins,cfg", [("double_cartpole_swingup", 8, "force:4,0,4,8,1,1:1,1,2,4,4"),
                                           ("cartpole", 12, "force:2,0,4,8,2,1:1,3,6"),
                                           ("double_pendulum_swingup", 12, "force:4,0,4,8,1,1:2,4,6")])
-def test_full_policy_iteration_with_the_xline_sweep_matches_the_reference(env, bins, cfg, monkeypatch, ref_runner):
+def test_full_policy_iteration_with_the_xline_sweep_matches_the_reference(env, bins, cfg, monkeypatch, reference):
     """Complete run() with the x-line sweep forced on: PI iterations, sweep counts, policy and V bits
     equal the reference's own kernels."""
     monkeypatch.setenv("DPB200_FAST_DIM", "0")
@@ -62,12 +62,8 @@ def test_full_policy_iteration_with_the_xline_sweep_matches_the_reference(env, b
     eng.build_table()
     info = eng.eval_kernel_info()
     assert info["xline"], info
-    ref = ref_runner.from_engine_env(env, bins=bins, config=c)
     eng.run()
-    ref.run()
-    assert eng.total_eval_sweeps == ref.total_sweeps and eng.pi_iterations == ref.pi_iterations
-    np.testing.assert_array_equal(eng.policy, ref.policy)
-    np.testing.assert_array_equal(bits(eng.value_function), bits(ref.value_function))
+    reference.check_run(eng)
 
 
 def test_autotune_reports_its_choice_and_never_changes_results(monkeypatch):
@@ -160,7 +156,7 @@ def test_scalar_sweep_tuning_variants_are_bit_identical(variant, monkeypatch):
         np.testing.assert_array_equal(res[0], res[1])
 
 
-def test_full_policy_iteration_with_the_single_state_jit_sweep_matches_the_reference(monkeypatch, ref_runner):
+def test_full_policy_iteration_with_the_single_state_jit_sweep_matches_the_reference(monkeypatch, reference):
     monkeypatch.setenv("DPB200_XLINE", "off")
     monkeypatch.setenv("DPB200_PAIR", "force:128,8,2,8,1")
     for env, bins in (("double_cartpole_swingup", 6), ("cartpole", 12)):
@@ -170,15 +166,11 @@ def test_full_policy_iteration_with_the_single_state_jit_sweep_matches_the_refer
         eng = spec.make(bins=bins, config=c)
         eng.build_table()
         assert "one state/thread" in eng.eval_kernel_info()["kernel"]
-        ref = ref_runner.from_engine_env(env, bins=bins, config=c)
         eng.run()
-        ref.run()
-        assert eng.total_eval_sweeps == ref.total_sweeps and eng.pi_iterations == ref.pi_iterations
-        np.testing.assert_array_equal(eng.policy, ref.policy)
-        np.testing.assert_array_equal(bits(eng.value_function), bits(ref.value_function))
+        reference.check_run(eng, f"{env} ")
 
 
-def test_full_policy_iteration_with_the_packed_pair_sweep_matches_the_reference(monkeypatch, ref_runner):
+def test_full_policy_iteration_with_the_packed_pair_sweep_matches_the_reference(monkeypatch, reference):
     monkeypatch.setenv("DPB200_XLINE", "off")
     monkeypatch.setenv("DPB200_PAIR", "force")
     spec = envs.REGISTRY["double_cartpole"]
@@ -187,9 +179,5 @@ def test_full_policy_iteration_with_the_packed_pair_sweep_matches_the_reference(
     eng = spec.make(bins=7, config=c)
     eng.build_table()
     assert "gp_sweep" in eng.eval_kernel_info()["kernel"]
-    ref = ref_runner.from_engine_env("double_cartpole", bins=7, config=c)
     eng.run()
-    ref.run()
-    assert eng.total_eval_sweeps == ref.total_sweeps and eng.pi_iterations == ref.pi_iterations
-    np.testing.assert_array_equal(eng.policy, ref.policy)
-    np.testing.assert_array_equal(bits(eng.value_function), bits(ref.value_function))
+    reference.check_run(eng)
