@@ -111,6 +111,13 @@ SIGNATURES = {
     "pi_lookup_create": (C.c_int, [C.POINTER(PiGrid), C.c_void_p, C.c_void_p, C.c_int32, C.c_int32, C.POINTER(C.c_void_p)]),
     "pi_lookup_query": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int64, C.c_void_p]),
     "pi_lookup_destroy": (None, [C.c_void_p]),
+    "pi_rollout_create": (C.c_int, [C.POINTER(PiGrid), C.c_void_p, C.c_void_p, C.c_int32, C.c_char_p, C.c_int32,
+                                    C.POINTER(C.c_void_p)]),
+    "pi_rollout_run": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int64, C.c_int32, C.c_double, C.c_void_p, C.c_void_p,
+                                 C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]),
+    "pi_rollout_step": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int64, C.c_void_p, C.c_void_p, C.c_void_p]),
+    "pi_rollout_destroy": (None, [C.c_void_p]),
+    "pi_rollout_compile_check": (C.c_int, [C.c_char_p, C.c_int32, C.POINTER(C.c_int64)]),
     "pi_eval_kernel_info": (C.c_int, [C.c_void_p, C.c_char_p, C.c_int32, C.POINTER(C.c_double), C.POINTER(C.c_double)]),
     "pi_xline_compile_check": (C.c_int, [C.c_int32, C.c_int32, C.c_char_p, C.POINTER(C.c_int64)]),
     "pi_debug_pair": (C.c_int, [C.c_void_p, C.c_int32, C.c_int32, C.c_int32, C.c_int32, C.c_int32, C.c_int32, C.POINTER(C.c_float), C.POINTER(C.c_float),

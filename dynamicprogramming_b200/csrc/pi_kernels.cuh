@@ -1325,58 +1325,42 @@ __global__ void count_mismatch_kernel(const unsigned* a, const unsigned* b, long
 }
 
 // ---------------------------------------------------------------------------
-// Batched policy lookup with get_optimal_action semantics (utils/barycentric.py:11-108):
-// action(p) = sum_c lambda_c(p) * action_space[policy[idx_c(p)]].  Arithmetic follows the
-// reference as numba types it (pinned by tests/golden/barycentric_inference_golden.npz and
-// oracle_inference_weights): step = f32((f64)f32(hi-lo) / (shape-1)); cell and the clamp in
-// float32; t = f32((f64 p - (f64 lo + idx*f64 step)) / f64 step); weights are float64 products
-// in dimension order rounded to float32; corner c follows corner_bits = product([0,1]^D)
-// (dimension 0 is the MOST significant bit).  The final dot product is accumulated in float32 in
-// ascending corner order without contraction (numpy uses a BLAS dot whose order is unspecified).
-// `stride[d]` addresses `policy` (reference strides for a reference-order table, the engine's
-// internal strides for its device-resident policy).  One thread per query point.
+// Batched policy lookup with get_optimal_action semantics (utils/barycentric.py:11-108).  The per-point
+// arithmetic (LookupGrid, lookup_point) lives in lookup_src.cuh, shared with the NVRTC-compiled rollout
+// kernels (rollout_src.cuh).  One thread per query point.
 // ---------------------------------------------------------------------------
-struct LookupGrid {
-    int n_dims;
-    int shape[kMaxDims];
-    int stride[kMaxDims];
-    float lo[kMaxDims];
-    float hi[kMaxDims];
-};
+#include "lookup_src.cuh"
 
 __global__ void __launch_bounds__(kBlock) lookup_actions_kernel(LookupGrid g, const float* __restrict__ points, long long n,
                                                                 const int* __restrict__ policy,
                                                                 const float* __restrict__ actions, float* __restrict__ out) {
     const long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
     if (i >= n) return;
-    const int D = g.n_dims;
-    int base[kMaxDims];
-    double t[kMaxDims];
-    for (int d = 0; d < D; ++d) {
-        const float step = (float)__ddiv_rn((double)__fsub_rn(g.hi[d], g.lo[d]), (double)(g.shape[d] - 1));
-        const float x = points[i * D + d];
-        float q = x < g.hi[d] ? x : g.hi[d];      // max(lo, min(p, hi)) as numba evaluates it
-        q = q > g.lo[d] ? q : g.lo[d];
-        const float cell = __fdiv_rn(__fsub_rn(q, g.lo[d]), step);
-        int id = (int)cell;
-        if (id >= g.shape[d] - 1) id = g.shape[d] - 2;
-        base[d] = id;
-        const double num = __dsub_rn((double)q, __dadd_rn((double)g.lo[d], __dmul_rn((double)id, (double)step)));
-        t[d] = (double)(float)__ddiv_rn(num, (double)step);
-    }
-    float acc = 0.0f;
-    const int C = 1 << D;
-    for (int c = 0; c < C; ++c) {
-        double w = 1.0;
-        long long flat = 0;
-        for (int d = 0; d < D; ++d) {
-            const int bit = (c >> (D - 1 - d)) & 1;   // corner_bits[c][d]
-            w = __dmul_rn(w, bit ? t[d] : __dsub_rn(1.0, t[d]));
-            flat += (long long)(base[d] + bit) * g.stride[d];
+    out[i] = lookup_point(g, g.n_dims, points + i * g.n_dims, policy, actions);
+}
+
+// Recorded rollout trajectories (rollout_src.cuh) are staged step-major: a rows x n matrix, row r = t * per + k,
+// column = episode.  This writes its transpose out[e][r] (the episode-major host layout) through 32 x 32 shared-memory
+// tiles, both sides coalesced, and puts NaN where step t = r / per lies beyond the episode (r >= (length[e] + extra) * per).
+// Block 32 x 8; grid.y strides over the rows.
+__global__ void __launch_bounds__(256) rollout_unstage_kernel(const float* __restrict__ in, float* __restrict__ out,
+                                                              long long rows, long long n, int per, int extra,
+                                                              const int* __restrict__ length) {
+    __shared__ float tile[32][33];
+    const long long e0 = (long long)blockIdx.x * 32;
+    for (long long r0 = (long long)blockIdx.y * 32; r0 < rows; r0 += (long long)gridDim.y * 32) {
+        for (int j = threadIdx.y; j < 32; j += blockDim.y) {
+            const long long r = r0 + j, e = e0 + threadIdx.x;
+            if (r < rows && e < n) tile[j][threadIdx.x] = in[r * n + e];
         }
-        acc = __fadd_rn(acc, __fmul_rn((float)w, actions[policy[flat]]));
+        __syncthreads();
+        for (int j = threadIdx.y; j < 32; j += blockDim.y) {
+            const long long e = e0 + j, r = r0 + threadIdx.x;
+            if (r < rows && e < n)
+                out[e * rows + r] = r < ((long long)length[e] + extra) * per ? tile[threadIdx.x][j] : __int_as_float(0x7fc00000);
+        }
+        __syncthreads();
     }
-    out[i] = acc;
 }
 
 }  // namespace pi

@@ -568,6 +568,43 @@ class _CudaPolicyIterationBase(abc.ABC):
             self._lookup = look
         return look[1](pts)
 
+    def _rollout_handle(self, need_current_policy: bool = True):
+        """The cached PolicyRollout of this object (see rollout()); rebuilt when the policy object or the dynamics text
+        changes.  A live engine's policy is taken through download(); an unchanged download reuses the handle.  A single
+        step does not use the policy (need_current_policy=False): any handle built from the same text serves it."""
+        from .utils import PolicyRollout
+        src = self._dynamics_cuda_src()
+        cached = getattr(self, "_rollout", None)
+        live = bool(getattr(self, "_engine", None))
+        if cached is not None and cached[1] == src and not need_current_policy:
+            return cached[2]
+        policy = self.download()[1] if live else self.policy
+        if cached is not None and cached[1] == src and (cached[0] is policy or (live and np.array_equal(cached[0], policy))):
+            return cached[2]
+        if cached is not None:
+            cached[2].close()
+            self._rollout = None
+        h = PolicyRollout(policy, self.action_space, self.bounds_low, self.bounds_high, self.grid_shape, src,
+                          device=int(getattr(self, "_device", os.environ.get("LOCAL_RANK", 0))))
+        self._rollout = (policy, src, h)
+        return h
+
+    def rollout(self, initial_states: np.ndarray, n_steps: int, gamma: float | None = None, record: bool = False):
+        """Closed-loop episodes of the current policy under this plugin's own `step_dynamics` (what the reference's
+        evaluate() does with get_optimal_action + an environment step, batched on the device: utils.PolicyRollout).
+        `initial_states` (n, D); each episode runs `n_steps` steps or until step_dynamics sets *terminated.  Works
+        after run() and after load() (host `policy`) and on a live engine (its current policy, through download()).
+        `gamma=None` is the engine's gamma as float32 (`self.config.gamma`); an instance made by load() carries the
+        default CudaPIConfig(), so pass its gamma explicitly there.  Returns a utils.RolloutResult."""
+        if gamma is None:
+            gamma = float(np.float32(self.config.gamma))
+        return self._rollout_handle().run(initial_states, n_steps, gamma, record=record)
+
+    def simulate_step(self, states: np.ndarray, actions: np.ndarray):
+        """One step of this plugin's `step_dynamics` per (states[i], actions[i]) on the device ->
+        (next_states (n, D) float32, rewards (n,) float32, terminated (n,) bool)."""
+        return self._rollout_handle(need_current_policy=False).step(states, actions)
+
     def eval_kernel_info(self) -> dict:
         """Which evaluation-sweep kernel the build-time autotune selected (include/dpb200.h:
         pi_eval_kernel_info): the scalar gather sweep or the JIT-compiled x-line sweep."""

@@ -14,6 +14,12 @@ rows 5-7; those packages are not in this image): `--render`, `--record`, `--rand
 are accepted and reported as skipped.  Instead the runner prints a summary of the solution and, as
 a smoke check of the inference path, queries `--episodes` random states through the batched
 `get_optimal_action` (include/dpb200.h: pi_lookup_*).
+
+With `--rollout` it also runs what evaluate() runs — the policy in closed loop — on the device:
+`--episodes` episodes of up to `--steps` steps from the same seeded uniform start states, simulated
+with the plugin's own float32 `step_dynamics` (the model the DP solved, not gymnasium;
+include/dpb200.h: pi_rollout_*), discounted with the runner's gamma, and prints one summary line:
+mean return, mean discounted return, mean length, fraction of episodes that terminated.
 """
 from __future__ import annotations
 
@@ -47,8 +53,11 @@ def build_parser(runner: str) -> argparse.ArgumentParser:
     p.add_argument("--random", type=int, nargs="?", const=5, default=None, metavar="N",
                    help="(skipped: random-policy gymnasium episodes)")
     p.add_argument("--record", type=Path, default=None, metavar="PATH", help="(skipped: video recording)")
-    p.add_argument("--episodes", type=int, default=5, help="Number of states queried through get_optimal_action")
-    p.add_argument("--steps", type=int, default=1000, help="Accepted for compatibility")
+    p.add_argument("--episodes", type=int, default=5,
+                   help="Number of states queried through get_optimal_action (and of episodes with --rollout)")
+    p.add_argument("--steps", type=int, default=1000, help="Steps per episode with --rollout (else accepted for compatibility)")
+    p.add_argument("--rollout", action="store_true",
+                   help="Also run --episodes closed-loop episodes of --steps steps on the GPU with the plugin's dynamics")
     p.add_argument("--bins", type=int, default=spec.default_bins, help=f"Bins per dimension (default: {spec.default_bins})")
     p.add_argument("--seed", type=int, default=42, help="Random seed of the queried states (default: 42)")
     p.add_argument("--no-plot", action="store_true", help="Accepted for compatibility (plots are never produced)")
@@ -70,16 +79,35 @@ def train(runner: str, save_path: Path, bins: int | None = None, **kw):
     return pi
 
 
+def start_states(pi, n: int, seed: int) -> np.ndarray:
+    """`n` seeded uniform states inside the grid's bounds: the states summarize() queries and --rollout starts from."""
+    rng = np.random.default_rng(seed)
+    return (pi.bounds_low + (pi.bounds_high - pi.bounds_low) * rng.random((n, len(pi.bounds_low)))).astype(np.float32)
+
+
 def summarize(pi, n_queries: int, seed: int) -> dict:
     hist = np.bincount(pi.policy, minlength=len(pi.action_space))
     out = {"states": int(pi.policy.size), "V_min": float(pi.value_function.min()), "V_max": float(pi.value_function.max()),
            "policy_histogram": hist.tolist()}
     if n_queries > 0:
-        rng = np.random.default_rng(seed)
-        pts = (pi.bounds_low + (pi.bounds_high - pi.bounds_low) * rng.random((n_queries, len(pi.bounds_low)))).astype(np.float32)
+        pts = start_states(pi, n_queries, seed)
         out["queried_states"] = pts.tolist()
         out["interpolated_actions"] = pi.lookup_actions(pts).tolist()
     return out
+
+
+def rollout_summary(pi, episodes: int, steps: int, seed: int, gamma: float) -> dict:
+    """--rollout: closed-loop episodes from start_states() under the plugin's dynamics (pi.rollout)."""
+    res = pi.rollout(start_states(pi, episodes, seed), steps, gamma=gamma)
+    return {"episodes": episodes, "steps": steps, "mean_return": float(res.total_reward.mean()),
+            "mean_discounted_return": float(res.discounted_return.mean()), "mean_length": float(res.length.mean()),
+            "terminated": float(res.terminated.mean())}
+
+
+def format_rollout(r: dict) -> str:
+    return (f"[=] rollout {r['episodes']} episodes x {r['steps']} steps | mean return {r['mean_return']:.6f} | "
+            f"mean discounted return {r['mean_discounted_return']:.6f} | mean length {r['mean_length']:.2f} | "
+            f"terminated {r['terminated']:.4f}")
 
 
 def main(argv: list[str] | None = None) -> int:
@@ -109,6 +137,10 @@ def main(argv: list[str] | None = None) -> int:
     print(f"[=] {s['states']:,} states | V in [{s['V_min']:.4f}, {s['V_max']:.4f}] | policy histogram {s['policy_histogram']}")
     for p_, a_ in zip(s.get("queried_states", []), s.get("interpolated_actions", [])):
         print("    state " + np.array2string(np.asarray(p_), precision=3) + f" -> action {a_:.4f}")
+    if args.rollout and args.episodes > 0:
+        # the runner's gamma: a loaded policy carries the default CudaPIConfig, not the one it was trained with
+        gamma = float(np.float32(spec.config().gamma))
+        print(format_rollout(rollout_summary(pi, args.episodes, args.steps, args.seed, gamma)))
     return 0
 
 

@@ -273,6 +273,39 @@ int pi_lookup_create(const pi_grid* grid, const int32_t* policy, const float* ac
 int pi_lookup_query(pi_lookup* lookup, const float* points, int64_t n_points, float* out);
 void pi_lookup_destroy(pi_lookup* lookup);
 
+/* N5: closed-loop policy rollouts on the device.  Replaces the loop of every runner's evaluate() — get_optimal_action
+ * (utils/barycentric.py:76-108) followed by one environment step, once per simulated step on one CPU thread (e.g.
+ * runners/pendulum_cuda.py:161-166) — simulated with the plugin's own step_dynamics, compiled by NVRTC with the table
+ * builder's options (csrc/rollout_src.cuh).  One CUDA thread runs one whole episode:
+ *   x_0 = initial_states[e]; for t = 0..n_steps-1 until terminated:
+ *     a_t = the pi_lookup_query action at x_t (query clamped to the grid; x_t itself is never clamped or wrapped);
+ *     step_dynamics(x_t, a_t, &x_{t+1}, &r_t, &term_t);
+ *     total += (double)r_t;  ret += disc * (double)r_t;  disc *= gamma   (float64, disc starts at 1, no contraction);
+ *     length = t + 1; terminated = term_t.
+ * Episodes end only when step_dynamics sets *terminated; the terminal mask is not consulted.
+ *
+ * pi_rollout_create: the policy (reference order, n_states int32, validated like pi_lookup_create) and the action
+ * values are uploaded once; grid->axes is not used.  `dynamics_src` is the plugin's _dynamics_cuda_src() text
+ * (src/cuda_policy_iteration.py:113-125, :518-530, :941-954); errors as pi_create (PI_ERR_COMPILE with the NVRTC log,
+ * PI_ERR_NO_DEVICE: there is no CPU fallback). */
+typedef struct pi_rollout pi_rollout;
+int pi_rollout_create(const pi_grid* grid, const int32_t* policy, const float* actions, int32_t n_actions,
+                      const char* dynamics_src, int32_t device, pi_rollout** out);
+/* Host buffers, episode-major: initial_states / final_states n_episodes x D float32 (final = x_length);
+ * total_reward, discounted_return (f64), length (i32), terminated (u8) n_episodes each.  traj_*: all three or NULL;
+ * traj_states n x (n_steps+1) x D, traj_actions and traj_rewards n x n_steps, NaN after each episode's length.
+ * n_episodes == 0 and n_steps == 0 are valid; n_steps < 0 is PI_ERR_INVALID. */
+int pi_rollout_run(pi_rollout* r, const float* initial_states, int64_t n_episodes, int32_t n_steps, double gamma,
+                   double* total_reward, double* discounted_return, int32_t* length, uint8_t* terminated,
+                   float* final_states, float* traj_states, float* traj_actions, float* traj_rewards);
+/* One step_dynamics call per (states[i], actions[i]) pair — the environment step of evaluate() alone (n x D states,
+ * n actions in; n x D next states, n rewards, n terminated flags out). */
+int pi_rollout_step(pi_rollout* r, const float* states, const float* actions, int64_t n,
+                    float* next_states, float* rewards, uint8_t* terminated);
+void pi_rollout_destroy(pi_rollout* r);
+/* Compile-only check of a plugin's dynamics source against the rollout kernels (NVRTC, sm_100a); needs no GPU. */
+int pi_rollout_compile_check(const char* dynamics_src, int32_t n_dims, int64_t* cubin_bytes);
+
 #ifdef __cplusplus
 }
 #endif
