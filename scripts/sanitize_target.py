@@ -1,7 +1,11 @@
 #!/usr/bin/env python3
 """One sweep family on a small grid, for compute-sanitizer (tests/test_gpu_sanitizer.py):
     compute-sanitizer --tool memcheck --error-exitcode 1 python scripts/sanitize_target.py <family>
-families: aot | gp_single | gp_pair | xline | persistent | plane | plane_small | plane_scalar | plane_items_small | lookup"""
+families: aot | gp_single | gp_pair | xline | persistent | plane | plane_small | plane_scalar | plane_items_small | lookup |
+          rollout | odd_aot5 | odd_xline3 | odd_plane5
+The odd_* families run the chain-of-integrators fixture of tests/fixtures/odd_dims.py at D = 3 or 5 (rows with an odd
+number of words)."""
+import importlib.util
 import os
 import sys
 from pathlib import Path
@@ -21,6 +25,10 @@ cfg = {
     "plane_scalar": {"DPB200_PLANE": "force:0,0,2,2,0"},
     "plane_items_small": {"DPB200_PLANE": "force:34,5,2,2,2"},
     "lookup": {},
+    "rollout": {},
+    "odd_aot5": {"DPB200_PLANE": "off", "DPB200_XLINE": "off", "DPB200_PAIR": "off"},
+    "odd_xline3": {"DPB200_PLANE": "off", "DPB200_FAST_DIM": "0", "DPB200_XLINE": "force:2,0,4,8,2,1:1,1"},
+    "odd_plane5": {"DPB200_FAST_DIM": "0,1", "DPB200_PLANE": "force:0,0,2,2,2"},
 }[family]
 os.environ.update(cfg)
 os.environ["DPB200_CACHE"] = "off"
@@ -30,11 +38,18 @@ import numpy as np
 
 from dynamicprogramming_b200 import envs
 
-eng = envs.make(env, bins=bins)
+if family.startswith("odd_"):
+    spec = importlib.util.spec_from_file_location("odd_dims", ROOT / "tests" / "fixtures" / "odd_dims.py")
+    odd = importlib.util.module_from_spec(spec)
+    spec.loader.exec_module(odd)
+    eng = odd.make(int(family[-1]))
+else:
+    eng = envs.make(env, bins=bins)
 eng.build_table()
 info = eng.eval_kernel_info()["kernel"]
 want = {"aot": "eval_sweep_kernel", "gp_single": "gp_sweep", "gp_pair": "gp_sweep", "xline": "xl_sweep",
-        "persistent": "eval_persistent_kernel", "plane": "ps_sweep", "plane_small": "ps_sweep", "plane_scalar": "ps_sweep", "plane_items_small": "ps_sweep", "lookup": ""}[family]
+        "persistent": "eval_persistent_kernel", "plane": "ps_sweep", "plane_small": "ps_sweep", "plane_scalar": "ps_sweep", "plane_items_small": "ps_sweep", "lookup": "", "rollout": "",
+        "odd_aot5": "eval_sweep_kernel<5>", "odd_xline3": "xl_sweep", "odd_plane5": "ps_sweep"}[family]
 assert want in info, (family, info)
 eng.sweeps(3)
 eng.policy_improvement()
@@ -44,6 +59,13 @@ eng.sweeps(2)
 if family == "lookup":
     pts = np.random.default_rng(2).uniform(-1, 1, (257, eng.N_DIMS)).astype(np.float32)
     eng.lookup_actions(pts)
+if family == "rollout":   # pi_rollout_episodes, pi_step_states and the shared-memory tiles of rollout_unstage_kernel
+    rng = np.random.default_rng(3)
+    lo, hi = eng.bounds_low, eng.bounds_high
+    x0 = (lo + (hi - lo) * rng.uniform(-0.1, 1.1, (333, eng.N_DIMS))).astype(np.float32)
+    res = eng.rollout(x0, 37, record=True)
+    assert res.states.shape == (333, 38, eng.N_DIMS) and (res.length >= 1).all()
+    eng.simulate_step(x0, np.full(len(x0), eng.action_space[0], np.float32))
 v, p = eng.download()
 assert np.isfinite(v).all()
 eng.close()

@@ -1,6 +1,7 @@
 """compute-sanitizer over every sweep family (judge's round-1 finding: a heap-corrupting residual-buffer bug was found by
 a crashing bench, not by a test).  Each family runs scripts/sanitize_target.py — table build, sweeps with and without the
-residual, an improvement pass, a policy upload, a download — on a small grid under memcheck (out-of-bounds / misaligned
+residual, an improvement pass, a policy upload, a download (and for the rollout family a recorded closed-loop rollout and
+a single step) — on a small grid under memcheck (out-of-bounds / misaligned
 accesses, leaks of device memory are not checked) and synccheck; racecheck runs on the families that synchronise with
 bar.sync / shuffles.  The plane-staged sweep is excluded from racecheck only: its shared-memory hand-offs are mbarrier
 transactions (cp.async.bulk complete_tx -> try_wait), which racecheck reports as write/read hazards because it does not
@@ -28,9 +29,10 @@ def _sanitizer_usable() -> bool:
         return False
     return res.returncode == 0 and "Compute Sanitizer" in res.stdout
 
-FAMILIES = ["aot", "gp_single", "gp_pair", "xline", "persistent", "plane", "plane_small", "plane_scalar", "plane_items_small", "lookup"]
+FAMILIES = ["aot", "gp_single", "gp_pair", "xline", "persistent", "plane", "plane_small", "plane_scalar", "plane_items_small", "lookup",
+            "rollout", "odd_aot5", "odd_xline3", "odd_plane5"]
 CASES = [("memcheck", f) for f in FAMILIES] + [("synccheck", f) for f in ("plane", "plane_small", "plane_scalar", "persistent", "xline")] + \
-        [("racecheck", f) for f in ("aot", "gp_single", "xline", "persistent")]
+        [("racecheck", f) for f in ("aot", "gp_single", "xline", "persistent", "rollout")]
 
 
 @pytest.fixture(scope="module")
