@@ -135,3 +135,32 @@ def test_pipelined_policy_upload_equals_the_serial_upload(env, bins, plane, monk
     for mode in ("pipelined", "gather"):
         np.testing.assert_array_equal(res[mode][0], res["serial"][0])
         np.testing.assert_array_equal(res[mode][1], res["serial"][1])
+
+
+def test_debug_hooks_under_the_plane_sweep_leave_the_engine_as_it_was(monkeypatch):
+    """debug_pair and debug_xline on an engine that runs the plane-staged sweep: they set it aside with the other JIT
+    sweeps and compare their candidate with the gather sweep; afterwards the engine selects the same kernel and sweeps
+    to the same V bits as a twin that never called them."""
+    monkeypatch.setenv("DPB200_FAST_DIM", "0,1")   # dims 0, 1 fastest: a plane layout on which x-line sweeps apply
+    monkeypatch.setenv("DPB200_PLANE", "force")
+    engines = []
+    for _ in range(2):
+        eng = envs.make("double_cartpole_swingup", bins=8)
+        eng.build_table()
+        eng.sweeps(3)
+        eng.policy_improvement()
+        eng.sweeps(4)
+        engines.append(eng)
+    eng, twin = engines
+    before = eng.eval_kernel_info()
+    assert before["plane"] and "ps_sweep" in before["kernel"], before
+    out = eng.debug_pair(128, 8, iters=1, lv=2, group=8, single=1)
+    assert out["mismatches"] == 0, out
+    out = eng.debug_xline("4,0,4,8,1,1:1,1,2,4,4", iters=1)
+    assert out["mismatches"] == 0, out
+    assert eng.eval_kernel_info() == before
+    for e in engines:
+        e.sweeps(5)
+    np.testing.assert_array_equal(bits(eng.download()[0]), bits(twin.download()[0]))
+    for e in engines:
+        e.close()
