@@ -108,6 +108,7 @@ SIGNATURES = {
     "pi_launch_count": (C.c_int64, [C.c_void_p]),
     "pi_get_stats": (C.c_int, [C.c_void_p, C.POINTER(PiStats)]),
     "pi_lookup_actions": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int64, C.c_void_p]),
+    "pi_prolong_values": (C.c_int, [C.c_void_p, C.POINTER(PiGrid), C.c_void_p, C.POINTER(C.c_float)]),
     "pi_lookup_create": (C.c_int, [C.POINTER(PiGrid), C.c_void_p, C.c_void_p, C.c_int32, C.c_int32, C.POINTER(C.c_void_p)]),
     "pi_lookup_query": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int64, C.c_void_p]),
     "pi_lookup_destroy": (None, [C.c_void_p]),

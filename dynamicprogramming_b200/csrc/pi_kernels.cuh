@@ -1339,6 +1339,39 @@ __global__ void __launch_bounds__(kBlock) lookup_actions_kernel(LookupGrid g, co
     out[i] = lookup_point(g, g.n_dims, points + i * g.n_dims, policy, actions);
 }
 
+// Warm start (pi_prolong_values): V[s] = the source value function `src` (reference order, grid `sg`, taken as uniform)
+// interpolated at the node of state s of this rank's slice, with interp_value_point's arithmetic.  One thread per local
+// state in storage order; the node is read from the engine's axes (the float32 bits of states_space).  Absorbing states
+// (term[k], the per-state flag the table builder turned into PI_ROW_ABSORBING rows) keep the value they hold.  Writes
+// both V buffers.
+struct AxisPtrs {
+    const float* a[kMaxDims];
+};
+
+template <int D>
+__global__ void __launch_bounds__(kBlock) prolong_values_kernel(GridDesc g, AxisPtrs axes, LookupGrid sg,
+                                                                const float* __restrict__ src,
+                                                                const unsigned char* __restrict__ term, long long s_begin,
+                                                                long long n_local, float* V0, float* V1) {
+    const long long k = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+    if (k >= n_local || term[k]) return;
+    float x[D];
+    long long r = s_begin + k;
+#pragma unroll
+    for (int j = D - 1; j >= 0; --j) {   // storage position j holds logical dimension perm[j]
+        const int d = g.perm[j];
+        const long long q = r / g.shape[d];
+        const float node = axes.a[d][r - q * g.shape[d]];
+        r = q;
+#pragma unroll
+        for (int e = 0; e < D; ++e)      // x stays in registers: no run-time index into it
+            if (e == d) x[e] = node;
+    }
+    const float v = interp_value_point(sg, D, x, src);
+    V0[s_begin + k] = v;
+    V1[s_begin + k] = v;
+}
+
 // Recorded rollout trajectories (rollout_src.cuh) are staged step-major: a rows x n matrix, row r = t * per + k,
 // column = episode.  This writes its transpose out[e][r] (the episode-major host layout) through 32 x 32 shared-memory
 // tiles, both sides coalesced, and puts NaN where step t = r / per lies beyond the episode (r >= (length[e] + extra) * per).

@@ -516,6 +516,27 @@ class _CudaPolicyIterationBase(abc.ABC):
         assert v.shape == (self.n_states,)
         _ffi.check(_ffi.lib().pi_upload_values(self._engine, _ffi.ptr(v)))
 
+    def warm_start(self, source) -> dict:
+        """Start from another grid's solution instead of V = 0, policy = 0 (include/dpb200.h: pi_prolong_values).
+
+        `source` is a saved-policy .npz path, an instance after run() or load() (`value_function`, `bounds_low`,
+        `bounds_high`, `grid_shape`), or a `(values, bounds_low, bounds_high, grid_shape)` tuple; its grid is taken as
+        uniform.  Every non-absorbing state gets the source V interpolated at its node (clamped to the source box, the
+        arithmetic of lookup_actions); absorbing states keep their values.  Then one policy_improvement() makes the
+        policy greedy with respect to that V, and a following run() evaluates it starting from the prolonged V.
+        Returns {"prolong_ms": device time of the prolongation kernel, "changed": states whose action differs from the
+        policy held before (pi = 0 on a fresh engine)}.  retrain() resets V and the policy as usual."""
+        values, lo, hi, shape = _warm_start_source(source)
+        self.build_table()
+        grid = _ffi.PiGrid()
+        grid.n_dims = len(shape)
+        for d in range(len(shape)):
+            grid.shape[d], grid.lo[d], grid.hi[d] = int(shape[d]), float(lo[d]), float(hi[d])
+        ms = C.c_float()
+        _ffi.check(_ffi.lib().pi_prolong_values(self._engine, C.byref(grid), _ffi.ptr(values), C.byref(ms)))
+        self.policy_improvement()
+        return {"prolong_ms": float(ms.value), "changed": self.last_changed}
+
     def download(self, values: np.ndarray | None = None, policy: np.ndarray | None = None):
         if values is None:
             values = np.empty(self.n_states, dtype=np.float32)
@@ -666,6 +687,37 @@ class _CudaPolicyIterationBase(abc.ABC):
         _ffi.check(lib.pi_expand_rows(self._engine, int(action), int(s_begin), int(count), _ffi.ptr(idx), _ffi.ptr(w),
                                       _ffi.ptr(r), _ffi.ptr(t)))
         return idx, w, r, t
+
+
+def _warm_start_source(source):
+    """(values float32, bounds_low, bounds_high, grid_shape) of a warm-start source (see warm_start), validated on the
+    host before any device work: a missing .npz entry raises KeyError, a dimensionality the C ABI cannot take raises
+    ValueError, and a value count other than prod(grid_shape) raises EngineError (PI_ERR_INVALID)."""
+    keys = ("value_function", "bounds_low", "bounds_high", "grid_shape")
+    if isinstance(source, (str, Path)):
+        path = Path(source).with_suffix(".npz")
+        with np.load(path) as data:
+            missing = [k for k in keys if k not in data.files]
+            if missing:
+                raise KeyError(f"{path}: warm-start source lacks {missing}")
+            parts = [data[k] for k in keys]
+    elif isinstance(source, tuple):
+        if len(source) != 4:
+            raise ValueError("a warm-start tuple is (values, bounds_low, bounds_high, grid_shape)")
+        parts = list(source)
+    else:
+        parts = [getattr(source, k) for k in keys]
+    values = np.ascontiguousarray(np.asarray(parts[0]).ravel(), dtype=np.float32)
+    lo = np.asarray(parts[1], dtype=np.float32).ravel()
+    hi = np.asarray(parts[2], dtype=np.float32).ravel()
+    shape = np.asarray(parts[3], dtype=np.int64).ravel()
+    if not 1 <= len(shape) <= _ffi.PI_MAX_DIMS or len(lo) != len(shape) or len(hi) != len(shape):
+        raise ValueError(f"warm-start source: grid_shape {shape.tolist()} and bounds of {len(lo)} / {len(hi)} entries "
+                         f"do not describe a 1..{_ffi.PI_MAX_DIMS}-D grid")
+    if values.size != int(np.prod(shape)):
+        raise _ffi.EngineError(_ffi.PI_ERR_INVALID, f"warm-start source has {values.size} values for a grid of shape "
+                                                    f"{shape.tolist()} ({int(np.prod(shape))} states)")
+    return values, lo, hi, shape
 
 
 class CudaPolicyIteration2D(_CudaPolicyIterationBase):

@@ -20,11 +20,17 @@ With `--rollout` it also runs what evaluate() runs — the policy in closed loop
 with the plugin's own float32 `step_dynamics` (the model the DP solved, not gymnasium;
 include/dpb200.h: pi_rollout_*), discounted with the runner's gamma, and prints one summary line:
 mean return, mean discounted return, mean length, fraction of episodes that terminated.
+
+With `--warm-start-bins B` a training run first solves the same runner with the same config at `B` bins and starts
+the `--bins` solve from that value function (engine.warm_start); `--warm-start-from PATH` starts it from a saved
+policy's value function instead.  Either flag adds one line per solve: bins, PI iterations, evaluation sweeps and
+host seconds (construction, warm start and run(), not the save).
 """
 from __future__ import annotations
 
 import argparse
 import sys
+import time
 from pathlib import Path
 
 import numpy as np
@@ -63,6 +69,11 @@ def build_parser(runner: str) -> argparse.ArgumentParser:
     p.add_argument("--no-plot", action="store_true", help="Accepted for compatibility (plots are never produced)")
     p.add_argument("--retrain", action="store_true", help="Force retraining even if a saved policy exists")
     p.add_argument("--save-path", type=Path, default=Path(f"results/{runner}_policy.npz"))
+    warm = p.add_mutually_exclusive_group()
+    warm.add_argument("--warm-start-bins", type=int, default=None, metavar="B",
+                      help="When training: first solve at B bins, then start the --bins solve from its value function")
+    warm.add_argument("--warm-start-from", type=Path, default=None, metavar="PATH",
+                      help="When training: start the --bins solve from the value function of a saved policy (.npz)")
     if runner == "overhead_crane_cuda":
         p.add_argument("--start-x", type=float, default=2.5, help="Accepted for compatibility (roll-out start)")
         p.add_argument("--target-x", type=float, default=-2.5, help="Target trolley position (m), baked into the CUDA source")
@@ -77,6 +88,35 @@ def train(runner: str, save_path: Path, bins: int | None = None, **kw):
     pi.run()
     pi.save(save_path)
     return pi
+
+
+def train_warm(runner: str, save_path: Path, bins: int | None = None, warm_bins: int | None = None,
+               warm_from: Path | None = None, **kw):
+    """train() started from a coarser solution: a solve at `warm_bins` (same runner, same config), or the saved policy
+    `warm_from`, warm-starts the solve at `bins` (engine.warm_start).  Returns the trained engine and one dict per solve
+    (bins, PI iterations, evaluation sweeps, host seconds)."""
+    spec = envs.REGISTRY[RUNNERS[runner]]
+    solves = []
+
+    def solve(b, source=None):
+        t0 = time.perf_counter()
+        pi = spec.make(bins=b, **kw)
+        if source is not None:
+            pi.warm_start(source)
+        pi.run()
+        solves.append({"bins": spec.default_bins if b is None else int(b), "pi_iterations": pi.pi_iterations, "sweeps": pi.total_eval_sweeps,
+                       "seconds": time.perf_counter() - t0})
+        return pi
+
+    source = solve(warm_bins) if warm_from is None else warm_from
+    pi = solve(bins, source)
+    pi.save(save_path)
+    return pi, solves
+
+
+def format_solve(s: dict) -> str:
+    return (f"[=] solve at {s['bins']} bins | {s['pi_iterations']} PI iterations | {s['sweeps']} evaluation sweeps | "
+            f"{s['seconds']:.2f} s")
 
 
 def start_states(pi, n: int, seed: int) -> np.ndarray:
@@ -129,7 +169,13 @@ def main(argv: list[str] | None = None) -> int:
         pi = spec.cls.load(args.save_path)
     else:
         print("[*] Training new policy...")
-        pi = train(runner, args.save_path, bins=args.bins, **kw)
+        if args.warm_start_bins is None and args.warm_start_from is None:
+            pi = train(runner, args.save_path, bins=args.bins, **kw)
+        else:
+            pi, solves = train_warm(runner, args.save_path, bins=args.bins, warm_bins=args.warm_start_bins,
+                                    warm_from=args.warm_start_from, **kw)
+            for s_ in solves:
+                print(format_solve(s_))
     for flag, what in ((args.render, "--render"), (args.record, "--record")):
         if flag:
             print(f"[!] {what}: rendering / recording needs gymnasium + pygame and is outside the DP path; skipped")

@@ -264,6 +264,22 @@ int pi_debug_pair(pi_engine* e, int32_t threads, int32_t minb, int32_t lv, int32
  * points: n_points x n_dims float32 (host); out: n_points float32 (host). */
 int pi_lookup_actions(pi_engine* e, const float* points, int64_t n_points, float* out);
 
+/* N6: warm start from another grid's value function (new; the reference has no counterpart — every run of it starts
+ * from V = 0, policy = 0, src/cuda_policy_iteration.py:142-175).  Enables solving at a coarse --bins first (the
+ * autoresearch loop trains and scores at --bins 12, runners/trial_runner.sh) and starting the fine solve from that V.
+ * For every state of this rank's slice that is not absorbing (terminal mask), both V buffers get the source value
+ * function interpolated at the state's node (grid->axes bits) with the arithmetic of pi_lookup_actions: the node is
+ * clamped to the source box, the source grid is taken as uniform from source->lo / hi / shape (source->axes is not
+ * used), float64 fractions and weight products, corner_bits order, float32 sum in ascending corner order.  Absorbing
+ * states keep the value they hold (pi_set_terminal / pi_set_values).  `source_values` has prod(source->shape) floats in
+ * reference order.  *device_ms (may be NULL) = CUDA-event time of the prolongation kernel.  Sharded engines: collective;
+ * every rank computes its slice and the full V is all-gathered.  PI_ERR_INVALID for a null pointer, a different n_dims,
+ * a source shape[d] < 2, lo[d] >= hi[d] or a call before pi_build_table; the engine stays usable.
+ * The policy is not touched: pi_improve afterwards makes it greedy with respect to the prolonged V (and re-compacts the
+ * rows, re-plans and reselects the sweep kernel); its `stable` / n_changed then compare with the policy held before the
+ * warm start, not with a converged one, and mean nothing for convergence. */
+int pi_prolong_values(pi_engine* e, const pi_grid* source, const float* source_values, float* device_ms);
+
 /* The same lookup for a SAVED policy (Cls.load(path), src/cuda_policy_iteration.py:411-432;
  * runners/hybrid_double_cartpole.py:35-43): the policy table (reference order, n_states int32)
  * and the action values are uploaded once, queries are batched.  grid->axes is not used. */

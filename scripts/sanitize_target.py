@@ -2,7 +2,9 @@
 """One sweep family on a small grid, for compute-sanitizer (tests/test_gpu_sanitizer.py):
     compute-sanitizer --tool memcheck --error-exitcode 1 python scripts/sanitize_target.py <family>
 families: aot | gp_single | gp_pair | xline | persistent | plane | plane_small | plane_scalar | plane_items_small | lookup |
-          rollout | odd_aot5 | odd_xline3 | odd_plane5
+          rollout | odd_aot5 | odd_xline3 | odd_plane5 | warm_start
+warm_start prolongs a coarser and a finer source value function onto an engine with a terminal mask (the overhead
+crane, whose goal states also carry values from set_values) and runs an improvement and sweeps from it.
 The odd_* families run the chain-of-integrators fixture of tests/fixtures/odd_dims.py at D = 3 or 5 (rows with an odd
 number of words)."""
 import importlib.util
@@ -29,11 +31,14 @@ cfg = {
     "odd_aot5": {"DPB200_PLANE": "off", "DPB200_XLINE": "off", "DPB200_PAIR": "off"},
     "odd_xline3": {"DPB200_PLANE": "off", "DPB200_FAST_DIM": "0", "DPB200_XLINE": "force:2,0,4,8,2,1:1,1"},
     "odd_plane5": {"DPB200_FAST_DIM": "0,1", "DPB200_PLANE": "force:0,0,2,2,2"},
+    "warm_start": {},
 }[family]
 os.environ.update(cfg)
 os.environ["DPB200_CACHE"] = "off"
 if family == "persistent":
     env, bins = "cartpole", 10
+if family == "warm_start":
+    env, bins = "overhead_crane", 11
 import numpy as np
 
 from dynamicprogramming_b200 import envs
@@ -49,7 +54,8 @@ eng.build_table()
 info = eng.eval_kernel_info()["kernel"]
 want = {"aot": "eval_sweep_kernel", "gp_single": "gp_sweep", "gp_pair": "gp_sweep", "xline": "xl_sweep",
         "persistent": "eval_persistent_kernel", "plane": "ps_sweep", "plane_small": "ps_sweep", "plane_scalar": "ps_sweep", "plane_items_small": "ps_sweep", "lookup": "", "rollout": "",
-        "odd_aot5": "eval_sweep_kernel<5>", "odd_xline3": "xl_sweep", "odd_plane5": "ps_sweep"}[family]
+        "odd_aot5": "eval_sweep_kernel<5>", "odd_xline3": "xl_sweep", "odd_plane5": "ps_sweep",
+        "warm_start": ""}[family]
 assert want in info, (family, info)
 eng.sweeps(3)
 eng.policy_improvement()
@@ -66,6 +72,12 @@ if family == "rollout":   # pi_rollout_episodes, pi_step_states and the shared-m
     res = eng.rollout(x0, 37, record=True)
     assert res.states.shape == (333, 38, eng.N_DIMS) and (res.length >= 1).all()
     eng.simulate_step(x0, np.full(len(x0), eng.action_space[0], np.float32))
+if family == "warm_start":   # pi_prolong_values from a coarser and a finer source, then improvement + sweeps
+    for b in (7, 16):
+        n = b ** eng.N_DIMS
+        src = np.random.default_rng(b).standard_normal(n).astype(np.float32)
+        eng.warm_start((src, eng.bounds_low, eng.bounds_high, np.full(eng.N_DIMS, b)))
+        eng.sweeps(3)
 v, p = eng.download()
 assert np.isfinite(v).all()
 eng.close()
