@@ -78,6 +78,7 @@ SIGNATURES = {
     "pi_nccl_unique_id": (C.c_int, [C.c_void_p]),
     "pi_nvrtc_counters": (C.c_int, [C.POINTER(C.c_int64), C.POINTER(C.c_int64)]),
     "pi_compile_check": (C.c_int, [C.c_char_p, C.c_int32, C.POINTER(C.c_int64)]),
+    "pi_recompute_compile_check": (C.c_int, [C.c_char_p, C.c_int32, C.POINTER(C.c_int64)]),
     "pi_create": (C.c_int, [C.POINTER(PiGrid), C.POINTER(C.c_float), C.c_int32, C.POINTER(PiConfig), C.c_char_p,
                             C.c_int32, C.POINTER(PiShard), C.POINTER(C.c_void_p)]),
     "pi_destroy": (None, [C.c_void_p]),
@@ -105,6 +106,7 @@ SIGNATURES = {
     "pi_local_begin": (C.c_int64, [C.c_void_p]),
     "pi_local_end": (C.c_int64, [C.c_void_p]),
     "pi_table_bytes": (C.c_int64, [C.c_void_p]),
+    "pi_table_mode": (C.c_int32, [C.c_void_p]),
     "pi_launch_count": (C.c_int64, [C.c_void_p]),
     "pi_get_stats": (C.c_int, [C.c_void_p, C.POINTER(PiStats)]),
     "pi_lookup_actions": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int64, C.c_void_p]),

@@ -229,11 +229,6 @@ __device__ __forceinline__ unsigned ld_stream4_hint(const void* p, unsigned long
     asm volatile("ld.global.nc.L1::no_allocate.L2::cache_hint.u32 %0, [%1], %2;" : "=r"(r) : "l"(p), "l"(pol));
     return r;
 }
-__device__ __forceinline__ float ld_keep4(const float* p, unsigned long long pol) {
-    float r;
-    asm volatile("ld.global.nc.L2::cache_hint.f32 %0, [%1], %2;" : "=f"(r) : "l"(p), "l"(pol));
-    return r;
-}
 
 // load_row with an L2 eviction policy on every plane
 template <int D>
@@ -291,22 +286,8 @@ __device__ __forceinline__ void store_row(unsigned char* __restrict__ tab, long 
     }
 }
 
-// ---------------------------------------------------------------------------
-// Corner enumeration of the reference.
-//   D == 2 : idxs[0..3] = (i0,i1) (i0,i1+1) (i0+1,i1) (i0+1,i1+1)   (:201-209)
-//            -> bit of dim d in corner c is (c >> (1-d)) & 1
-//   D >= 3 : bit d of c selects i[d] or i[d]+1                       (:602-613, :1030-1041)
-// ---------------------------------------------------------------------------
-template <int D>
-__host__ __device__ constexpr int corner_bit(int c, int d) {
-    return D == 2 ? ((c >> (1 - d)) & 1) : ((c >> d) & 1);
-}
+#include "row_value_src.cuh"
 
-// Expected next-state value  sum_c w_c * V[idx_c]  with the reference's exact
-// arithmetic: w_c = ((((1*f_0)*f_1)...)*f_{D-1}), f_d = bit ? frac_d : 1-frac_d,
-// accumulated as ev = fmaf(w_c, V[idx_c], ev) for c = 0 .. 2^D-1 from ev = 0
-// (:236-239, :643-646, :1074-1076).  Prefix products are shared between corners
-// (same multiplication order per corner, so the same rounding).
 __device__ __forceinline__ float ld_nc_ordered(const float* p) {   // volatile: keeps its place among the other gathers
     float r;
     asm volatile("ld.global.nc.f32 %0, [%1];" : "=f"(r) : "l"(p));
@@ -366,148 +347,11 @@ __device__ __forceinline__ float expected_value_grouped(const float* __restrict_
     return ev;
 }
 
-// CG = true: gathers bypass the L1 (ld.global.cg) — the persistent multi-sweep kernel reads values other
-// SMs wrote one grid barrier ago, and the L1 is not coherent.
-template <bool CG>
-__device__ __forceinline__ float ld_v(const float* p) {
-    if constexpr (CG) return __ldcg(p);
-    else return *p;
-}
-
-template <int D, bool KEEP = false, int LV = 0, bool CG = false>
-__device__ __forceinline__ float expected_value(const float* __restrict__ V, int base,
-                                                const float (&frac)[D], const int (&stride)[D],
-                                                unsigned long long keep_pol = 0ull) {
-    constexpr int C = 1 << D;
-    if constexpr (LV == 1 && D >= 4) {
-        // Register-lean form: prefix products over the first D-2 dims only (2^(D-2) registers instead of
-        // 2^(D-1)); the factors of dims D-2 and D-1 are applied per corner, in the same left-to-right
-        // order ((pre * f_{D-2}) * f_{D-1}) — one more multiply per corner, identical rounding.
-        constexpr int Q = C / 4;
-        float pre[Q];
-        pre[0] = 1.0f - frac[0];
-        pre[1] = frac[0];
-#pragma unroll
-        for (int d = 1; d < D - 2; ++d) {
-            const float g = 1.0f - frac[d];
-#pragma unroll
-            for (int c = (1 << d) - 1; c >= 0; --c) {
-                const float p = pre[c];
-                pre[c + (1 << d)] = p * frac[d];
-                pre[c] = p * g;
-            }
-        }
-        const float fm = frac[D - 2], gm = 1.0f - fm, fl = frac[D - 1], gl = 1.0f - fl;
-        const float* v = V + base;
-        float ev = 0.0f;
-#pragma unroll
-        for (int c = 0; c < C; ++c) {
-            int off = 0;
-#pragma unroll
-            for (int d = 0; d < D; ++d)
-                if (corner_bit<D>(c, d)) off += stride[d];
-            float x;
-            if constexpr (KEEP) x = ld_keep4(v + off, keep_pol);
-            else x = v[off];
-            const float w = (pre[c & (Q - 1)] * (((c >> (D - 2)) & 1) ? fm : gm)) * ((c >> (D - 1)) ? fl : gl);
-            ev = fmaf(w, x, ev);
-        }
-        return ev;
-    } else
-    if constexpr (D == 1) {
-        const float* v = V + base;
-        float ev = fmaf(1.0f - frac[0], ld_v<CG>(v), 0.0f);
-        return fmaf(frac[0], ld_v<CG>(v + stride[0]), ev);
-    } else if constexpr (D == 2) {
-        const float g0 = 1.0f - frac[0], g1 = 1.0f - frac[1];
-        const float* v = V + base;
-        const float v00 = ld_v<CG>(v), v01 = ld_v<CG>(v + stride[1]), v10 = ld_v<CG>(v + stride[0]),
-                    v11 = ld_v<CG>(v + stride[0] + stride[1]);
-        float ev = 0.0f;
-        ev = fmaf(g0 * g1, v00, ev);
-        ev = fmaf(g0 * frac[1], v01, ev);
-        ev = fmaf(frac[0] * g1, v10, ev);
-        ev = fmaf(frac[0] * frac[1], v11, ev);
-        return ev;
-    } else {
-        // weights over the first D-1 dims (2^(D-1) prefix products), last dim applied on the fly
-        constexpr int H = C / 2;
-        float pre[H];
-        pre[0] = 1.0f - frac[0];
-        pre[1] = frac[0];
-#pragma unroll
-        for (int d = 1; d < D - 1; ++d) {
-            const float g = 1.0f - frac[d];
-#pragma unroll
-            for (int c = (1 << d) - 1; c >= 0; --c) {
-                const float p = pre[c];
-                pre[c + (1 << d)] = p * frac[d];
-                pre[c] = p * g;
-            }
-        }
-        const float gl = 1.0f - frac[D - 1];
-        const float* v = V + base;
-        float val[C];
-#pragma unroll
-        for (int c = 0; c < C; ++c) {
-            int off = 0;
-#pragma unroll
-            for (int d = 0; d < D; ++d)
-                if (corner_bit<D>(c, d)) off += stride[d];
-            if constexpr (KEEP) val[c] = ld_keep4(v + off, keep_pol);
-            else val[c] = ld_v<CG>(v + off);
-        }
-        float ev = 0.0f;
-#pragma unroll
-        for (int c = 0; c < H; ++c) ev = fmaf(pre[c] * gl, val[c], ev);
-#pragma unroll
-        for (int c = 0; c < H; ++c) ev = fmaf(pre[c] * frac[D - 1], val[c + H], ev);
-        return ev;
-    }
-}
 
 __device__ __forceinline__ float warp_max(float v) {
 #pragma unroll
     for (int o = 16; o > 0; o >>= 1) v = fmaxf(v, __shfl_xor_sync(0xffffffffu, v, o));
     return v;
-}
-
-// How regular are the rows of the current policy along the fast-stored dimension?  A group of K
-// consecutive states is regular when every live state has base_j - j == A with A % K in {0, K-1}
-// (the window condition of the x-line sweep, xline_sweep_src.cuh).  Called by all threads of a
-// block whose thread index == local state index modulo 32 (groups never straddle a warp);
-// counters: [0] pairs, [1] regular pairs, [2] quads, [3] regular quads.
-__device__ __forceinline__ void count_regular_groups(int base, bool in, unsigned long long* counters) {
-    if (counters == nullptr) return;
-    // Only the FRACTION matters: on large grids every 4th block is counted, reduced in shared memory,
-    // and adds 4 global atomics (an atomic per warp cost 8 ms on K5: 8 M same-address atomics).
-    if (gridDim.x > 1024 && (blockIdx.x & 3) != 0) return;
-    __shared__ unsigned s_cnt[4];
-    if (threadIdx.x < 4) s_cnt[threadIdx.x] = 0;
-    __syncthreads();
-    const unsigned full = 0xffffffffu;
-    const int lane = threadIdx.x & 31;
-    const bool live = base >= 0;
-    const unsigned livem = __ballot_sync(full, live);
-#pragma unroll
-    for (int K = 2; K <= 4; K += 2) {
-        const int j = lane % K;
-        const unsigned gmask = ((1u << K) - 1u) << (lane - j);
-        const unsigned lm = livem & gmask;
-        const int t = base - j;
-        const int A = __shfl_sync(full, t, lm ? __ffs(lm) - 1 : lane);
-        const unsigned okm = __ballot_sync(full, !live || t == A) & gmask;
-        const int m = A & (K - 1);
-        const bool regular = lm == 0 || (okm == gmask && (m == 0 || m == K - 1));
-        const unsigned heads = __ballot_sync(full, in && j == 0);
-        const unsigned regs = __ballot_sync(full, in && j == 0 && regular);
-        if (lane == 0 && heads) {
-            atomicAdd(&s_cnt[K - 2], (unsigned)__popc(heads));
-            atomicAdd(&s_cnt[K - 1], (unsigned)__popc(regs));
-        }
-    }
-    __syncthreads();
-    if (threadIdx.x < 4 && s_cnt[threadIdx.x]) atomicAdd(counters + threadIdx.x, (unsigned long long)s_cnt[threadIdx.x]);
 }
 
 // ---------------------------------------------------------------------------

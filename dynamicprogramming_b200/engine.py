@@ -387,6 +387,7 @@ class _CudaPolicyIterationBase(abc.ABC):
         d = st.as_dict()
         d["launches"] = int(_ffi.lib().pi_launch_count(self._engine))
         d["table_bytes"] = int(_ffi.lib().pi_table_bytes(self._engine))
+        d["table_mode"] = "recompute" if _ffi.lib().pi_table_mode(self._engine) == 1 else "full"
         return d
 
     def _pull_tensors_from_gpu(self) -> None:

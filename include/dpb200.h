@@ -107,6 +107,9 @@ int pi_nvrtc_counters(int64_t* compiles, int64_t* cache_hits);
  * template (NVRTC, sm_100a); needs no GPU.  Errors carry the NVRTC log — the
  * analogue of cupy's CompileException at src/cuda_policy_iteration.py:289. */
 int pi_compile_check(const char* dynamics_src, int32_t n_dims, int64_t* cubin_bytes);
+/* The same compile, checked for the recompute-mode kernels of the builder program (pi_improve_recompute,
+ * pi_policy_rows; see pi_table_mode); needs no GPU.  Errors carry the NVRTC log. */
+int pi_recompute_compile_check(const char* dynamics_src, int32_t n_dims, int64_t* cubin_bytes);
 
 /* ncclGetUniqueId for pi_shard.nccl_id: rank 0 calls it and ships the 128 bytes
  * to the other ranks through its own process group (torch.distributed). */
@@ -116,7 +119,17 @@ int pi_nccl_unique_id(uint8_t out[128]);
  * :142-175, :288-296).  `dynamics_src` is the string returned by the plugin's
  * _dynamics_cuda_src() (:113-125, :518-530, :941-954); it is compiled by NVRTC
  * (default options, like cupy.RawModule) into the transition-table builder.
- * policy := 0, V := 0.  `shard` may be NULL (single GPU). */
+ * policy := 0, V := 0.  `shard` may be NULL (single GPU).
+ *
+ * Table mode (N7), read from DPB200_TABLE = auto | full | recompute here (any other value: PI_ERR_INVALID) and kept
+ * for the engine's life, pi_retrain and pooled reuse included:
+ *   full       the all-action table (A rows per state) is allocated and built once; the improvement pass reads it.
+ *   recompute  no table is allocated: wherever the table was read (improvement, policy rows, pi_expand_rows, the
+ *              sharded exchange plan) the rows are recomputed on the device by the builder's own code.  Results are
+ *              bit-identical to full mode; only memory and time differ.
+ *   auto       full when the table plus the engine's other buffers plus a fixed reserve fit the free device
+ *              memory (cudaMemGetInfo) and the table's allocation succeeds, else recompute.  Each rank of a sharded
+ *              engine decides for its own slice. */
 int pi_create(const pi_grid* grid, const float* actions, int32_t n_actions,
               const pi_config* config, const char* dynamics_src, int32_t device,
               const pi_shard* shard, pi_engine** out);
@@ -141,7 +154,8 @@ int pi_set_values_buffer(pi_engine* e, int32_t which, const uint8_t* mask, float
 /* Transition-table build (new stage; arithmetic oracle = step_dynamics +
  * get_barycentric_{2,4,6}d, src/cuda_policy_iteration.py:183-210, :580-614,
  * :1007-1042).  One compact row per (state, action): base flat index,
- * n_dims interpolation fractions, reward.  Must follow pi_set_terminal. */
+ * n_dims interpolation fractions, reward.  Must follow pi_set_terminal.  Recompute mode: only the rows of the
+ * current policy are built (pi_stats.build_ms is their device time). */
 int pi_build_table(pi_engine* e);
 
 /* N4 — a persistent engine across autoresearch trials (runners/trial_runner.sh:33-60 starts a new Python process per trial;
@@ -150,7 +164,8 @@ int pi_build_table(pi_engine* e);
  * and rebuilds the transition table, recompiling the builder only when `dynamics_src` differs from the text it was built
  * from (*recompiled).  Everything that does not depend on the dynamics is kept: CUDA context, buffers, storage order,
  * the JIT-compiled sweep kernels, CUDA graphs, the NCCL communicator and the peer mappings.  Equivalent to
- * pi_destroy + pi_create + pi_set_terminal + pi_build_table for the same grid, bit for bit. */
+ * pi_destroy + pi_create + pi_set_terminal + pi_build_table for the same grid, bit for bit.  The table mode is kept;
+ * in recompute mode only the policy-0 rows are rebuilt. */
 int pi_retrain(pi_engine* e, const char* dynamics_src, const uint8_t* terminal_mask, float terminal_value, int32_t* recompiled);
 
 /* policy_evaluation() (src/cuda_policy_iteration.py:300-336): Jacobi sweeps,
@@ -161,7 +176,8 @@ int pi_evaluate(pi_engine* e, float* delta, int32_t* sweeps);
 
 /* policy_improvement() (src/cuda_policy_iteration.py:338-355): greedy argmax,
  * strict '>' from -1e30f so the lowest action index wins ties; *stable = 1 iff
- * no state changed its action. */
+ * no state changed its action.  Recompute mode: every (state, action) row is recomputed from the dynamics in this
+ * pass, with the same result; pi_stats.improve_ms includes that work. */
 int pi_improve(pi_engine* e, int32_t* stable, int64_t* n_changed);
 
 /* run() (src/cuda_policy_iteration.py:357-370) without the final D2H. */
@@ -191,7 +207,8 @@ int pi_sweeps(pi_engine* e, int32_t n_sweeps, float* delta, float* device_ms);
  * rank's range) and action `action`, writes idx[count][C], w[count][C],
  * reward[count], terminated[count] exactly as step_dynamics +
  * get_barycentric_Nd would produce them (corner c, bit d <-> dim d for
- * D=4,6; the 2-D corner order of :201-209 for D=2).  Any output may be NULL. */
+ * D=4,6; the 2-D corner order of :201-209 for D=2).  Any output may be NULL.  Recompute mode: the action's rows of
+ * this rank's slice are recomputed into a temporary buffer first (same bits as the table). */
 int pi_expand_rows(pi_engine* e, int32_t action, int64_t s_begin, int64_t count,
                    int32_t* idx, float* w, float* reward, uint8_t* terminated);
 
@@ -214,10 +231,14 @@ int pi_layout(const pi_engine* e, int32_t* fast_dim, int32_t perm[PI_MAX_DIMS],
 int64_t pi_n_states(const pi_engine* e);
 int64_t pi_local_begin(const pi_engine* e);
 int64_t pi_local_end(const pi_engine* e);
+/* Device bytes of the all-action table plus the policy's rows; 0 in recompute mode (no table). */
 int64_t pi_table_bytes(const pi_engine* e);
+/* 0 = full table, 1 = recompute (see pi_create). */
+int32_t pi_table_mode(const pi_engine* e);
 /* Number of kernel launches issued by this engine so far (bench bookkeeping). */
 int64_t pi_launch_count(const pi_engine* e);
-/* Last-stage device timings in ms (build, eval, improve). */
+/* Last-stage device timings in ms (build, eval, improve).  Recompute mode: build_ms is the device time of the current
+ * policy's rows, improve_ms includes recomputing every row. */
 int pi_get_stats(const pi_engine* e, pi_stats* stats);
 
 /* Evaluation-sweep kernel selection (new; no reference counterpart).  At pi_build_table the

@@ -2,11 +2,12 @@
 """One sweep family on a small grid, for compute-sanitizer (tests/test_gpu_sanitizer.py):
     compute-sanitizer --tool memcheck --error-exitcode 1 python scripts/sanitize_target.py <family>
 families: aot | gp_single | gp_pair | xline | persistent | plane | plane_small | plane_scalar | plane_items_small | lookup |
-          rollout | odd_aot5 | odd_xline3 | odd_plane5 | warm_start
+          rollout | odd_aot5 | odd_xline3 | odd_plane5 | warm_start | recompute
 warm_start prolongs a coarser and a finer source value function onto an engine with a terminal mask (the overhead
 crane, whose goal states also carry values from set_values) and runs an improvement and sweeps from it.
 The odd_* families run the chain-of-integrators fixture of tests/fixtures/odd_dims.py at D = 3 or 5 (rows with an odd
-number of words)."""
+number of words).  recompute runs the same steps with DPB200_TABLE=recompute (pi_improve_recompute, pi_policy_rows and
+the per-action row builds of expand_rows)."""
 import importlib.util
 import os
 import sys
@@ -32,6 +33,7 @@ cfg = {
     "odd_xline3": {"DPB200_PLANE": "off", "DPB200_FAST_DIM": "0", "DPB200_XLINE": "force:2,0,4,8,2,1:1,1"},
     "odd_plane5": {"DPB200_FAST_DIM": "0,1", "DPB200_PLANE": "force:0,0,2,2,2"},
     "warm_start": {},
+    "recompute": {"DPB200_TABLE": "recompute"},
 }[family]
 os.environ.update(cfg)
 os.environ["DPB200_CACHE"] = "off"
@@ -55,7 +57,7 @@ info = eng.eval_kernel_info()["kernel"]
 want = {"aot": "eval_sweep_kernel", "gp_single": "gp_sweep", "gp_pair": "gp_sweep", "xline": "xl_sweep",
         "persistent": "eval_persistent_kernel", "plane": "ps_sweep", "plane_small": "ps_sweep", "plane_scalar": "ps_sweep", "plane_items_small": "ps_sweep", "lookup": "", "rollout": "",
         "odd_aot5": "eval_sweep_kernel<5>", "odd_xline3": "xl_sweep", "odd_plane5": "ps_sweep",
-        "warm_start": ""}[family]
+        "warm_start": "", "recompute": ""}[family]
 assert want in info, (family, info)
 eng.sweeps(3)
 eng.policy_improvement()
@@ -78,6 +80,9 @@ if family == "warm_start":   # pi_prolong_values from a coarser and a finer sour
         src = np.random.default_rng(b).standard_normal(n).astype(np.float32)
         eng.warm_start((src, eng.bounds_low, eng.bounds_high, np.full(eng.N_DIMS, b)))
         eng.sweeps(3)
+if family == "recompute":
+    assert eng.engine_stats()["table_mode"] == "recompute"
+    eng.expand_rows(eng.n_actions - 1, eng.n_states // 3, 1000)
 v, p = eng.download()
 assert np.isfinite(v).all()
 eng.close()
