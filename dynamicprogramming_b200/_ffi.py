@@ -129,6 +129,8 @@ SIGNATURES = {
                                  C.POINTER(C.c_int64), C.POINTER(C.c_double), C.POINTER(C.c_int32)]),
     "pi_debug_xline": (C.c_int, [C.c_void_p, C.c_char_p, C.c_int32, C.POINTER(C.c_float), C.POINTER(C.c_float),
                                  C.POINTER(C.c_int64), C.POINTER(C.c_double), C.POINTER(C.c_int32)]),
+    "pi_debug_plane_schedule": (C.c_int, [C.c_void_p, C.c_char_p, C.c_int32, C.c_int32, C.POINTER(C.c_int64), C.POINTER(C.c_double),
+                                          C.POINTER(C.c_int32), C.POINTER(C.c_int32), C.c_int64, C.c_void_p, C.c_int64]),
 }
 
 _lib = None

@@ -16,8 +16,10 @@
 //     gather from global memory in the sweep.
 //
 // Two passes: plane_cells_kernel (one CTA per state-plane, fully parallel, memory-bound) finds the cells and writes
-// the code words; plane_slots_kernel (one warp per chunk of `L` consecutive state-planes, sequential over the chunk
-// because the slot state of step i depends on step i-1) assigns slots and writes the load lists.
+// the code words; plane_slots_kernel (one warp per chunk of consecutive state-planes, sequential over the chunk
+// because the slot state of step i depends on step i-1) assigns slots and writes the load lists.  Every chunk is planned
+// as if it started cold; plane_stitch_kernel and plane_relabel_kernel then renumber the slots of each chunk so that the
+// first step's loads go to slots the CTA's previous chunk no longer reads, and issue those loads one step ahead too.
 #pragma once
 
 #include <cuda_runtime.h>
@@ -51,6 +53,29 @@ struct PlaneCells {
 };
 static_assert(sizeof(PlaneCells) == 64, "PlaneCells layout");
 
+// First state-plane of chunk c (== ps_chunk_begin in plane_sweep_src.cuh).  The sweep's G persistent CTAs take chunks
+// c, c + G, ... of n_chunks = k G: the first n_full = (k - 1) G chunks have exactly L planes (whole lines of the fastest
+// outer dimension: consecutive planes share their V-planes), the last G chunks split the rest evenly, so that every CTA
+// sweeps the same number of planes to within one.
+__host__ __device__ __forceinline__ long long plan_chunk_begin(long long c, int L, int n_full, int n_chunks, int n_planes) {
+    if (c <= n_full) return c * L;
+    const long long base = (long long)n_full * L;
+    return base + (c - n_full) * (n_planes - base) / (n_chunks - n_full);
+}
+
+// Per chunk: the slots its first step loads and the slots its last step reads (bit s of 128 = slot s), written by
+// plane_slots_kernel; and the renumbering plane_stitch_kernel chose for it.
+struct ChunkSlots {
+    unsigned first[4];
+    unsigned last[4];
+};
+struct ChunkStitch {
+    unsigned busy[4];                        // slots (new numbers) the previous chunk of the same CTA reads in its last step
+    unsigned char perm[kPlanMaxSlots];       // planned slot -> slot
+    int relabel;                             // 0: the CTA's first chunk, kept as planned
+    int pad[3];
+};
+
 struct PlanParams {
     const unsigned char* rows;   // the policy's rows; plane 0 = [base, f0, f1, f2] per state (16 B)
     unsigned char* prow0;        // out: [code, f0, f1, f2]
@@ -58,10 +83,14 @@ struct PlanParams {
     PlaneCells* cells;           // scratch: one per local state-plane (written by plane_cells_kernel)
     unsigned long long* stats;   // out (atomic): [0] plane loads, [1] late loads, [2] fallback states, [3] live states,
                                  //               [4] staged cells, [5] state-planes
+    ChunkSlots* chunk_slots;     // out: one per chunk
+    ChunkStitch* stitch;         // one per chunk (plane_stitch_kernel -> plane_relabel_kernel)
     int n_planes;                // local state-planes
-    int pl_begin;                // this launch plans the state-planes [pl_begin, pl_end) (pl_begin a multiple of L): a policy upload
-    int pl_end;                  // is planned range by range while the rest is still on its way (pi_upload_policy_local)
-    int L;                       // state-planes per chunk
+    int pl_begin;                // this launch plans the state-planes [pl_begin, pl_end) = the chunks [c_begin, c_end): a policy
+    int pl_end;                  // upload is planned range by range while the rest is still on its way (pi_upload_policy_local)
+    int c_begin, c_end;
+    int L, n_full, n_chunks;     // chunk geometry (plan_chunk_begin)
+    int grid, rot;               // the sweep's schedule: CTA b takes the chunks (b + rot), (b + G + rot), ... mod n_chunks
     int P;                       // states per plane
     int NS;                      // shared-memory slots of the sweep
     int noc;                     // outer corners per cell (power of two)
@@ -549,10 +578,10 @@ __global__ void __launch_bounds__(kSlotWarps * 32) plane_slots_kernel(const Plan
     __shared__ int s_cs[kSlotWarps][kPlanMaxCells * kPlanMaxOC];
     __shared__ unsigned s_early[kSlotWarps][kPlanMaxLoads], s_late[kSlotWarps][kPlanMaxLoads];
     const int lane = threadIdx.x & 31, wq = threadIdx.x >> 5;
-    const int chunk = q.pl_begin / q.L + blockIdx.x * kSlotWarps + wq;
-    const int pl0 = chunk * q.L;
-    if (pl0 >= q.pl_end) return;
-    const int Lc = min(q.L, q.n_planes - pl0);
+    const int chunk = q.c_begin + blockIdx.x * kSlotWarps + wq;
+    if (chunk >= q.c_end) return;
+    const int pl0 = (int)plan_chunk_begin(chunk, q.L, q.n_full, q.n_chunks, q.n_planes);
+    const int Lc = (int)plan_chunk_begin(chunk + 1, q.L, q.n_full, q.n_chunks, q.n_planes) - pl0;
     int* slot_vp = s_slot_vp[wq];
     int* slot_used = s_slot_used[wq];
     int* cs = s_cs[wq];
@@ -602,7 +631,7 @@ __global__ void __launch_bounds__(kSlotWarps * 32) plane_slots_kernel(const Plan
                 const unsigned ml = __ballot_sync(0xffffffffu, best_late >= 0);
                 int slot = -1, kind = 0;   // kind 1: early, 2: late
                 if (mm) slot = __shfl_sync(0xffffffffu, mine, __ffs(mm) - 1);
-                else if (me) { slot = __shfl_sync(0xffffffffu, best_early, __ffs(me) - 1); kind = i > 0 ? 1 : 2; }   // first plane of a chunk: nothing was issued ahead
+                else if (me) { slot = __shfl_sync(0xffffffffu, best_early, __ffs(me) - 1); kind = i > 0 ? 1 : 2; }   // first plane of a chunk: late until stitched
                 else if (ml) { slot = __shfl_sync(0xffffffffu, best_late, __ffs(ml) - 1); kind = 2; }
                 if (slot < 0 || (kind && n_early + n_late >= kPlanMaxLoads)) {
                     bad |= 1u << k;
@@ -642,6 +671,26 @@ __global__ void __launch_bounds__(kSlotWarps * 32) plane_slots_kernel(const Plan
             rec->cs[k][j] = v;
         }
         for (int t = lane; t < n_early + n_late; t += 32) rec->loads[t] = t < n_early ? early[t] : late[t - n_early];
+        // what plane_stitch_kernel works with: the slots the first step loads (all of its loads are late so far), and the
+        // slots the last step reads or loads (slot_used == i: also the planes of a cell that was given up half-way)
+        if (i == 0) {
+            unsigned m[4] = {0u, 0u, 0u, 0u};
+            for (int t = lane; t < n_early + n_late; t += 32) {
+                const unsigned s = (t < n_early ? early[t] : late[t - n_early]) >> 24;
+                m[s >> 5] |= 1u << (s & 31);
+            }
+#pragma unroll
+            for (int w = 0; w < 4; ++w) m[w] = __reduce_or_sync(0xffffffffu, m[w]);
+            if (lane < 4) q.chunk_slots[chunk].first[lane] = m[lane];
+        }
+        if (i == Lc - 1) {
+            unsigned m[4] = {0u, 0u, 0u, 0u};
+            for (int s = lane; s < q.NS; s += 32)
+                if (slot_used[s] == i) m[s >> 5] |= 1u << (s & 31);
+#pragma unroll
+            for (int w = 0; w < 4; ++w) m[w] = __reduce_or_sync(0xffffffffu, m[w]);
+            if (lane < 4) q.chunk_slots[chunk].last[lane] = m[lane];
+        }
         a_loads += (unsigned long long)(n_early + n_late);
         a_late += (unsigned long long)n_late;
         a_fb += (unsigned long long)pc.n_unstaged;
@@ -660,6 +709,148 @@ __global__ void __launch_bounds__(kSlotWarps * 32) plane_slots_kernel(const Plan
         atomicAdd(q.stats + 3, a_live);
         atomicAdd(q.stats + 4, a_cells);
         atomicAdd(q.stats + 5, (unsigned long long)Lc);
+    }
+}
+
+// Pass 3 — one WARP per CTA of the sweep, sequential over that CTA's chunks (the numbering of a chunk depends on the one
+// before it): a chunk's first step loads every plane it reads, into slots numbered as if the chunk started cold.  A slot
+// renumbering (a bijection: inside the chunk every load keeps its early / late kind) moves as many of those loads as
+// possible into slots the CTA's previous chunk neither reads nor loads in its last step; the sweep issues them one step
+// ahead, as inside a chunk.  The CTA's first chunk keeps its numbering and has no early loads there.
+__device__ __forceinline__ int plan_rank(const unsigned (&m)[4], int s) {   // set bits of m below bit s
+    int r = 0;
+#pragma unroll
+    for (int w = 0; w < 4; ++w) r += 32 * w + 32 <= s ? __popc(m[w]) : 32 * w < s ? __popc(m[w] & ((1u << (s - 32 * w)) - 1u)) : 0;
+    return r;
+}
+__device__ __forceinline__ int plan_select(const unsigned (&m)[4], int j) {   // bit number of the j-th set bit of m
+#pragma unroll
+    for (int w = 0; w < 4; ++w) {
+        unsigned x = m[w];
+        const int c = __popc(x);
+        if (j < c) {
+            for (; j > 0; --j) x &= x - 1u;
+            return 32 * w + __ffs(x) - 1;
+        }
+        j -= c;
+    }
+    return -1;
+}
+__global__ void __launch_bounds__(kSlotWarps * 32) plane_stitch_kernel(const PlanParams q) {
+    constexpr int kPer = (kPlanMaxSlots + 31) / 32;
+    const int lane = threadIdx.x & 31;
+    const int b = blockIdx.x * kSlotWarps + (threadIdx.x >> 5);
+    if (b >= q.grid) return;
+    unsigned valid[4];
+#pragma unroll
+    for (int w = 0; w < 4; ++w) valid[w] = q.NS >= 32 * w + 32 ? 0xffffffffu : q.NS > 32 * w ? (1u << (q.NS - 32 * w)) - 1u : 0u;
+    int perm[kPer];   // numbering of the previous chunk: slot lane + 32 w -> perm[w]
+    int prev = -1;
+    for (int ci = b; ci < q.n_chunks; ci += q.grid) {
+        const int c = ci + q.rot < q.n_chunks ? ci + q.rot : ci + q.rot - q.n_chunks;
+        ChunkStitch* st = q.stitch + c;
+        unsigned busy[4] = {0u, 0u, 0u, 0u};
+        if (prev < 0) {
+#pragma unroll
+            for (int w = 0; w < kPer; ++w) perm[w] = lane + 32 * w;
+        } else {
+            const ChunkSlots cp = q.chunk_slots[prev], cc = q.chunk_slots[c];
+#pragma unroll
+            for (int w = 0; w < kPer; ++w) {
+                const int s = lane + 32 * w;
+                if (s < q.NS && ((cp.last[w] >> lane) & 1u)) busy[perm[w] >> 5] |= 1u << (perm[w] & 31);
+            }
+            unsigned fr[4];
+#pragma unroll
+            for (int w = 0; w < 4; ++w) {
+                busy[w] = __reduce_or_sync(0xffffffffu, busy[w]);
+                fr[w] = ~busy[w] & valid[w];
+            }
+            // planned order: the first step's loads, then the other slots; target order: free slots, then busy ones
+            int n_t = 0, n_free = 0;
+#pragma unroll
+            for (int w = 0; w < 4; ++w) { n_t += __popc(cc.first[w] & valid[w]); n_free += __popc(fr[w]); }
+#pragma unroll
+            for (int w = 0; w < kPer; ++w) {
+                const int s = lane + 32 * w;
+                if (s >= q.NS) continue;
+                const int r = plan_rank(cc.first, s);
+                const int j = ((cc.first[w] >> lane) & 1u) ? r : n_t + (s - r);
+                perm[w] = j < n_free ? plan_select(fr, j) : plan_select(busy, j - n_free);
+            }
+        }
+        if (lane < 4) st->busy[lane] = busy[lane];
+#pragma unroll
+        for (int w = 0; w < kPer; ++w)
+            if (lane + 32 * w < kPlanMaxSlots) st->perm[lane + 32 * w] = (unsigned char)perm[w];
+        if (lane == 0) st->relabel = prev >= 0;
+        prev = c;
+    }
+}
+
+// Pass 4 — one CTA per chunk: apply plane_stitch_kernel's numbering to the chunk's slot offsets and load lists; the loads
+// of the first step whose new slot the previous chunk does not touch become early (listed first).
+constexpr int kRelabelThreads = 128;
+__global__ void __launch_bounds__(kRelabelThreads) plane_relabel_kernel(const PlanParams q) {
+    __shared__ unsigned char perm[kPlanMaxSlots];
+    __shared__ unsigned busy[4];
+    const int c = blockIdx.x, tid = threadIdx.x, lane = tid & 31;
+    const ChunkStitch* st = q.stitch + c;
+    if (!st->relabel) return;
+    if (tid < kPlanMaxSlots) perm[tid] = st->perm[tid];
+    if (tid < 4) busy[tid] = st->busy[tid];
+    __syncthreads();
+    const int pl0 = (int)plan_chunk_begin(c, q.L, q.n_full, q.n_chunks, q.n_planes);
+    const int pl1 = (int)plan_chunk_begin(c + 1, q.L, q.n_full, q.n_chunks, q.n_planes);
+    const unsigned unit = (unsigned)q.pitch / 4u;   // slot offset entry = slot * pitch * 4 / 16
+    for (int pl = pl0; pl < pl1; ++pl) {
+        PlaneRec* r = q.plan + pl;
+        const unsigned hdr = *reinterpret_cast<const unsigned*>(r);
+        const int K = (hdr >> 16) & 0xff, flags = hdr >> 24, n = (hdr & 0xff) + ((hdr >> 8) & 0xff);
+        for (int t = tid; t < kPlanMaxCells * kPlanMaxOC; t += kRelabelThreads) {
+            const int k = t / kPlanMaxOC, j = t % kPlanMaxOC;
+            if (k < K && j < q.noc && !((flags >> k) & 1)) r->cs[k][j] = (unsigned short)(perm[r->cs[k][j] / unit] * unit);
+        }
+        if (pl > pl0) {
+            for (int t = tid; t < n; t += kRelabelThreads) {
+                const unsigned e = r->loads[t];
+                r->loads[t] = ((unsigned)perm[e >> 24] << 24) | (e & 0xffffffu);
+            }
+        } else if (tid < 32) {
+            constexpr int kPer = (kPlanMaxLoads + 31) / 32;
+            unsigned e[kPer];
+            bool early[kPer];
+            unsigned me[kPer];
+            int n_early = 0;
+#pragma unroll
+            for (int w = 0; w < kPer; ++w) {
+                const int t = lane + 32 * w;
+                e[w] = 0u;
+                early[w] = false;
+                if (t < n) {
+                    const unsigned s = perm[r->loads[t] >> 24];
+                    e[w] = (s << 24) | (r->loads[t] & 0xffffffu);
+                    early[w] = !((busy[s >> 5] >> (s & 31)) & 1u);
+                }
+                me[w] = __ballot_sync(0xffffffffu, t < n && early[w]);
+                n_early += __popc(me[w]);
+            }
+            __syncwarp();
+            int before_e = 0;
+#pragma unroll
+            for (int w = 0; w < kPer; ++w) {
+                const int t = lane + 32 * w;
+                const int re = before_e + __popc(me[w] & ((1u << lane) - 1u));   // early loads before this one
+                if (t < n) r->loads[early[w] ? re : n_early + (t - re)] = e[w];
+                before_e += __popc(me[w]);
+            }
+            if (lane == 0) {
+                r->n_early = (unsigned char)n_early;
+                r->n_late = (unsigned char)(n - n_early);
+                atomicAdd(q.stats + 1, 0ull - (unsigned long long)n_early);
+            }
+        }
+        __syncthreads();
     }
 }
 

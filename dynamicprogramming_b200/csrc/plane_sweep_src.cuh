@@ -6,7 +6,7 @@
 //
 //   * the two fastest-stored dimensions (f0 fastest, f1 next) span a "V-plane" of PS_P = n_f0 * n_f1
 //     floats that is contiguous and 16-byte aligned in HBM; the other D-2 dimensions enumerate planes;
-//   * one CTA walks a chunk of PS_L consecutive state-planes.  All states of a plane that take the same
+//   * one CTA walks chunks of consecutive state-planes.  All states of a plane that take the same
 //     action land in the same cell of the outer dimensions when the dynamics are translation-invariant
 //     in f0/f1 (cart position and velocity: every cart-pole environment), so a state-plane needs only a
 //     handful of V-planes: 2^(D-2) corner planes per distinct successor cell;
@@ -36,7 +36,7 @@
 // (value kept) ride along with pair items.
 //
 // The host prepends (dpb200.cu: plane_preamble):
-//   PS_D, PS_P, PS_NS, PS_THREADS (consumer threads = PS_P rounded up to a warp), PS_MINB, PS_L, PS_LV,
+//   PS_D, PS_P, PS_NS, PS_THREADS (consumer threads = PS_P rounded up to a warp), PS_MINB, PS_LV,
 //   PS_PACK, PS_N0 (extent of the fastest dimension), ps_cj[2^D] (outer-corner number of corner c), ps_imm[2^D] (in-plane float offset of corner c),
 //   gp_off[2^D] (global V offset of corner c, fallback path).
 
@@ -88,18 +88,32 @@ struct PsParams {
     long long n_pad;
     long long s_begin;
     int n_planes;                // local state-planes
-    int n_chunks;
+    int n_chunks;                // chunks of the schedule (ps_chunk_begin): n_full of exactly L planes, then gridDim.x uneven ones
+    int L;
+    int n_full;
     int chunk_rot;               // sharded runs: chunk visited first (the chunks whose values peers need go first, so their NVLink
                                  // stores drain while the interior is swept); 0 on one GPU
     int n_peer_chunks;           // ... and how many chunks from there on can hold states a peer needs (the rest is interior)
-    int sched_begin;             // this launch sweeps the chunks [sched_begin, sched_end) of the (rotated) schedule: sharded runs with
-    int sched_end;               // the DMA exchange launch the boundary part and the interior part separately
+    int sched_begin;             // this launch sweeps the chunks [sched_begin, sched_end) of the (rotated) schedule; CTA b takes
+    int sched_end;               // sched_begin + b, sched_begin + b + gridDim.x, ... (the sequence the plan was stitched for)
     int partial_off;             // first slot of p.partial this launch writes
     float gamma;
     int j;
     int check;
     PsPeerOut peers;
 };
+
+// first state-plane of chunk c (== pi::plan_chunk_begin in plane_plan.cuh): n_full chunks of L planes, then the rest split
+// evenly over the last n_chunks - n_full
+__device__ __forceinline__ int ps_chunk_begin(const PsParams& p, int c) {
+    if (c <= p.n_full) return c * p.L;
+    const int base = p.n_full * p.L;
+    return base + (int)((long long)(c - p.n_full) * (p.n_planes - base) / (p.n_chunks - p.n_full));
+}
+// chunk visited at schedule position ci
+__device__ __forceinline__ int ps_chunk_at(const PsParams& p, int ci) {
+    return ci + p.chunk_rot < p.n_chunks ? ci + p.chunk_rot : ci + p.chunk_rot - p.n_chunks;
+}
 
 #define PS_W (PS_D + 2)
 #define PS_N4 (PS_W / 4)
@@ -469,21 +483,34 @@ extern "C" __global__ void __launch_bounds__(PS_THREADS + 32, PS_MINB) ps_sweep(
             }
             __syncwarp();
         };
+        // The CTA's steps run on across its chunks: the record of the step after next is fetched, and the next step's early
+        // loads are issued, also when that step is the first of the next chunk (the planner stitched the chunks for this
+        // sequence).  Only the first step of the launch issues all of its loads itself.
         bool armed = false;   // full[it & 1] was already armed one step ahead
+        int f_ci = p.sched_begin + blockIdx.x, f_pl = 0, f_end = 0;   // fetch cursor: the step whose record is fetched next
+        if (f_ci < p.sched_end) { f_pl = ps_chunk_begin(p, ps_chunk_at(p, f_ci)); f_end = ps_chunk_begin(p, ps_chunk_at(p, f_ci) + 1); }
+        auto fetch_next = [&](Fetched& f) {
+            if (f_ci >= p.sched_end) return;
+            fetch_rec(p.plan + f_pl, f);
+            if (++f_pl == f_end) {
+                f_ci += gridDim.x;
+                if (f_ci < p.sched_end) { f_pl = ps_chunk_begin(p, ps_chunk_at(p, f_ci)); f_end = ps_chunk_begin(p, ps_chunk_at(p, f_ci) + 1); }
+            }
+        };
+        Fetched cur, nxt, nn;
+        fetch_next(cur);
+        nxt = cur;
+        fetch_next(nxt);
+        nn = nxt;
         for (int ci = p.sched_begin + blockIdx.x; ci < p.sched_end; ci += gridDim.x) {
-            const int chunk = ci + p.chunk_rot < p.n_chunks ? ci + p.chunk_rot : ci + p.chunk_rot - p.n_chunks;
-            const int pl0 = chunk * PS_L;
-            const int Lc = (p.n_planes - pl0) < PS_L ? (p.n_planes - pl0) : PS_L;
-            const PsRec* rec = p.plan + pl0;
-            Fetched cur, nxt, nn;
-            fetch_rec(rec, cur);
-            nxt = cur;
-            if (Lc > 1) fetch_rec(rec + 1, nxt);
-            nn = nxt;
+            const int chunk = ps_chunk_at(p, ci);
+            const int pl0 = ps_chunk_begin(p, chunk);
+            const int Lc = ps_chunk_begin(p, chunk + 1) - pl0;
+            const bool next_chunk = ci + (int)gridDim.x < p.sched_end;
             for (int i = 0; i < Lc; ++i, ++it) {
-                const bool more = i + 1 < Lc;
+                const bool more = i + 1 < Lc || next_chunk;
                 const unsigned b = it & 1;
-                if (i + 2 < Lc) fetch_rec(rec + i + 2, nn);   // in flight while this warp waits for the consumers
+                fetch_next(nn);   // in flight while this warp waits for the consumers
 #if PS_ROW_PF > 0
                 // The consumers load the rows of a plane one step before they use them — less than a DRAM round trip once a step
                 // takes about a microsecond (ncu: 21 % of the warp samples waited for those loads).  One bulk L2 prefetch per plane,
@@ -491,12 +518,11 @@ extern "C" __global__ void __launch_bounds__(PS_THREADS + 32, PS_MINB) ps_sweep(
                 if (lane == 0) {
                     int pf_pl = pl0 + i + PS_ROW_PF;
                     if (i + PS_ROW_PF >= Lc) {
-                        const int cn = ci + (int)gridDim.x;
                         pf_pl = -1;
-                        if (cn < p.sched_end) {
-                            const int chn = cn + p.chunk_rot < p.n_chunks ? cn + p.chunk_rot : cn + p.chunk_rot - p.n_chunks;
-                            pf_pl = chn * PS_L + (i + PS_ROW_PF - Lc);
-                            if (pf_pl >= p.n_planes) pf_pl = -1;
+                        if (next_chunk) {
+                            const int chn = ps_chunk_at(p, ci + (int)gridDim.x);
+                            pf_pl = ps_chunk_begin(p, chn) + (i + PS_ROW_PF - Lc);
+                            if (pf_pl >= ps_chunk_begin(p, chn + 1)) pf_pl = -1;
                         }
                     }
                     if (pf_pl >= 0) {
@@ -514,7 +540,7 @@ extern "C" __global__ void __launch_bounds__(PS_THREADS + 32, PS_MINB) ps_sweep(
 #if PS_PF_AHEAD > 0
                 // optional (off by default, see PS_PF_AHEAD): pull the planes of a later step into L2 now
                 if (i + PS_PF_AHEAD < Lc) {
-                    const PsRec* rp = rec + i + PS_PF_AHEAD;
+                    const PsRec* rp = p.plan + pl0 + i + PS_PF_AHEAD;
                     const unsigned np = (unsigned)rp->n_early + rp->n_late;
                     for (unsigned q = lane; q < np; q += 32)
                         ps_bulk_prefetch_l2(Vin + (size_t)(rp->loads[q] & 0xffffffu) * PS_P, PS_PLANE_BYTES);
@@ -527,14 +553,16 @@ extern "C" __global__ void __launch_bounds__(PS_THREADS + 32, PS_MINB) ps_sweep(
                 if (prev_g0 >= 0) store_plane(it - 1, prev_g0);
                 prev_g0 = p.s_begin + (long long)(pl0 + i) * PS_P;
                 if (!armed) {
+                    // the first step of the launch: nothing was issued ahead, its early loads go out now too
+                    const unsigned first = it == 0 ? 0u : ne, n = it == 0 ? ne + nl : nl;
                     stage_cs_regs(cur.cs, b);
                     __syncwarp();
                     if (lane == 0) {
-                        if (nl) ps_mbar_arrive_expect(&full[b], nl * (unsigned)PS_PLANE_BYTES);
+                        if (n) ps_mbar_arrive_expect(&full[b], n * (unsigned)PS_PLANE_BYTES);
                         else ps_mbar_arrive(&full[b]);
                     }
                     __syncwarp();
-                    copies(cur, ne, nl, &full[b]);
+                    copies(cur, first, n, &full[b]);
                 }
                 armed = false;
                 if (more) {
@@ -564,12 +592,14 @@ extern "C" __global__ void __launch_bounds__(PS_THREADS + 32, PS_MINB) ps_sweep(
     } else {
         // ------------------------------------------------------------------ consumer warps
 #if PS_PACK == 2
+        // the item of the CTA's next step is in flight while this one is backed up, across chunk boundaries too
+        unsigned u[4 * PS_NQ];
+        if (p.sched_begin + (int)blockIdx.x < p.sched_end) ps_load_item(p, ps_chunk_begin(p, ps_chunk_at(p, p.sched_begin + blockIdx.x)), tid, u);
         for (int ci = p.sched_begin + blockIdx.x; ci < p.sched_end; ci += gridDim.x) {
-            const int chunk = ci + p.chunk_rot < p.n_chunks ? ci + p.chunk_rot : ci + p.chunk_rot - p.n_chunks;
-            const int pl0 = chunk * PS_L;
-            const int Lc = (p.n_planes - pl0) < PS_L ? (p.n_planes - pl0) : PS_L;
-            unsigned u[4 * PS_NQ];
-            ps_load_item(p, pl0, tid, u);
+            const int chunk = ps_chunk_at(p, ci);
+            const int pl0 = ps_chunk_begin(p, chunk);
+            const int Lc = ps_chunk_begin(p, chunk + 1) - pl0;
+            const int pl_next = ci + (int)gridDim.x < p.sched_end ? ps_chunk_begin(p, ps_chunk_at(p, ci + (int)gridDim.x)) : -1;
             for (int i = 0; i < Lc; ++i, ++it) {
                 const unsigned b = it & 1;
                 const long long sp = (long long)(pl0 + i) * PS_P;   // first local state of the plane
@@ -590,6 +620,7 @@ extern "C" __global__ void __launch_bounds__(PS_THREADS + 32, PS_MINB) ps_sweep(
                 const float ra = __uint_as_float(u[PS_D + 1]), rb = __uint_as_float(u[PS_W + PS_D + 1]);
                 // the next plane's item: in flight while this one is backed up
                 if (i + 1 < Lc) ps_load_item(p, pl0 + i + 1, tid, u);
+                else if (pl_next >= 0) ps_load_item(p, pl_next, tid, u);
                 const unsigned kinda = PS_KIND(ca), kindb = PS_KIND(cb);
                 const unsigned pa = ca & 0xfffu, pb = cb & 0xfffu;
                 float volda = 0.0f, voldb = 0.0f, vpass = 0.0f;
@@ -650,12 +681,15 @@ extern "C" __global__ void __launch_bounds__(PS_THREADS + 32, PS_MINB) ps_sweep(
             }
         }
 #else
+        // the row of the CTA's next step is in flight while this one is backed up, across chunk boundaries too
+        unsigned w[PS_W];
+        if (has_state && p.sched_begin + (int)blockIdx.x < p.sched_end)
+            ps_load_row(p, (long long)ps_chunk_begin(p, ps_chunk_at(p, p.sched_begin + blockIdx.x)) * PS_P + tid, w);
         for (int ci = p.sched_begin + blockIdx.x; ci < p.sched_end; ci += gridDim.x) {
-            const int chunk = ci + p.chunk_rot < p.n_chunks ? ci + p.chunk_rot : ci + p.chunk_rot - p.n_chunks;
-            const int pl0 = chunk * PS_L;
-            const int Lc = (p.n_planes - pl0) < PS_L ? (p.n_planes - pl0) : PS_L;
-            unsigned w[PS_W];
-            if (has_state) ps_load_row(p, (long long)pl0 * PS_P + tid, w);
+            const int chunk = ps_chunk_at(p, ci);
+            const int pl0 = ps_chunk_begin(p, chunk);
+            const int Lc = ps_chunk_begin(p, chunk + 1) - pl0;
+            const int pl_next = ci + (int)gridDim.x < p.sched_end ? ps_chunk_begin(p, ps_chunk_at(p, ci + (int)gridDim.x)) : -1;
             for (int i = 0; i < Lc; ++i, ++it) {
                 const unsigned b = it & 1;
                 const long long s = (long long)(pl0 + i) * PS_P + tid;   // local state
@@ -670,6 +704,7 @@ extern "C" __global__ void __launch_bounds__(PS_THREADS + 32, PS_MINB) ps_sweep(
                 const float reward = __uint_as_float(w[PS_D + 1]);
                 // the next plane's row: in flight while this plane is backed up
                 if (i + 1 < Lc && has_state) ps_load_row(p, s + PS_P, w);
+                else if (pl_next >= 0 && has_state) ps_load_row(p, (long long)pl_next * PS_P + tid, w);
                 float vold = 0.0f;
                 if (has_state && (p.check || code == -2)) vold = Vin[g];
 

@@ -649,6 +649,23 @@ class _CudaPolicyIterationBase(abc.ABC):
                 "pairs_per_plane": st[4], "stray_pairs_per_plane": st[5], "singles_paired_per_plane": st[6], "registers": int(info[0]), "grid": int(info[1]), "block": int(info[2]), "smem": int(info[3]),
                 "slots": int(info[4]), "chunk": int(info[5])}
 
+    def debug_plane_schedule(self, cfg: str = "", rot: int = -1, iters: int = 1) -> dict:
+        """Test hook: as debug_plane, with the plan stitched for the chunk rotation `rot` (-1: the engine's own); also
+        returns the schedule (`chunk_begin`: first state-plane of every chunk and the end) and the plan records
+        (`records`: one row of bytes per local state-plane, the layout of pi::PlaneRec)."""
+        mism, st, sched = C.c_int64(), (C.c_double * 8)(), (C.c_int32 * 8)()
+        lib = _ffi.lib()
+        _ffi.check(lib.pi_debug_plane_schedule(self._engine, cfg.encode(), int(rot), 0, None, None, sched, None, 0, None, 0))
+        n_planes, n_chunks, rec_bytes = int(sched[0]), int(sched[1]), int(sched[7])
+        begin = np.zeros(n_chunks + 1, np.int32)
+        records = np.zeros((n_planes, rec_bytes), np.uint8)
+        _ffi.check(lib.pi_debug_plane_schedule(self._engine, cfg.encode(), int(rot), int(iters), C.byref(mism), st, sched,
+                                               begin.ctypes.data_as(C.POINTER(C.c_int32)), begin.size,
+                                               records.ctypes.data_as(C.c_void_p), records.nbytes))
+        return {"mismatches": int(mism.value), "loads_per_plane": st[0], "late_per_plane": st[1], "fallback_frac": st[3],
+                "n_planes": n_planes, "n_chunks": n_chunks, "grid": int(sched[2]), "rot": int(sched[3]), "slots": int(sched[4]),
+                "pitch": int(sched[5]), "noc": int(sched[6]), "chunk_begin": begin, "records": records}
+
     def debug_xline(self, cfg: str, iters: int = 5) -> dict:
         """Test hook: run the x-line sweep configuration `cfg` and the scalar sweep on the current
         rows and V; returns timings and the number of differing V words (must be 0)."""

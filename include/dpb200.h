@@ -268,6 +268,14 @@ int pi_debug_xline(pi_engine* e, const char* cfg, int32_t iters, float* ms_xline
 int pi_debug_plane(pi_engine* e, const char* cfg, int32_t iters, float* ms_plane, float* ms_base, int64_t* mismatches,
                    double* stats, int32_t* info);
 
+/* Test hook: as pi_debug_plane, with the plan stitched for the chunk rotation `rot` (-1: the engine's own, 0 on one GPU),
+ * and the schedule and plan it ran.  sched = {state-planes, chunks, grid, rotation, slots, slot pitch in floats, outer
+ * corners per cell, bytes per plan record} — EIGHT int32; chunk_begin (>= chunks + 1 entries, or null) = first state-plane
+ * of every chunk and the end; records (or null) = the plan records of every local state-plane, as the sweep reads them.
+ * CTA b of the sweep takes the chunks (b + rot) mod chunks, (b + grid + rot) mod chunks, ... */
+int pi_debug_plane_schedule(pi_engine* e, const char* cfg, int32_t rot, int32_t iters, int64_t* mismatches, double* stats,
+                            int32_t* sched, int32_t* chunk_begin, int64_t chunk_cap, void* records, int64_t record_cap);
+
 /* Test hook for the JIT sweeps of csrc/pair_sweep_src.cuh (grid strides as immediates): compiles the
  * configuration (threads per block, blocks per SM, lean weight-tree levels 1..3, gathers per explicitly
  * scheduled group or 0, single = 1: one state per thread / 0: two states per thread with packed f32x2
