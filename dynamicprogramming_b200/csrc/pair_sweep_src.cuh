@@ -20,6 +20,8 @@
 //   GP_G        gathers per explicitly scheduled group (0: leave the schedule to ptxas)
 //   gp_off[]    V offset of corner c: sum of the storage strides of the set bits (bit d <-> dim d)
 //
+// and then sweep_common_src.cuh (pi::GpParams, pi::Ctl, pi::load_row, the shared device helpers).
+//
 // Why the packed form (DESIGN.md §5).  The scalar sweep (pi::eval_sweep_kernel) spends 2^D scalar FMUL for the
 // leaf weights, 2^D-4 for the tree, 2^D FFMA for the chain and ~2^D IMAD for the gather
 // addresses per state — all on the FMA pipe, where a 3-register FFMA/FMUL/IMAD issues at half
@@ -34,55 +36,7 @@
 
 typedef unsigned long long gp_u64;
 
-struct GpCtl {   // == pi::Ctl
-    int base, parity0, done, conv_sweep;
-    float last_delta, check_delta;
-    unsigned long long changed;
-    unsigned int pad[8];
-};
-
-
-// == pi::PeerOut (pi_kernels.cuh): sharded runs store new values straight into the V buffers of the
-// ranks that need them (CUDA IPC peer pointers over NVLink); n == 0 otherwise.
-struct GpPeerOut {
-    int n;
-    int pad;
-    float* V0[7];
-    float* V1[7];
-    long long lo[7];
-    long long hi[7];
-};
-// unrolled over the 7 entries: a run-time-indexed loop over a kernel-parameter struct is compiled into local-memory copies
-__device__ __forceinline__ void gp_store_peers(const GpPeerOut& po, bool out_is_V0, long long g, float v) {
-#pragma unroll
-    for (int r = 0; r < 7; ++r)
-        if (r < po.n && g >= po.lo[r] && g < po.hi[r]) (out_is_V0 ? po.V0[r] : po.V1[r])[g] = v;
-}
-
-struct GpParams {
-    const unsigned char* rows;   // compacted rows of the policy, 16/8/4-byte planes (pi::Row<D>)
-    float* V0;
-    float* V1;
-    const GpCtl* ctl;
-    float* partial;              // [gridDim.x]
-    long long n_local;
-    long long n_pad;
-    long long s_begin;
-    float gamma;
-    int j;
-    int check;
-    GpPeerOut peers;
-    int rot;                     // sharded runs: block visited first (blocks whose values peers need go first); 0 on one GPU
-    int n_peer_blocks;           // ... and how many blocks from there on can hold states a peer needs (the rest is interior)
-    int sched_begin;             // one state per thread: this launch sweeps blocks [sched_begin, sched_begin + gridDim.x) of the (rotated)
-    int n_blocks;                // schedule of n_blocks blocks (sharded runs with the DMA exchange launch boundary and interior separately)
-    float2* P0;                  // GP_PAIRV: pair shadow of V0, P0[i] = (V0[i], V0[i+1]); else unused
-    float2* P1;                  //           ... of V1
-};
-
 #define GP_W (GP_D + 2)
-#define GP_N4 (GP_W / 4)
-#define GP_N2 ((GP_W % 4) / 2)
 #define GP_C (1 << GP_D)
 #define GP_H (GP_C / 2)
 #ifndef GP_LV
@@ -93,26 +47,6 @@ struct GpParams {
 #define GP_G 0        // gathers per explicitly scheduled group (0: leave the schedule to ptxas)
 #endif
 
-__device__ __forceinline__ gp_u64 gp_pk(float a, float b) {
-    gp_u64 r;
-    asm("mov.b64 %0, {%1, %2};" : "=l"(r) : "f"(a), "f"(b));
-    return r;
-}
-__device__ __forceinline__ void gp_unpk(gp_u64 v, float& a, float& b) {
-    asm("mov.b64 {%0, %1}, %2;" : "=f"(a), "=f"(b) : "l"(v));
-}
-__device__ __forceinline__ gp_u64 gp_mul2(gp_u64 a, gp_u64 b) {
-    gp_u64 r;
-    asm("mul.rn.f32x2 %0, %1, %2;" : "=l"(r) : "l"(a), "l"(b));
-    return r;
-}
-// same multiply, opaque to common-subexpression elimination (GP_LV >= 2: the partial products of the
-// trailing dimensions are RE-computed per corner, not kept in registers)
-__device__ __forceinline__ gp_u64 gp_mul2_nocse(gp_u64 a, gp_u64 b) {
-    gp_u64 r;
-    asm volatile("mul.rn.f32x2 %0, %1, %2;" : "=l"(r) : "l"(a), "l"(b));
-    return r;
-}
 __device__ __forceinline__ float gp_mul_nocse(float a, float b) {
     float r;
     asm volatile("mul.rn.f32 %0, %1, %2;" : "=f"(r) : "f"(a), "f"(b));
@@ -122,45 +56,6 @@ __device__ __forceinline__ float gp_ld_ordered(const float* p) {
     float r;
     asm volatile("ld.global.nc.f32 %0, [%1];" : "=f"(r) : "l"(p));
     return r;
-}
-__device__ __forceinline__ gp_u64 gp_fma2(gp_u64 a, gp_u64 b, gp_u64 c) {
-    gp_u64 r;
-    asm("fma.rn.f32x2 %0, %1, %2, %3;" : "=l"(r) : "l"(a), "l"(b), "l"(c));
-    return r;
-}
-__device__ __forceinline__ float gp_warp_max(float v) {
-#pragma unroll
-    for (int o = 16; o > 0; o >>= 1) v = fmaxf(v, __shfl_xor_sync(0xffffffffu, v, o));
-    return v;
-}
-
-// row of local state s (streaming: read once, keep V in L1/L2)
-__device__ __forceinline__ void gp_load_row(const unsigned char* __restrict__ tab, long long n_pad, long long s,
-                                            unsigned (&w)[GP_W]) {
-#pragma unroll
-    for (int q = 0; q < GP_N4; ++q) {
-        uint4 v;
-        asm volatile("ld.global.nc.L1::no_allocate.v4.u32 {%0,%1,%2,%3}, [%4];"
-                     : "=r"(v.x), "=r"(v.y), "=r"(v.z), "=r"(v.w)
-                     : "l"(tab + (size_t)q * 16u * (size_t)n_pad + (size_t)s * 16u));
-        w[4 * q] = v.x; w[4 * q + 1] = v.y; w[4 * q + 2] = v.z; w[4 * q + 3] = v.w;
-    }
-#if GP_N2
-    {
-        uint2 v;
-        asm volatile("ld.global.nc.L1::no_allocate.v2.u32 {%0,%1}, [%2];" : "=r"(v.x), "=r"(v.y)
-                     : "l"(tab + (size_t)GP_N4 * 16u * (size_t)n_pad + (size_t)s * 8u));
-        w[4 * GP_N4] = v.x; w[4 * GP_N4 + 1] = v.y;
-    }
-#endif
-#if GP_W % 2
-    {
-        unsigned v;
-        asm volatile("ld.global.nc.L1::no_allocate.u32 %0, [%1];" : "=r"(v)
-                     : "l"(tab + ((size_t)GP_N4 * 16u + (size_t)GP_N2 * 8u) * (size_t)n_pad + (size_t)s * 4u));
-        w[GP_W - 1] = v;
-    }
-#endif
 }
 
 #ifndef GP_SINGLE
@@ -186,9 +81,9 @@ __device__ __forceinline__ float2 gp_ld_pair_ordered(const float2* p) {
 #if GP_SINGLE
 // One state per thread: the scalar sweep (pi::eval_sweep_kernel + expected_value_grouped) with the grid's
 // strides as immediates — no address arithmetic, fewer registers, more resident warps.
-extern "C" __global__ void __launch_bounds__(GP_THREADS, GP_MINB) gp_sweep(const GpParams p)
+extern "C" __global__ void __launch_bounds__(GP_THREADS, GP_MINB) gp_sweep(const pi::GpParams p)
 {
-    const GpCtl* __restrict__ ctl = p.ctl;
+    const pi::Ctl* __restrict__ ctl = p.ctl;
     if (ctl->done) return;
     const int par = (ctl->base + p.j + ctl->parity0) & 1;
     const float* __restrict__ Vin = par ? p.V1 : p.V0;
@@ -206,7 +101,7 @@ extern "C" __global__ void __launch_bounds__(GP_THREADS, GP_MINB) gp_sweep(const
     float res = 0.0f;
     if (s < p.n_local) {
         unsigned w[GP_W];
-        gp_load_row(p.rows, p.n_pad, s, w);
+        pi::load_row<GP_D>(p.rows, p.n_pad, s, w);
         const int b = (int)w[0];
         const float vold = Vin[p.s_begin + s];
         float vnew;
@@ -298,24 +193,24 @@ extern "C" __global__ void __launch_bounds__(GP_THREADS, GP_MINB) gp_sweep(const
             if (g > 0) Pout[g - 1].y = vnew;
         }
 #endif
-        if (peer_blk) gp_store_peers(p.peers, par != 0, p.s_begin + s, vnew);
+        if (peer_blk) pi::store_peers(p.peers, par != 0, p.s_begin + s, vnew);
         res = fabsf(vnew - vold);
     }
     if (!p.check) return;
     __shared__ float s_red[32];
-    res = gp_warp_max(res);
+    res = pi::warp_max(res);
     if (lane == 0) s_red[warp] = res;
     __syncthreads();
     if (threadIdx.x < 32) {
         float r = threadIdx.x < GP_THREADS / 32 ? s_red[threadIdx.x] : 0.0f;
-        r = gp_warp_max(r);
+        r = pi::warp_max(r);
         if (threadIdx.x == 0) p.partial[sched] = r;
     }
 }
 #else
-extern "C" __global__ void __launch_bounds__(GP_THREADS, GP_MINB) gp_sweep(const GpParams p)
+extern "C" __global__ void __launch_bounds__(GP_THREADS, GP_MINB) gp_sweep(const pi::GpParams p)
 {
-    const GpCtl* __restrict__ ctl = p.ctl;
+    const pi::Ctl* __restrict__ ctl = p.ctl;
     if (ctl->done) return;
     const int par = (ctl->base + p.j + ctl->parity0) & 1;
     const float* __restrict__ Vin = par ? p.V1 : p.V0;
@@ -329,8 +224,8 @@ extern "C" __global__ void __launch_bounds__(GP_THREADS, GP_MINB) gp_sweep(const
 
     if (inA) {
         unsigned wA[GP_W], wB[GP_W];
-        gp_load_row(p.rows, p.n_pad, sA, wA);
-        if (inB) gp_load_row(p.rows, p.n_pad, sB, wB);
+        pi::load_row<GP_D>(p.rows, p.n_pad, sA, wA);
+        if (inB) pi::load_row<GP_D>(p.rows, p.n_pad, sB, wB);
         else {
 #pragma unroll
             for (int k = 0; k < GP_W; ++k) wB[k] = k == 0 ? 0xfffffffeu : 0u;
@@ -346,18 +241,18 @@ extern "C" __global__ void __launch_bounds__(GP_THREADS, GP_MINB) gp_sweep(const
         gp_u64 node[GP_NT];
         {
             const float fa = __uint_as_float(wA[1]), fb = __uint_as_float(wB[1]);
-            node[0] = gp_pk(1.0f - fa, 1.0f - fb);
-            node[1] = gp_pk(fa, fb);
+            node[0] = pi::pk(1.0f - fa, 1.0f - fb);
+            node[1] = pi::pk(fa, fb);
 #pragma unroll
             for (int d = 1; d < GP_D - GP_LV; ++d) {
                 const float xa = __uint_as_float(wA[1 + d]), xb = __uint_as_float(wB[1 + d]);
-                const gp_u64 f = gp_pk(xa, xb), g = gp_pk(1.0f - xa, 1.0f - xb);
+                const gp_u64 f = pi::pk(xa, xb), g = pi::pk(1.0f - xa, 1.0f - xb);
 #pragma unroll
                 for (int c = GP_NT / 2 - 1; c >= 0; --c) {   // constant trip count: node[] stays in registers
                     if (c < (1 << d)) {
                         const gp_u64 t = node[c];
-                        node[c + (1 << d)] = gp_mul2(t, f);
-                        node[c] = gp_mul2(t, g);
+                        node[c + (1 << d)] = pi::mul2(t, f);
+                        node[c] = pi::mul2(t, g);
                     }
                 }
             }
@@ -367,11 +262,11 @@ extern "C" __global__ void __launch_bounds__(GP_THREADS, GP_MINB) gp_sweep(const
 #pragma unroll
         for (int k = 0; k < GP_LV; ++k) {
             const float la = __uint_as_float(wA[1 + GP_D - GP_LV + k]), lb = __uint_as_float(wB[1 + GP_D - GP_LV + k]);
-            wt[k][0] = gp_pk(1.0f - la, 1.0f - lb);
-            wt[k][1] = gp_pk(la, lb);
+            wt[k][0] = pi::pk(1.0f - la, 1.0f - lb);
+            wt[k][1] = pi::pk(la, lb);
         }
 
-        gp_u64 ev = gp_pk(0.0f, 0.0f);
+        gp_u64 ev = pi::pk(0.0f, 0.0f);
 #if GP_G == 0
 #pragma unroll
         for (int c = 0; c < GP_C; ++c) {
@@ -379,9 +274,9 @@ extern "C" __global__ void __launch_bounds__(GP_THREADS, GP_MINB) gp_sweep(const
 #pragma unroll
             for (int k = 0; k < GP_LV; ++k) {
                 const gp_u64 f = wt[k][(c >> (GP_D - GP_LV + k)) & 1];
-                leaf = (k + 1 < GP_LV) ? gp_mul2_nocse(leaf, f) : gp_mul2(leaf, f);
+                leaf = (k + 1 < GP_LV) ? pi::mul2_nocse(leaf, f) : pi::mul2(leaf, f);
             }
-            ev = gp_fma2(leaf, gp_pk(__ldg(vA + gp_off[c]), __ldg(vB + gp_off[c])), ev);
+            ev = pi::fma2(leaf, pi::pk(__ldg(vA + gp_off[c]), __ldg(vB + gp_off[c])), ev);
         }
 #else
         // explicitly scheduled gathers (see pi::expected_value_grouped): groups of GP_G corners, the loads of
@@ -405,34 +300,34 @@ extern "C" __global__ void __launch_bounds__(GP_THREADS, GP_MINB) gp_sweep(const
 #pragma unroll
                 for (int k = 0; k < GP_LV; ++k) {
                     const gp_u64 f = wt[k][(c >> (GP_D - GP_LV + k)) & 1];
-                    leaf = (k + 1 < GP_LV) ? gp_mul2_nocse(leaf, f) : gp_mul2(leaf, f);
+                    leaf = (k + 1 < GP_LV) ? pi::mul2_nocse(leaf, f) : pi::mul2(leaf, f);
                 }
-                ev = gp_fma2(leaf, gp_pk(bufA[g & 1][i], bufB[g & 1][i]), ev);
+                ev = pi::fma2(leaf, pi::pk(bufA[g & 1][i], bufB[g & 1][i]), ev);
             }
         }
 #endif
         float evA, evB;
-        gp_unpk(ev, evA, evB);
+        pi::unpk(ev, evA, evB);
         // sentinel rows: terminated (-1) -> sum := 0 (:231-232); absorbing (-2) -> new_V := V (:221)
         const float vnewA = bA == -2 ? voldA : fmaf(p.gamma, bA >= 0 ? evA : 0.0f, __uint_as_float(wA[GP_D + 1]));
         Vout[p.s_begin + sA] = vnewA;
-        if (p.peers.n) gp_store_peers(p.peers, par != 0, p.s_begin + sA, vnewA);
+        if (p.peers.n) pi::store_peers(p.peers, par != 0, p.s_begin + sA, vnewA);
         res = fabsf(vnewA - voldA);
         if (inB) {
             const float vnewB = bB == -2 ? voldB : fmaf(p.gamma, bB >= 0 ? evB : 0.0f, __uint_as_float(wB[GP_D + 1]));
             Vout[p.s_begin + sB] = vnewB;
-            if (p.peers.n) gp_store_peers(p.peers, par != 0, p.s_begin + sB, vnewB);
+            if (p.peers.n) pi::store_peers(p.peers, par != 0, p.s_begin + sB, vnewB);
             res = fmaxf(res, fabsf(vnewB - voldB));
         }
     }
     if (!p.check) return;
     __shared__ float s_red[32];
-    res = gp_warp_max(res);
+    res = pi::warp_max(res);
     if (lane == 0) s_red[warp] = res;
     __syncthreads();
     if (threadIdx.x < 32) {
         float r = threadIdx.x < GP_THREADS / 32 ? s_red[threadIdx.x] : 0.0f;
-        r = gp_warp_max(r);
+        r = pi::warp_max(r);
         if (threadIdx.x == 0) p.partial[blockIdx.x] = r;
     }
 }

@@ -19,6 +19,8 @@
 #include <cuda_runtime.h>
 #include <stdint.h>
 
+#include "sweep_common_src.cuh"   // Ctl, PeerOut, PlaneRec, the JIT sweeps' parameter blocks, Row<D>, load_row<D>, warp_max
+
 #define PI_ROW_TERMINATED (-1)
 #define PI_ROW_ABSORBING (-2)
 
@@ -26,23 +28,6 @@ namespace pi {
 
 constexpr int kBlock = 256;
 constexpr int kMaxDims = 6;
-
-// ---------------------------------------------------------------------------
-// Device control block: lets a stream of identical sweep launches sequence
-// itself (sweep counter, ping-pong parity, residual, convergence flag) with no
-// host round trip per sweep.  Mirrors the loop state of policy_evaluation()
-// (src/cuda_policy_iteration.py:300-336).
-// ---------------------------------------------------------------------------
-struct Ctl {
-    int base;                   // sweeps completed before the batch in flight
-    int parity0;                // V buffer that was "current" when the evaluation started
-    int done;                   // 1 once a sync-point residual was < theta
-    int conv_sweep;             // index i of the sweep at which the evaluation converged
-    float last_delta;           // residual of the last examined sweep (local to this rank)
-    float check_delta;          // residual examined at the last sync point (global)
-    unsigned long long changed; // improvement: states whose action changed (local)
-    unsigned int pad[8];
-};
 
 // Grid geometry.  `stride` is the reference's row-major flat index (dim 0 slowest,
 // what callers see); `istride` is the engine's INTERNAL storage order, in which one
@@ -77,34 +62,6 @@ __host__ __device__ inline long long ref_to_internal(const GridDesc& g, long lon
         r = q;
     }
     return out;
-}
-
-// ---------------------------------------------------------------------------
-// Sharded runs: fused V exchange.  Every evaluation-sweep kernel stores a new value not only into
-// its own V buffer but also, through peer pointers (CUDA IPC over NVLink / NVSwitch), directly into
-// the V buffer of every rank whose transition rows reference that state (`[lo, hi)` = the sub-range
-// of THIS rank's slice that peer r needs, computed once after the table build).  The transfer
-// overlaps the sweep tile by tile; a sweep ends with xgpu_barrier_kernel instead of an NCCL
-// send/recv group.  Replaces nothing in the reference (single GPU); SURVEY §5 / §8(e).
-// ---------------------------------------------------------------------------
-constexpr int kMaxPeers = 7;
-struct PeerOut {
-    int n;
-    int pad;
-    float* V0[kMaxPeers];
-    float* V1[kMaxPeers];
-    long long lo[kMaxPeers];
-    long long hi[kMaxPeers];
-};
-
-// out_is_V0: the sweep writes buffer 0 (of every rank) this time
-// Fully unrolled over the (few) entries: a run-time-indexed loop over a kernel-parameter struct makes the compiler copy
-// the struct to local memory and turns every range test into local loads (measured at N = 2: +34 us per K5 sweep in the
-// gather sweep, +71 us in the plane-staged sweep, before any byte crossed NVLink).
-__device__ __forceinline__ void store_peers(const PeerOut& po, bool out_is_V0, long long g, float v) {
-#pragma unroll
-    for (int r = 0; r < kMaxPeers; ++r)
-        if (r < po.n && g >= po.lo[r] && g < po.hi[r]) (out_is_V0 ? po.V0[r] : po.V1[r])[g] = v;
 }
 
 // Cross-GPU barrier at the end of a sweep: thread t publishes this rank's epoch into rank t's flag
@@ -153,39 +110,10 @@ __global__ void xgpu_barrier_kernel(const BarrierParams b) {
 // ---------------------------------------------------------------------------
 // Row layout helpers
 // ---------------------------------------------------------------------------
-template <int D>
-struct Row {
-    static constexpr int W = D + 2;
-    static constexpr int N4 = W / 4;        // 16-byte planes
-    static constexpr int N2 = (W % 4) / 2;  // 8-byte plane (0/1)
-    static constexpr int N1 = W % 2;        // 4-byte plane (0/1)
-    static constexpr int kBytes = W * 4;
-};
-
 __host__ __device__ inline size_t row_table_bytes(int D, long long n_pad) {
     return (size_t)(D + 2) * 4u * (size_t)n_pad;
 }
 
-// streaming (read-once) loads: do not pollute L1, mark evict-first in L2
-__device__ __forceinline__ uint4 ld_stream16(const void* p) {
-    uint4 r;
-    asm volatile("ld.global.nc.L1::no_allocate.v4.u32 {%0,%1,%2,%3}, [%4];"
-                 : "=r"(r.x), "=r"(r.y), "=r"(r.z), "=r"(r.w)
-                 : "l"(p));
-    return r;
-}
-__device__ __forceinline__ uint2 ld_stream8(const void* p) {
-    uint2 r;
-    asm volatile("ld.global.nc.L1::no_allocate.v2.u32 {%0,%1}, [%2];"
-                 : "=r"(r.x), "=r"(r.y)
-                 : "l"(p));
-    return r;
-}
-__device__ __forceinline__ unsigned ld_stream4(const void* p) {
-    unsigned r;
-    asm volatile("ld.global.nc.L1::no_allocate.u32 %0, [%1];" : "=r"(r) : "l"(p));
-    return r;
-}
 __device__ __forceinline__ void st_stream16(void* p, uint4 v) {
     asm volatile("st.global.L1::no_allocate.v4.u32 [%0], {%1,%2,%3,%4};" ::"l"(p), "r"(v.x), "r"(v.y),
                  "r"(v.z), "r"(v.w)
@@ -246,25 +174,6 @@ __device__ __forceinline__ void load_row_hint(const unsigned char* __restrict__ 
     }
     if constexpr (R::N1 != 0) {
         w[R::W - 1] = ld_stream4_hint(tab + ((size_t)R::N4 * 16u + (size_t)R::N2 * 8u) * (size_t)n_pad + (size_t)s * 4u, pol);
-    }
-}
-
-// Load the row of local state `s` from the table that starts at `tab`.
-template <int D>
-__device__ __forceinline__ void load_row(const unsigned char* __restrict__ tab, long long n_pad, long long s,
-                                         unsigned (&w)[Row<D>::W]) {
-    using R = Row<D>;
-#pragma unroll
-    for (int p = 0; p < R::N4; ++p) {
-        uint4 v = ld_stream16(tab + (size_t)p * 16u * (size_t)n_pad + (size_t)s * 16u);
-        w[4 * p + 0] = v.x; w[4 * p + 1] = v.y; w[4 * p + 2] = v.z; w[4 * p + 3] = v.w;
-    }
-    if constexpr (R::N2 != 0) {
-        uint2 v = ld_stream8(tab + (size_t)R::N4 * 16u * (size_t)n_pad + (size_t)s * 8u);
-        w[4 * R::N4 + 0] = v.x; w[4 * R::N4 + 1] = v.y;
-    }
-    if constexpr (R::N1 != 0) {
-        w[R::W - 1] = ld_stream4(tab + ((size_t)R::N4 * 16u + (size_t)R::N2 * 8u) * (size_t)n_pad + (size_t)s * 4u);
     }
 }
 
@@ -347,12 +256,6 @@ __device__ __forceinline__ float expected_value_grouped(const float* __restrict_
     return ev;
 }
 
-
-__device__ __forceinline__ float warp_max(float v) {
-#pragma unroll
-    for (int o = 16; o > 0; o >>= 1) v = fmaxf(v, __shfl_xor_sync(0xffffffffu, v, o));
-    return v;
-}
 
 // ---------------------------------------------------------------------------
 // Evaluation sweep: one Jacobi Bellman backup of every local state with the

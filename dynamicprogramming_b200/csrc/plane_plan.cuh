@@ -24,24 +24,13 @@
 
 #include <cuda_runtime.h>
 
+#include "sweep_common_src.cuh"   // PlaneRec, its limits and the chunk schedule (plan_chunk_begin)
+
 namespace pi {
 
-constexpr int kPlanMaxCells = 8;
-constexpr int kPlanMaxOC = 16;
-constexpr int kPlanMaxLoads = 80;
 constexpr int kPlanMaxSlots = 80;
 constexpr int kPlanHash = 32;
-constexpr int kPlanFallback = 0x40000000;
-constexpr unsigned short kPlanBadSlot = 0xffff;   // cs entry of a cell whose planes found no slot: its states gather from global memory
 constexpr int kPlanThreads = 256;
-
-struct PlaneRec {   // == PsRec in plane_sweep_src.cuh
-    unsigned char n_early, n_late, n_cells, flags;
-    unsigned int pad[3];
-    unsigned short cs[kPlanMaxCells][kPlanMaxOC];   // slot byte offset / 16 of (cell, outer corner)
-    unsigned int loads[kPlanMaxLoads];              // (slot << 24) | V-plane number; early loads first
-};
-static_assert(sizeof(PlaneRec) == 16 + 2 * kPlanMaxCells * kPlanMaxOC + 4 * kPlanMaxLoads, "PlaneRec layout");
 
 // Per state-plane: its distinct successor cells (lower-corner V-plane numbers) and how many states fall into each.
 struct PlaneCells {
@@ -52,16 +41,6 @@ struct PlaneCells {
     int pad[2];
 };
 static_assert(sizeof(PlaneCells) == 64, "PlaneCells layout");
-
-// First state-plane of chunk c (== ps_chunk_begin in plane_sweep_src.cuh).  The sweep's G persistent CTAs take chunks
-// c, c + G, ... of n_chunks = k G: the first n_full = (k - 1) G chunks have exactly L planes (whole lines of the fastest
-// outer dimension: consecutive planes share their V-planes), the last G chunks split the rest evenly, so that every CTA
-// sweeps the same number of planes to within one.
-__host__ __device__ __forceinline__ long long plan_chunk_begin(long long c, int L, int n_full, int n_chunks, int n_planes) {
-    if (c <= n_full) return c * L;
-    const long long base = (long long)n_full * L;
-    return base + (c - n_full) * (n_planes - base) / (n_chunks - n_full);
-}
 
 // Per chunk: the slots its first step loads and the slots its last step reads (bit s of 128 = slot s), written by
 // plane_slots_kernel; and the renumbering plane_stitch_kernel chose for it.
@@ -90,7 +69,7 @@ struct PlanParams {
     int pl_end;                  // upload is planned range by range while the rest is still on its way (pi_upload_policy_local)
     int c_begin, c_end;
     int L, n_full, n_chunks;     // chunk geometry (plan_chunk_begin)
-    int grid, rot;               // the sweep's schedule: CTA b takes the chunks (b + rot), (b + G + rot), ... mod n_chunks
+    int grid, chunk_rot;         // the sweep's schedule: CTA b takes the chunks (b + chunk_rot), (b + G + chunk_rot), ... mod n_chunks
     int P;                       // states per plane
     int NS;                      // shared-memory slots of the sweep
     int noc;                     // outer corners per cell (power of two)
@@ -580,8 +559,8 @@ __global__ void __launch_bounds__(kSlotWarps * 32) plane_slots_kernel(const Plan
     const int lane = threadIdx.x & 31, wq = threadIdx.x >> 5;
     const int chunk = q.c_begin + blockIdx.x * kSlotWarps + wq;
     if (chunk >= q.c_end) return;
-    const int pl0 = (int)plan_chunk_begin(chunk, q.L, q.n_full, q.n_chunks, q.n_planes);
-    const int Lc = (int)plan_chunk_begin(chunk + 1, q.L, q.n_full, q.n_chunks, q.n_planes) - pl0;
+    const int pl0 = plan_chunk_begin(q, chunk);
+    const int Lc = plan_chunk_begin(q, chunk + 1) - pl0;
     int* slot_vp = s_slot_vp[wq];
     int* slot_used = s_slot_used[wq];
     int* cs = s_cs[wq];
@@ -747,7 +726,7 @@ __global__ void __launch_bounds__(kSlotWarps * 32) plane_stitch_kernel(const Pla
     int perm[kPer];   // numbering of the previous chunk: slot lane + 32 w -> perm[w]
     int prev = -1;
     for (int ci = b; ci < q.n_chunks; ci += q.grid) {
-        const int c = ci + q.rot < q.n_chunks ? ci + q.rot : ci + q.rot - q.n_chunks;
+        const int c = plan_chunk_at(q, ci);
         ChunkStitch* st = q.stitch + c;
         unsigned busy[4] = {0u, 0u, 0u, 0u};
         if (prev < 0) {
@@ -800,8 +779,8 @@ __global__ void __launch_bounds__(kRelabelThreads) plane_relabel_kernel(const Pl
     if (tid < kPlanMaxSlots) perm[tid] = st->perm[tid];
     if (tid < 4) busy[tid] = st->busy[tid];
     __syncthreads();
-    const int pl0 = (int)plan_chunk_begin(c, q.L, q.n_full, q.n_chunks, q.n_planes);
-    const int pl1 = (int)plan_chunk_begin(c + 1, q.L, q.n_full, q.n_chunks, q.n_planes);
+    const int pl0 = plan_chunk_begin(q, c);
+    const int pl1 = plan_chunk_begin(q, c + 1);
     const unsigned unit = (unsigned)q.pitch / 4u;   // slot offset entry = slot * pitch * 4 / 16
     for (int pl = pl0; pl < pl1; ++pl) {
         PlaneRec* r = q.plan + pl;

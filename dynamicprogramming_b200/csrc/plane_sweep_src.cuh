@@ -38,82 +38,12 @@
 // The host prepends (dpb200.cu: plane_preamble):
 //   PS_D, PS_P, PS_NS, PS_THREADS (consumer threads = PS_P rounded up to a warp), PS_MINB, PS_LV,
 //   PS_PACK, PS_N0 (extent of the fastest dimension), ps_cj[2^D] (outer-corner number of corner c), ps_imm[2^D] (in-plane float offset of corner c),
-//   gp_off[2^D] (global V offset of corner c, fallback path).
+//   gp_off[2^D] (global V offset of corner c, fallback path);
+// and then sweep_common_src.cuh: pi::PsParams, pi::PlaneRec and its limits, the chunk schedule, the shared device helpers.
 
 typedef unsigned long long ps_u64;
 
-struct PsCtl {   // == pi::Ctl
-    int base, parity0, done, conv_sweep;
-    float last_delta, check_delta;
-    unsigned long long changed;
-    unsigned int pad[8];
-};
-struct PsPeerOut {   // == pi::PeerOut
-    int n;
-    int pad;
-    float* V0[7];
-    float* V1[7];
-    long long lo[7];
-    long long hi[7];
-};
-// unrolled over the 7 entries: a run-time-indexed loop over a kernel-parameter struct is compiled into local-memory copies
-__device__ __forceinline__ void ps_store_peers(const PsPeerOut& po, bool out_is_V0, long long g, float v) {
-#pragma unroll
-    for (int r = 0; r < 7; ++r)
-        if (r < po.n && g >= po.lo[r] && g < po.hi[r]) (out_is_V0 ? po.V0[r] : po.V1[r])[g] = v;
-}
-
-#define PS_MAXC 8          // staged successor cells per state-plane
-#define PS_MAXOC 16        // outer corners per cell (2^(D-2), D <= 6)
-#define PS_MAXLOADS 80     // plane loads per step
-#define PS_FALLBACK 0x40000000
-#define PS_BAD_SLOT (0xffffu << 4)   // staged slot offset of a cell that is not resident (pi::kPlanBadSlot << 4)
-
-struct PsRec {   // == pi::PlaneRec (plane_plan.cuh)
-    unsigned char n_early, n_late, n_cells, flags;
-    unsigned int pad[3];
-    unsigned short cs[PS_MAXC][PS_MAXOC];   // slot byte offset / 16 of (cell, outer corner)
-    unsigned int loads[PS_MAXLOADS];        // (slot << 24) | V-plane number; early loads first
-};
-
-struct PsParams {
-    const unsigned char* prow0;  // planned first row plane: [code, f0, f1, f2] per state (16 B)
-    const unsigned char* rows;   // the policy's rows (pi::Row<D> planes); plane 0 is read on the fallback path only
-    const PsRec* plan;           // one record per local state-plane
-    float* V0;
-    float* V1;
-    const PsCtl* ctl;
-    float* partial;              // [gridDim.x]
-    long long n_local;
-    long long n_pad;
-    long long s_begin;
-    int n_planes;                // local state-planes
-    int n_chunks;                // chunks of the schedule (ps_chunk_begin): n_full of exactly L planes, then gridDim.x uneven ones
-    int L;
-    int n_full;
-    int chunk_rot;               // sharded runs: chunk visited first (the chunks whose values peers need go first, so their NVLink
-                                 // stores drain while the interior is swept); 0 on one GPU
-    int n_peer_chunks;           // ... and how many chunks from there on can hold states a peer needs (the rest is interior)
-    int sched_begin;             // this launch sweeps the chunks [sched_begin, sched_end) of the (rotated) schedule; CTA b takes
-    int sched_end;               // sched_begin + b, sched_begin + b + gridDim.x, ... (the sequence the plan was stitched for)
-    int partial_off;             // first slot of p.partial this launch writes
-    float gamma;
-    int j;
-    int check;
-    PsPeerOut peers;
-};
-
-// first state-plane of chunk c (== pi::plan_chunk_begin in plane_plan.cuh): n_full chunks of L planes, then the rest split
-// evenly over the last n_chunks - n_full
-__device__ __forceinline__ int ps_chunk_begin(const PsParams& p, int c) {
-    if (c <= p.n_full) return c * p.L;
-    const int base = p.n_full * p.L;
-    return base + (int)((long long)(c - p.n_full) * (p.n_planes - base) / (p.n_chunks - p.n_full));
-}
-// chunk visited at schedule position ci
-__device__ __forceinline__ int ps_chunk_at(const PsParams& p, int ci) {
-    return ci + p.chunk_rot < p.n_chunks ? ci + p.chunk_rot : ci + p.chunk_rot - p.n_chunks;
-}
+enum : unsigned { ps_bad_slot = (unsigned)pi::kPlanBadSlot << 4 };   // staged slot offset of a cell that is not resident
 
 #define PS_W (PS_D + 2)
 #define PS_N4 (PS_W / 4)
@@ -139,7 +69,7 @@ __device__ __forceinline__ int ps_chunk_at(const PsParams& p, int ci) {
 #define PS_SLOTS_BYTES (PS_NS * PS_PITCH)
 #define PS_KSTRIDE 20                // words between the slot offsets of two cells: 16 + 4, so that the 128-bit reads of different
                                      // cells by the lanes of a warp fall into different banks
-#define PS_CS_WORDS (PS_MAXC * PS_KSTRIDE)
+#define PS_CS_WORDS (pi::kPlanMaxCells * PS_KSTRIDE)
 #ifndef PS_NOUT
 #define PS_NOUT 4                    // output planes in flight (ring): written by the consumers of step it, stored by TMA after it
 #endif
@@ -190,62 +120,25 @@ __device__ __forceinline__ void ps_bulk_wait_read() { asm volatile("cp.async.bul
 __device__ __forceinline__ void ps_bulk_wait_all() { asm volatile("cp.async.bulk.wait_group 0;" ::: "memory"); }
 __device__ __forceinline__ void ps_fence_async_smem() { asm volatile("fence.proxy.async.shared::cta;" ::: "memory"); }
 
-__device__ __forceinline__ float ps_warp_max(float v) {
-#pragma unroll
-    for (int o = 16; o > 0; o >>= 1) v = fmaxf(v, __shfl_xor_sync(0xffffffffu, v, o));
-    return v;
-}
-
-__device__ __forceinline__ ps_u64 ps_pk(float a, float b) {
-    ps_u64 r;
-    asm("mov.b64 %0, {%1, %2};" : "=l"(r) : "f"(a), "f"(b));
-    return r;
-}
-__device__ __forceinline__ void ps_unpk(ps_u64 v, float& a, float& b) {
-    asm("mov.b64 {%0, %1}, %2;" : "=f"(a), "=f"(b) : "l"(v));
-}
-__device__ __forceinline__ ps_u64 ps_mul2(ps_u64 a, ps_u64 b) {
-    ps_u64 r;
-    asm("mul.rn.f32x2 %0, %1, %2;" : "=l"(r) : "l"(a), "l"(b));
-    return r;
-}
-
-// streaming loads of the row planes (read once per sweep)
-__device__ __forceinline__ uint4 ps_ld16(const void* p) {
-    uint4 v;
-    asm volatile("ld.global.nc.L1::no_allocate.v4.u32 {%0,%1,%2,%3}, [%4];" : "=r"(v.x), "=r"(v.y), "=r"(v.z), "=r"(v.w) : "l"(p));
-    return v;
-}
-__device__ __forceinline__ uint2 ps_ld8(const void* p) {
-    uint2 v;
-    asm volatile("ld.global.nc.L1::no_allocate.v2.u32 {%0,%1}, [%2];" : "=r"(v.x), "=r"(v.y) : "l"(p));
-    return v;
-}
-__device__ __forceinline__ unsigned ps_ld4(const void* p) {
-    unsigned v;
-    asm volatile("ld.global.nc.L1::no_allocate.u32 %0, [%1];" : "=r"(v) : "l"(p));
-    return v;
-}
-
 // row of local state s: word 0 = planner code (prow0), words 1..D = fractions, word D+1 = reward
-__device__ __forceinline__ void ps_load_row(const PsParams& p, long long s, unsigned (&w)[PS_W]) {
+__device__ __forceinline__ void ps_load_row(const pi::PsParams& p, long long s, unsigned (&w)[PS_W]) {
     {
-        const uint4 v = ps_ld16(p.prow0 + (size_t)s * 16u);
+        const uint4 v = pi::ld_stream16(p.prow0 + (size_t)s * 16u);
         w[0] = v.x; w[1] = v.y; w[2] = v.z; w[3] = v.w;
     }
 #pragma unroll
     for (int q = 1; q < PS_N4; ++q) {
-        const uint4 v = ps_ld16(p.rows + (size_t)q * 16u * (size_t)p.n_pad + (size_t)s * 16u);
+        const uint4 v = pi::ld_stream16(p.rows + (size_t)q * 16u * (size_t)p.n_pad + (size_t)s * 16u);
         w[4 * q] = v.x; w[4 * q + 1] = v.y; w[4 * q + 2] = v.z; w[4 * q + 3] = v.w;
     }
 #if PS_N2
     {
-        const uint2 v = ps_ld8(p.rows + (size_t)PS_N4 * 16u * (size_t)p.n_pad + (size_t)s * 8u);
+        const uint2 v = pi::ld_stream8(p.rows + (size_t)PS_N4 * 16u * (size_t)p.n_pad + (size_t)s * 8u);
         w[4 * PS_N4] = v.x; w[4 * PS_N4 + 1] = v.y;
     }
 #endif
 #if PS_W % 2
-    w[PS_W - 1] = ps_ld4(p.rows + ((size_t)PS_N4 * 16u + (size_t)PS_N2 * 8u) * (size_t)p.n_pad + (size_t)s * 4u);
+    w[PS_W - 1] = pi::ld_stream4(p.rows + ((size_t)PS_N4 * 16u + (size_t)PS_N2 * 8u) * (size_t)p.n_pad + (size_t)s * 4u);
 #endif
 }
 
@@ -292,17 +185,12 @@ __device__ __noinline__ float ps_gather_global(const float* __restrict__ Vin, in
 #define PS_NQ ((2 * PS_W + 3) / 4)       // 16-byte quarters per item
 #define PS_KIND(c) (((c) >> 27) & 7u)
 #define PS_EMPTY (4u << 27)
-__device__ __forceinline__ ps_u64 ps_fma2(ps_u64 a, ps_u64 b, ps_u64 c) {
-    ps_u64 r;
-    asm("fma.rn.f32x2 %0, %1, %2, %3;" : "=l"(r) : "l"(a), "l"(b), "l"(c));
-    return r;
-}
 // item `t` of local state-plane `pl`: state A in words [0, W), state B in words [W, 2W)
-__device__ __forceinline__ void ps_load_item(const PsParams& p, long long pl, int t, unsigned (&u)[4 * PS_NQ]) {
+__device__ __forceinline__ void ps_load_item(const pi::PsParams& p, long long pl, int t, unsigned (&u)[4 * PS_NQ]) {
     const unsigned char* src = p.prow0 + ((size_t)pl * PS_NQ * PS_NI + (size_t)t) * 16u;
 #pragma unroll
     for (int q = 0; q < PS_NQ; ++q) {
-        const uint4 v = ps_ld16(src + (size_t)q * PS_NI * 16u);
+        const uint4 v = pi::ld_stream16(src + (size_t)q * PS_NI * 16u);
         u[4 * q] = v.x; u[4 * q + 1] = v.y; u[4 * q + 2] = v.z; u[4 * q + 3] = v.w;
     }
 }
@@ -352,17 +240,17 @@ __device__ __forceinline__ ps_u64 ps_backup_pair(const unsigned* csk, const unsi
         cso[j] = v.x; cso[j + 1] = v.y; cso[j + 2] = v.z; cso[j + 3] = v.w;
     }
     ps_u64 pre[PS_NT];
-    pre[0] = ps_pk(1.0f - fa[0], 1.0f - fb[0]);
-    pre[1] = ps_pk(fa[0], fb[0]);
+    pre[0] = pi::pk(1.0f - fa[0], 1.0f - fb[0]);
+    pre[1] = pi::pk(fa[0], fb[0]);
 #pragma unroll
     for (int d = 1; d < PS_D - PS_LV; ++d) {
-        const ps_u64 ff = ps_pk(fa[d], fb[d]), gg = ps_pk(1.0f - fa[d], 1.0f - fb[d]);
+        const ps_u64 ff = pi::pk(fa[d], fb[d]), gg = pi::pk(1.0f - fa[d], 1.0f - fb[d]);
 #pragma unroll
         for (int c = PS_NT / 2 - 1; c >= 0; --c) {
             if (c < (1 << d)) {
                 const ps_u64 t = pre[c];
-                pre[c + (1 << d)] = ps_mul2(t, ff);
-                pre[c] = ps_mul2(t, gg);
+                pre[c + (1 << d)] = pi::mul2(t, ff);
+                pre[c] = pi::mul2(t, gg);
             }
         }
     }
@@ -370,23 +258,23 @@ __device__ __forceinline__ ps_u64 ps_backup_pair(const unsigned* csk, const unsi
 #pragma unroll
     for (int q = 0; q < PS_LV; ++q) {
         const float la = fa[PS_D - PS_LV + q], lb = fb[PS_D - PS_LV + q];
-        wt[q][0] = ps_pk(1.0f - la, 1.0f - lb);
-        wt[q][1] = ps_pk(la, lb);
+        wt[q][0] = pi::pk(1.0f - la, 1.0f - lb);
+        wt[q][1] = pi::pk(la, lb);
     }
-    ps_u64 ev = ps_pk(0.0f, 0.0f);
+    ps_u64 ev = pi::pk(0.0f, 0.0f);
 #pragma unroll
     for (int c = 0; c < PS_C; ++c) {
         ps_u64 leaf = pre[c & (PS_NT - 1)];
 #pragma unroll
-        for (int q = 0; q < PS_LV; ++q) leaf = ps_mul2(leaf, wt[q][(c >> (PS_D - PS_LV + q)) & 1]);
+        for (int q = 0; q < PS_LV; ++q) leaf = pi::mul2(leaf, wt[q][(c >> (PS_D - PS_LV + q)) & 1]);
         const float* a = reinterpret_cast<const float*>(sbase + cso[ps_cj[c]]);
         // the compiler loads each float once: 3 per (outer corner, f1 corner)
         // the planner starts pairs at even in-plane offsets only (rows have even length), so the first two floats are one
         // aligned 64-bit load (lanes two floats apart: a 32-bit load would pay a two-way bank conflict)
         const int i0 = ps_imm[c] & ~1;
         const float2 lo = *reinterpret_cast<const float2*>(a + i0);
-        const ps_u64 vv = (ps_imm[c] & 1) ? ps_pk(lo.y, a[i0 + 2]) : ps_pk(lo.x, lo.y);
-        ev = ps_fma2(leaf, vv, ev);
+        const ps_u64 vv = (ps_imm[c] & 1) ? pi::pk(lo.y, a[i0 + 2]) : pi::pk(lo.x, lo.y);
+        ev = pi::fma2(leaf, vv, ev);
     }
     return ev;
 }
@@ -401,7 +289,7 @@ __device__ __forceinline__ ps_u64 ps_backup_pair(const unsigned* csk, const unsi
 //            shared memory.  Early loads of step it+1 are issued — and, when that step has no late loads, the barrier
 //            is armed — while step `it` is still being computed, so a warp that finishes early runs one step ahead;
 //   done[b]  (PS_CWARPS arrivals): every consumer warp has finished step `it`: its slots may be overwritten.
-extern "C" __global__ void __launch_bounds__(PS_THREADS + 32, PS_MINB) ps_sweep(const PsParams p)
+extern "C" __global__ void __launch_bounds__(PS_THREADS + 32, PS_MINB) ps_sweep(const pi::PsParams p)
 {
     extern __shared__ __align__(128) unsigned char ps_smem[];
     unsigned* const cs_s = reinterpret_cast<unsigned*>(ps_smem + PS_SLOTS_BYTES);                    // [2][PS_CS_WORDS] slot byte offsets
@@ -410,7 +298,7 @@ extern "C" __global__ void __launch_bounds__(PS_THREADS + 32, PS_MINB) ps_sweep(
     float* const out_s = reinterpret_cast<float*>(ps_smem + PS_SLOTS_BYTES + 2 * PS_CS_WORDS * 4 + 32);   // [PS_NOUT][PS_P] new values of a plane
     __shared__ float s_red[(PS_THREADS + 32) / 32];
 
-    const PsCtl* __restrict__ ctl = p.ctl;
+    const pi::Ctl* __restrict__ ctl = p.ctl;
     if (ctl->done) return;
     const int par = (ctl->base + p.j + ctl->parity0) & 1;
     const float* __restrict__ Vin = par ? p.V1 : p.V0;
@@ -440,16 +328,16 @@ extern "C" __global__ void __launch_bounds__(PS_THREADS + 32, PS_MINB) ps_sweep(
         // with independent loads (the whole load list, whatever the counts): the producer's trigger after `done` never waits
         // for global memory.  (Fetching a record when it was needed — header first, then the entries it announces — put two
         // dependent DRAM round trips into every step: the sweep took the same 1.31 ms with half the consumer instructions.)
-        constexpr int kPerLane = (PS_MAXLOADS + 31) / 32;
+        constexpr int kPerLane = (pi::kPlanMaxLoads + 31) / 32;
         struct Fetched {
             unsigned hdr;               // n_early | n_late << 8 | n_cells << 16 | flags << 24
             unsigned e[kPerLane];       // loads[lane + 32 q]: early loads first, then the late ones
             uint2 cs;                   // slot offsets of (cell lane / 4, outer corners 4 (lane % 4) ..)
         };
-        auto fetch_rec = [&](const PsRec* r, Fetched& f) {
+        auto fetch_rec = [&](const pi::PlaneRec* r, Fetched& f) {
             f.hdr = *reinterpret_cast<const unsigned*>(r);
 #pragma unroll
-            for (int q = 0; q < kPerLane; ++q) f.e[q] = lane + 32 * q < PS_MAXLOADS ? r->loads[lane + 32 * q] : 0u;
+            for (int q = 0; q < kPerLane; ++q) f.e[q] = lane + 32 * q < pi::kPlanMaxLoads ? r->loads[lane + 32 * q] : 0u;
             f.cs = *reinterpret_cast<const uint2*>(reinterpret_cast<const unsigned short*>(r->cs) + lane * 4);
         };
         // entries [first, first + n) of the record's list: one TMA bulk copy each
@@ -488,13 +376,19 @@ extern "C" __global__ void __launch_bounds__(PS_THREADS + 32, PS_MINB) ps_sweep(
         // sequence).  Only the first step of the launch issues all of its loads itself.
         bool armed = false;   // full[it & 1] was already armed one step ahead
         int f_ci = p.sched_begin + blockIdx.x, f_pl = 0, f_end = 0;   // fetch cursor: the step whose record is fetched next
-        if (f_ci < p.sched_end) { f_pl = ps_chunk_begin(p, ps_chunk_at(p, f_ci)); f_end = ps_chunk_begin(p, ps_chunk_at(p, f_ci) + 1); }
+        if (f_ci < p.sched_end) {
+            f_pl = pi::plan_chunk_begin(p, pi::plan_chunk_at(p, f_ci));
+            f_end = pi::plan_chunk_begin(p, pi::plan_chunk_at(p, f_ci) + 1);
+        }
         auto fetch_next = [&](Fetched& f) {
             if (f_ci >= p.sched_end) return;
             fetch_rec(p.plan + f_pl, f);
             if (++f_pl == f_end) {
                 f_ci += gridDim.x;
-                if (f_ci < p.sched_end) { f_pl = ps_chunk_begin(p, ps_chunk_at(p, f_ci)); f_end = ps_chunk_begin(p, ps_chunk_at(p, f_ci) + 1); }
+                if (f_ci < p.sched_end) {
+                    f_pl = pi::plan_chunk_begin(p, pi::plan_chunk_at(p, f_ci));
+                    f_end = pi::plan_chunk_begin(p, pi::plan_chunk_at(p, f_ci) + 1);
+                }
             }
         };
         Fetched cur, nxt, nn;
@@ -503,9 +397,9 @@ extern "C" __global__ void __launch_bounds__(PS_THREADS + 32, PS_MINB) ps_sweep(
         fetch_next(nxt);
         nn = nxt;
         for (int ci = p.sched_begin + blockIdx.x; ci < p.sched_end; ci += gridDim.x) {
-            const int chunk = ps_chunk_at(p, ci);
-            const int pl0 = ps_chunk_begin(p, chunk);
-            const int Lc = ps_chunk_begin(p, chunk + 1) - pl0;
+            const int chunk = pi::plan_chunk_at(p, ci);
+            const int pl0 = pi::plan_chunk_begin(p, chunk);
+            const int Lc = pi::plan_chunk_begin(p, chunk + 1) - pl0;
             const bool next_chunk = ci + (int)gridDim.x < p.sched_end;
             for (int i = 0; i < Lc; ++i, ++it) {
                 const bool more = i + 1 < Lc || next_chunk;
@@ -520,9 +414,9 @@ extern "C" __global__ void __launch_bounds__(PS_THREADS + 32, PS_MINB) ps_sweep(
                     if (i + PS_ROW_PF >= Lc) {
                         pf_pl = -1;
                         if (next_chunk) {
-                            const int chn = ps_chunk_at(p, ci + (int)gridDim.x);
-                            pf_pl = ps_chunk_begin(p, chn) + (i + PS_ROW_PF - Lc);
-                            if (pf_pl >= ps_chunk_begin(p, chn + 1)) pf_pl = -1;
+                            const int chn = pi::plan_chunk_at(p, ci + (int)gridDim.x);
+                            pf_pl = pi::plan_chunk_begin(p, chn) + (i + PS_ROW_PF - Lc);
+                            if (pf_pl >= pi::plan_chunk_begin(p, chn + 1)) pf_pl = -1;
                         }
                     }
                     if (pf_pl >= 0) {
@@ -540,7 +434,7 @@ extern "C" __global__ void __launch_bounds__(PS_THREADS + 32, PS_MINB) ps_sweep(
 #if PS_PF_AHEAD > 0
                 // optional (off by default, see PS_PF_AHEAD): pull the planes of a later step into L2 now
                 if (i + PS_PF_AHEAD < Lc) {
-                    const PsRec* rp = p.plan + pl0 + i + PS_PF_AHEAD;
+                    const pi::PlaneRec* rp = p.plan + pl0 + i + PS_PF_AHEAD;
                     const unsigned np = (unsigned)rp->n_early + rp->n_late;
                     for (unsigned q = lane; q < np; q += 32)
                         ps_bulk_prefetch_l2(Vin + (size_t)(rp->loads[q] & 0xffffffu) * PS_P, PS_PLANE_BYTES);
@@ -594,12 +488,13 @@ extern "C" __global__ void __launch_bounds__(PS_THREADS + 32, PS_MINB) ps_sweep(
 #if PS_PACK == 2
         // the item of the CTA's next step is in flight while this one is backed up, across chunk boundaries too
         unsigned u[4 * PS_NQ];
-        if (p.sched_begin + (int)blockIdx.x < p.sched_end) ps_load_item(p, ps_chunk_begin(p, ps_chunk_at(p, p.sched_begin + blockIdx.x)), tid, u);
+        if (p.sched_begin + (int)blockIdx.x < p.sched_end)
+            ps_load_item(p, pi::plan_chunk_begin(p, pi::plan_chunk_at(p, p.sched_begin + blockIdx.x)), tid, u);
         for (int ci = p.sched_begin + blockIdx.x; ci < p.sched_end; ci += gridDim.x) {
-            const int chunk = ps_chunk_at(p, ci);
-            const int pl0 = ps_chunk_begin(p, chunk);
-            const int Lc = ps_chunk_begin(p, chunk + 1) - pl0;
-            const int pl_next = ci + (int)gridDim.x < p.sched_end ? ps_chunk_begin(p, ps_chunk_at(p, ci + (int)gridDim.x)) : -1;
+            const int chunk = pi::plan_chunk_at(p, ci);
+            const int pl0 = pi::plan_chunk_begin(p, chunk);
+            const int Lc = pi::plan_chunk_begin(p, chunk + 1) - pl0;
+            const int pl_next = ci + (int)gridDim.x < p.sched_end ? pi::plan_chunk_begin(p, pi::plan_chunk_at(p, ci + (int)gridDim.x)) : -1;
             for (int i = 0; i < Lc; ++i, ++it) {
                 const unsigned b = it & 1;
                 const long long sp = (long long)(pl0 + i) * PS_P;   // first local state of the plane
@@ -632,9 +527,9 @@ extern "C" __global__ void __launch_bounds__(PS_THREADS + 32, PS_MINB) ps_sweep(
 
                 float eva = 0.0f, evb = 0.0f;
                 const unsigned* csa = cs_s + b * PS_CS_WORDS + ((ca >> 24) & 7u) * PS_KSTRIDE;
-                if (is_pair && csa[0] != PS_BAD_SLOT) {
+                if (is_pair && csa[0] != ps_bad_slot) {
                     const ps_u64 ev2 = ps_backup_pair(csa, ps_smem + ((ca >> 12) & 0xfffu) * 4u, fa, fb);
-                    ps_unpk(ev2, eva, evb);
+                    pi::unpk(ev2, eva, evb);
                 } else {
 #pragma unroll 1
                     for (int h = 0; h < 2; ++h) {
@@ -646,11 +541,11 @@ extern "C" __global__ void __launch_bounds__(PS_THREADS + 32, PS_MINB) ps_sweep(
                         for (int d = 0; d < PS_D; ++d) fr[d] = h ? fb[d] : fa[d];
                         const unsigned* csk = cs_s + b * PS_CS_WORDS + ((cc >> 24) & 7u) * PS_KSTRIDE;
                         float ev;
-                        if (kind == 0u && csk[0] != PS_BAD_SLOT) {
+                        if (kind == 0u && csk[0] != ps_bad_slot) {
                             ev = ps_backup_one(csk, ps_smem + ((cc >> 12) & 0xfffu) * 4u, fr);
                         } else {
                             // not staged: the original base index is word 0 of the policy's row
-                            const int base = (int)ps_ld4(p.rows + (size_t)(sp + (cc & 0xfffu)) * 16u);
+                            const int base = (int)pi::ld_stream4(p.rows + (size_t)(sp + (cc & 0xfffu)) * 16u);
                             ev = ps_gather_global(Vin, base, fr[0], fr[1], fr[2], fr[3]
 #if PS_D >= 5
                                                   , fr[4]
@@ -684,18 +579,18 @@ extern "C" __global__ void __launch_bounds__(PS_THREADS + 32, PS_MINB) ps_sweep(
         // the row of the CTA's next step is in flight while this one is backed up, across chunk boundaries too
         unsigned w[PS_W];
         if (has_state && p.sched_begin + (int)blockIdx.x < p.sched_end)
-            ps_load_row(p, (long long)ps_chunk_begin(p, ps_chunk_at(p, p.sched_begin + blockIdx.x)) * PS_P + tid, w);
+            ps_load_row(p, (long long)pi::plan_chunk_begin(p, pi::plan_chunk_at(p, p.sched_begin + blockIdx.x)) * PS_P + tid, w);
         for (int ci = p.sched_begin + blockIdx.x; ci < p.sched_end; ci += gridDim.x) {
-            const int chunk = ps_chunk_at(p, ci);
-            const int pl0 = ps_chunk_begin(p, chunk);
-            const int Lc = ps_chunk_begin(p, chunk + 1) - pl0;
-            const int pl_next = ci + (int)gridDim.x < p.sched_end ? ps_chunk_begin(p, ps_chunk_at(p, ci + (int)gridDim.x)) : -1;
+            const int chunk = pi::plan_chunk_at(p, ci);
+            const int pl0 = pi::plan_chunk_begin(p, chunk);
+            const int Lc = pi::plan_chunk_begin(p, chunk + 1) - pl0;
+            const int pl_next = ci + (int)gridDim.x < p.sched_end ? pi::plan_chunk_begin(p, pi::plan_chunk_at(p, ci + (int)gridDim.x)) : -1;
             for (int i = 0; i < Lc; ++i, ++it) {
                 const unsigned b = it & 1;
                 const long long s = (long long)(pl0 + i) * PS_P + tid;   // local state
                 const long long g = p.s_begin + s;
                 const int code = has_state ? (int)w[0] : -1;
-                const bool staged = code >= 0 && !(code & PS_FALLBACK);
+                const bool staged = code >= 0 && !(code & pi::kPlanFallback);
                 const unsigned k = staged ? ((unsigned)code >> 16) : 0u;
                 const unsigned ip = staged ? ((unsigned)code & 0xffffu) : 0u;
                 float fr[PS_D];
@@ -712,7 +607,7 @@ extern "C" __global__ void __launch_bounds__(PS_THREADS + 32, PS_MINB) ps_sweep(
 
                 float ev = 0.0f;
                 // a cell whose V-planes found no slot is marked in its slot offsets (plane_slots_kernel): gather from global
-                const bool resident = staged && cs_s[b * PS_CS_WORDS + k * PS_KSTRIDE] != PS_BAD_SLOT;
+                const bool resident = staged && cs_s[b * PS_CS_WORDS + k * PS_KSTRIDE] != ps_bad_slot;
                 if (resident) {
                     const unsigned* csk = cs_s + b * PS_CS_WORDS + k * PS_KSTRIDE;
                     const unsigned char* sbase = ps_smem + ip * 4u;
@@ -721,16 +616,16 @@ extern "C" __global__ void __launch_bounds__(PS_THREADS + 32, PS_MINB) ps_sweep(
                     // (1-f_d, 1-f_d) and (f_d, f_d) — one mul.rn.f32x2 per two products, each half rounded like the
                     // scalar product of the reference
                     ps_u64 node[PS_NT / 2];
-                    node[0] = ps_pk(1.0f - fr[0], fr[0]);
+                    node[0] = pi::pk(1.0f - fr[0], fr[0]);
 #pragma unroll
                     for (int d = 1; d < PS_D - PS_LV; ++d) {
-                        const ps_u64 ff = ps_pk(fr[d], fr[d]), gg = ps_pk(1.0f - fr[d], 1.0f - fr[d]);
+                        const ps_u64 ff = pi::pk(fr[d], fr[d]), gg = pi::pk(1.0f - fr[d], 1.0f - fr[d]);
 #pragma unroll
                         for (int c = PS_NT / 4 - 1; c >= 0; --c) {
                             if (c < (1 << (d - 1))) {
                                 const ps_u64 t = node[c];
-                                node[c + (1 << (d - 1))] = ps_mul2(t, ff);
-                                node[c] = ps_mul2(t, gg);
+                                node[c + (1 << (d - 1))] = pi::mul2(t, ff);
+                                node[c] = pi::mul2(t, gg);
                             }
                         }
                     }
@@ -738,16 +633,16 @@ extern "C" __global__ void __launch_bounds__(PS_THREADS + 32, PS_MINB) ps_sweep(
 #pragma unroll
                     for (int q = 0; q < PS_LV; ++q) {
                         const float l = fr[PS_D - PS_LV + q];
-                        wt[q][0] = ps_pk(1.0f - l, 1.0f - l);
-                        wt[q][1] = ps_pk(l, l);
+                        wt[q][0] = pi::pk(1.0f - l, 1.0f - l);
+                        wt[q][1] = pi::pk(l, l);
                     }
 #pragma unroll
                     for (int c = 0; c < PS_C; c += 2) {
                         ps_u64 leaf = node[(c & (PS_NT - 1)) >> 1];
 #pragma unroll
-                        for (int q = 0; q < PS_LV; ++q) leaf = ps_mul2(leaf, wt[q][(c >> (PS_D - PS_LV + q)) & 1]);
+                        for (int q = 0; q < PS_LV; ++q) leaf = pi::mul2(leaf, wt[q][(c >> (PS_D - PS_LV + q)) & 1]);
                         float l0, l1;
-                        ps_unpk(leaf, l0, l1);
+                        pi::unpk(leaf, l0, l1);
                         const float* a0 = reinterpret_cast<const float*>(sbase + csk[ps_cj[c]]);
                         const float* a1 = reinterpret_cast<const float*>(sbase + csk[ps_cj[c + 1]]);
                         ev = fmaf(l0, a0[ps_imm[c]], ev);
@@ -787,7 +682,7 @@ extern "C" __global__ void __launch_bounds__(PS_THREADS + 32, PS_MINB) ps_sweep(
 #endif
                 } else if (code >= 0) {
                     // not staged: the original base index is word 0 of the policy's row
-                    const int base = (int)ps_ld4(p.rows + (size_t)s * 16u);
+                    const int base = (int)pi::ld_stream4(p.rows + (size_t)s * 16u);
                     ev = ps_gather_global(Vin, base, fr[0], fr[1], fr[2], fr[3]
 #if PS_D >= 5
                                           , fr[4]
@@ -811,12 +706,12 @@ extern "C" __global__ void __launch_bounds__(PS_THREADS + 32, PS_MINB) ps_sweep(
     }
 
     if (!p.check) return;
-    res = ps_warp_max(res);
+    res = pi::warp_max(res);
     if (lane == 0) s_red[tid >> 5] = res;
     __syncthreads();
     if (tid < 32) {
         float r = tid < (PS_THREADS + 32) / 32 ? s_red[tid] : 0.0f;
-        r = ps_warp_max(r);
+        r = pi::warp_max(r);
         if (tid == 0) p.partial[p.partial_off + blockIdx.x] = r;
     }
 }

@@ -16,6 +16,8 @@
 //   xl_ntile[], xl_tline[]   tiles per storage position / V-line step between tiles
 //   xl_line_off[]            V-line offset of x-line xl inside a tile (__constant__)
 //
+// and then sweep_common_src.cuh (pi::XlParams, pi::Ctl, the shared device helpers).
+//
 // Design (DESIGN.md §5).  A thread owns K consecutive states of one x-line.  When their
 // successor cells are consecutive (base_j = A + j — the translation-invariant case the
 // layout probe picks the fast dimension for) the 2^D corners of all K states live in
@@ -34,48 +36,6 @@
 
 typedef unsigned long long xl_u64;
 
-struct XlCtl {   // == pi::Ctl
-    int base, parity0, done, conv_sweep;
-    float last_delta, check_delta;
-    unsigned long long changed;
-    unsigned int pad[8];
-};
-
-
-// == pi::PeerOut (pi_kernels.cuh): sharded runs store new values straight into the V buffers of the
-// ranks that need them (CUDA IPC peer pointers over NVLink); n == 0 otherwise.
-struct XlPeerOut {
-    int n;
-    int pad;
-    float* V0[7];
-    float* V1[7];
-    long long lo[7];
-    long long hi[7];
-};
-// unrolled over the 7 entries: a run-time-indexed loop over a kernel-parameter struct is compiled into local-memory copies
-__device__ __forceinline__ void xl_store_peers(const XlPeerOut& po, bool out_is_V0, long long g, float v) {
-#pragma unroll
-    for (int r = 0; r < 7; ++r)
-        if (r < po.n && g >= po.lo[r] && g < po.hi[r]) (out_is_V0 ? po.V0[r] : po.V1[r])[g] = v;
-}
-
-struct XlParams {
-    const unsigned* rows;      // plane w (word w of every row) at rows + w * plane_words
-    long long plane_words;
-    float* V0;
-    float* V1;
-    const XlCtl* ctl;
-    float* partial;            // [gridDim.x] residual maxima (check sweeps)
-    unsigned long long* stats; // optional: [0] += window-path threads, [1] += scalar-path threads
-    long long n_tiles;         // tiles owned by this rank
-    long long tile_begin;      // global index of the first of them
-    float gamma;
-    int j;
-    int check;
-    int prefetch;              // 1: TMA-prefetch the next tile's rows into L2
-    XlPeerOut peers;
-};
-
 #define XL_W (XL_D + 2)
 #define XL_TPL (XL_S / XL_K)          // threads per x-line
 #define XL_LPW (32 / XL_TPL)          // x-lines per warp
@@ -84,48 +44,6 @@ struct XlParams {
 #define XL_DT (XL_D - 1 - XL_LV)      // dims held in the stored weight tree
 #define XL_NN (1 << XL_DT)
 #define XL_NP (XL_K / 2)
-
-__device__ __forceinline__ xl_u64 xl_pk(float a, float b) {
-    xl_u64 r;
-    asm("mov.b64 %0, {%1, %2};" : "=l"(r) : "f"(a), "f"(b));
-    return r;
-}
-__device__ __forceinline__ void xl_unpk(xl_u64 v, float& a, float& b) {
-    asm("mov.b64 {%0, %1}, %2;" : "=f"(a), "=f"(b) : "l"(v));
-}
-__device__ __forceinline__ xl_u64 xl_mul2(xl_u64 a, xl_u64 b) {
-    xl_u64 r;
-    asm("mul.rn.f32x2 %0, %1, %2;" : "=l"(r) : "l"(a), "l"(b));
-    return r;
-}
-// same multiply, but opaque to common-subexpression elimination: with XL_LV == 1 the level D-2
-// weights are RE-computed per window instead of being kept in 2^(D-1) registers per state pair
-__device__ __forceinline__ xl_u64 xl_mul2_nocse(xl_u64 a, xl_u64 b) {
-    xl_u64 r;
-    asm volatile("mul.rn.f32x2 %0, %1, %2;" : "=l"(r) : "l"(a), "l"(b));
-    return r;
-}
-__device__ __forceinline__ xl_u64 xl_fma2(xl_u64 a, xl_u64 b, xl_u64 c) {
-    xl_u64 r;
-    asm("fma.rn.f32x2 %0, %1, %2, %3;" : "=l"(r) : "l"(a), "l"(b), "l"(c));
-    return r;
-}
-__device__ __forceinline__ uint4 xl_ld_stream16(const void* p) {
-    uint4 r;
-    asm volatile("ld.global.nc.L1::no_allocate.v4.u32 {%0,%1,%2,%3}, [%4];"
-                 : "=r"(r.x), "=r"(r.y), "=r"(r.z), "=r"(r.w) : "l"(p));
-    return r;
-}
-__device__ __forceinline__ uint2 xl_ld_stream8(const void* p) {
-    uint2 r;
-    asm volatile("ld.global.nc.L1::no_allocate.v2.u32 {%0,%1}, [%2];" : "=r"(r.x), "=r"(r.y) : "l"(p));
-    return r;
-}
-__device__ __forceinline__ float xl_warp_max(float v) {
-#pragma unroll
-    for (int o = 16; o > 0; o >>= 1) v = fmaxf(v, __shfl_xor_sync(0xffffffffu, v, o));
-    return v;
-}
 
 struct XlVec {
     float v[XL_K];
@@ -180,30 +98,30 @@ __device__ __forceinline__ void xl_window_path(const float* __restrict__ vb, con
 #pragma unroll
     for (int q = 0; q < XL_NP; ++q) {
         const float fa = frac[2 * q][0], fb = frac[2 * q + 1][0];
-        node[q][0] = xl_pk(1.0f - fa, 1.0f - fb);
-        node[q][1] = xl_pk(fa, fb);
+        node[q][0] = pi::pk(1.0f - fa, 1.0f - fb);
+        node[q][1] = pi::pk(fa, fb);
 #pragma unroll
         for (int d = 1; d < XL_DT; ++d) {
-            const xl_u64 f = xl_pk(frac[2 * q][d], frac[2 * q + 1][d]);
-            const xl_u64 g = xl_pk(1.0f - frac[2 * q][d], 1.0f - frac[2 * q + 1][d]);
+            const xl_u64 f = pi::pk(frac[2 * q][d], frac[2 * q + 1][d]);
+            const xl_u64 g = pi::pk(1.0f - frac[2 * q][d], 1.0f - frac[2 * q + 1][d]);
 #pragma unroll
             for (int c = XL_NN / 2 - 1; c >= 0; --c) {   // constant trip count: node[] stays in registers
                 if (c < (1 << d)) {
                     const xl_u64 t = node[q][c];
-                    node[q][c + (1 << d)] = xl_mul2(t, f);
-                    node[q][c] = xl_mul2(t, g);
+                    node[q][c + (1 << d)] = pi::mul2(t, f);
+                    node[q][c] = pi::mul2(t, g);
                 }
             }
         }
-        wl[q][0] = xl_pk(1.0f - frac[2 * q][XL_D - 1], 1.0f - frac[2 * q + 1][XL_D - 1]);
-        wl[q][1] = xl_pk(frac[2 * q][XL_D - 1], frac[2 * q + 1][XL_D - 1]);
-        wm[q][0] = xl_pk(1.0f - frac[2 * q][XL_D - 2], 1.0f - frac[2 * q + 1][XL_D - 2]);
-        wm[q][1] = xl_pk(frac[2 * q][XL_D - 2], frac[2 * q + 1][XL_D - 2]);
+        wl[q][0] = pi::pk(1.0f - frac[2 * q][XL_D - 1], 1.0f - frac[2 * q + 1][XL_D - 1]);
+        wl[q][1] = pi::pk(frac[2 * q][XL_D - 1], frac[2 * q + 1][XL_D - 1]);
+        wm[q][0] = pi::pk(1.0f - frac[2 * q][XL_D - 2], 1.0f - frac[2 * q + 1][XL_D - 2]);
+        wm[q][1] = pi::pk(frac[2 * q][XL_D - 2], frac[2 * q + 1][XL_D - 2]);
     }
 
     xl_u64 ev[XL_NP];
 #pragma unroll
-    for (int q = 0; q < XL_NP; ++q) ev[q] = xl_pk(0.0f, 0.0f);
+    for (int q = 0; q < XL_NP; ++q) ev[q] = pi::pk(0.0f, 0.0f);
 
     // The 2^(D-1) windows are walked as XL_ROLL run-time iterations of XL_NB fully unrolled
     // windows (the rolled loop bounds code size and the live ranges of the in-flight loads;
@@ -257,30 +175,30 @@ __device__ __forceinline__ void xl_window_path(const float* __restrict__ vb, con
                     if (XL_ROLL == 1) {
                         const int half = ob / XL_NH, ol = ob % XL_NH;
 #if XL_LV == 0
-                        leaf = xl_mul2(node[q][2 * ol + xb], wl[q][half]);
+                        leaf = pi::mul2(node[q][2 * ol + xb], wl[q][half]);
 #else
-                        leaf = xl_mul2(xl_mul2_nocse(node[q][2 * (ol % (XL_NH / 2)) + xb], wm[q][ol / (XL_NH / 2)]), wl[q][half]);
+                        leaf = pi::mul2(pi::mul2_nocse(node[q][2 * (ol % (XL_NH / 2)) + xb], wm[q][ol / (XL_NH / 2)]), wl[q][half]);
 #endif
                     } else {
 #if XL_LV == 0
-                        leaf = xl_mul2(node[q][2 * ob + xb], wls[q]);                       // NB == NH: ol == ob
+                        leaf = pi::mul2(node[q][2 * ob + xb], wls[q]);                       // NB == NH: ol == ob
 #else
-                        if (NB == XL_NH) leaf = xl_mul2(xl_mul2_nocse(node[q][2 * (ob % (XL_NH / 2)) + xb], wm[q][ob / (XL_NH / 2)]), wls[q]);
-                        else leaf = xl_mul2(xl_mul2_nocse(node[q][2 * ob + xb], wms[q]), wls[q]);   // NB == NH/2
+                        if (NB == XL_NH) leaf = pi::mul2(pi::mul2_nocse(node[q][2 * (ob % (XL_NH / 2)) + xb], wm[q][ob / (XL_NH / 2)]), wls[q]);
+                        else leaf = pi::mul2(pi::mul2_nocse(node[q][2 * ob + xb], wms[q]), wls[q]);   // NB == NH/2
 #endif
                     }
-                    ev[q] = xl_fma2(leaf, xl_pk(W[2 * q + xb], W[2 * q + 1 + xb]), ev[q]);
+                    ev[q] = pi::fma2(leaf, pi::pk(W[2 * q + xb], W[2 * q + 1 + xb]), ev[q]);
                 }
             }
         }
     }
 #pragma unroll
-    for (int q = 0; q < XL_NP; ++q) xl_unpk(ev[q], ev_out[2 * q], ev_out[2 * q + 1]);
+    for (int q = 0; q < XL_NP; ++q) pi::unpk(ev[q], ev_out[2 * q], ev_out[2 * q + 1]);
 }
 
-extern "C" __global__ void __launch_bounds__(XL_WARPS * 32, XL_MINB) xl_sweep(const XlParams p)
+extern "C" __global__ void __launch_bounds__(XL_WARPS * 32, XL_MINB) xl_sweep(const pi::XlParams p)
 {
-    const XlCtl* __restrict__ ctl = p.ctl;
+    const pi::Ctl* __restrict__ ctl = p.ctl;
     if (ctl->done) return;
     const int par = (ctl->base + p.j + ctl->parity0) & 1;
     const float* __restrict__ Vin = par ? p.V1 : p.V0;
@@ -334,10 +252,10 @@ extern "C" __global__ void __launch_bounds__(XL_WARPS * 32, XL_MINB) xl_sweep(co
             for (int k = 0; k < XL_W; ++k) {
                 const unsigned* src = p.rows + (size_t)k * (size_t)p.plane_words + r0;
 #if XL_K == 4
-                const uint4 t = xl_ld_stream16(src);
+                const uint4 t = pi::ld_stream16(src);
                 w[k][0] = t.x; w[k][1] = t.y; w[k][2] = t.z; w[k][3] = t.w;
 #else
-                const uint2 t = xl_ld_stream8(src);
+                const uint2 t = pi::ld_stream8(src);
                 w[k][0] = t.x; w[k][1] = t.y;
 #endif
             }
@@ -444,7 +362,7 @@ extern "C" __global__ void __launch_bounds__(XL_WARPS * 32, XL_MINB) xl_sweep(co
 #endif
             if (p.peers.n) {
 #pragma unroll
-                for (int j = 0; j < XL_K; ++j) xl_store_peers(p.peers, par != 0, v0 + j, vnew[j]);
+                for (int j = 0; j < XL_K; ++j) pi::store_peers(p.peers, par != 0, v0 + j, vnew[j]);
             }
         }
     }
@@ -455,12 +373,12 @@ extern "C" __global__ void __launch_bounds__(XL_WARPS * 32, XL_MINB) xl_sweep(co
     }
     if (!p.check) return;
     __shared__ float s_red[32];
-    res = xl_warp_max(res);
+    res = pi::warp_max(res);
     if (lane == 0) s_red[warp] = res;
     __syncthreads();
     if (threadIdx.x < 32) {
         float r = threadIdx.x < XL_WARPS ? s_red[threadIdx.x] : 0.0f;
-        r = xl_warp_max(r);
+        r = pi::warp_max(r);
         if (threadIdx.x == 0) p.partial[blockIdx.x] = r;
     }
 }
