@@ -590,37 +590,71 @@ class _CudaPolicyIterationBase(abc.ABC):
             self._lookup = look
         return look[1](pts)
 
-    def _rollout_handle(self, need_current_policy: bool = True):
+    def _rollout_handle(self, need_current_policy: bool = True, need_values: bool = False):
         """The cached PolicyRollout of this object (see rollout()); rebuilt when the policy object or the dynamics text
         changes.  A live engine's policy is taken through download(); an unchanged download reuses the handle.  A single
-        step does not use the policy (need_current_policy=False): any handle built from the same text serves it."""
+        step does not use the policy (need_current_policy=False): any handle built from the same text serves it.
+        need_values: the lookahead's value table is uploaded too, and again whenever it changes (a live engine's V
+        through the same download(), after run() / load() the host `value_function` object)."""
         from .utils import PolicyRollout
         src = self._dynamics_cuda_src()
         cached = getattr(self, "_rollout", None)
         live = bool(getattr(self, "_engine", None))
-        if cached is not None and cached[1] == src and not need_current_policy:
+        if cached is not None and cached[1] == src and not need_current_policy and not need_values:
             return cached[2]
-        policy = self.download()[1] if live else self.policy
-        if cached is not None and cached[1] == src and (cached[0] is policy or (live and np.array_equal(cached[0], policy))):
-            return cached[2]
-        if cached is not None:
-            cached[2].close()
-            self._rollout = None
-        h = PolicyRollout(policy, self.action_space, self.bounds_low, self.bounds_high, self.grid_shape, src,
-                          device=int(getattr(self, "_device", os.environ.get("LOCAL_RANK", 0))))
-        self._rollout = (policy, src, h)
-        return h
+        values, policy = self.download() if live else (getattr(self, "value_function", None), self.policy)
+        if not (cached is not None and cached[1] == src
+                and (cached[0] is policy or (live and np.array_equal(cached[0], policy)))):
+            if cached is not None:
+                cached[2].close()
+                self._rollout = None
+            h = PolicyRollout(policy, self.action_space, self.bounds_low, self.bounds_high, self.grid_shape, src,
+                              device=int(getattr(self, "_device", os.environ.get("LOCAL_RANK", 0))))
+            cached = (policy, src, h, None)
+            self._rollout = cached
+        if need_values:
+            if values is None:
+                raise ValueError("no value function: the lookahead needs a live engine, or run() / load() first")
+            held = cached[3]
+            if not (held is values or (live and held is not None and np.array_equal(held.view(np.uint32),
+                                                                                     values.view(np.uint32)))):
+                cached[2].set_values(values)
+                cached = (policy, src, cached[2], values)
+                self._rollout = cached
+        return cached[2]
 
-    def rollout(self, initial_states: np.ndarray, n_steps: int, gamma: float | None = None, record: bool = False):
+    def rollout(self, initial_states: np.ndarray, n_steps: int, gamma: float | None = None, record: bool = False,
+                controller: str = "policy"):
         """Closed-loop episodes of the current policy under this plugin's own `step_dynamics` (what the reference's
         evaluate() does with get_optimal_action + an environment step, batched on the device: utils.PolicyRollout).
         `initial_states` (n, D); each episode runs `n_steps` steps or until step_dynamics sets *terminated.  Works
         after run() and after load() (host `policy`) and on a live engine (its current policy, through download()).
         `gamma=None` is the engine's gamma as float32 (`self.config.gamma`); an instance made by load() carries the
-        default CudaPIConfig(), so pass its gamma explicitly there.  Returns a utils.RolloutResult."""
+        default CudaPIConfig(), so pass its gamma explicitly there.  `controller="lookahead"` acts with the one-step
+        lookahead on this object's value function instead of the interpolated grid policy (see lookahead(); Q under
+        float32(gamma)).  Returns a utils.RolloutResult."""
+        from .utils import CONTROLLERS
+        if controller not in CONTROLLERS:
+            raise ValueError(f"controller must be one of {CONTROLLERS}, got {controller!r}")
         if gamma is None:
             gamma = float(np.float32(self.config.gamma))
-        return self._rollout_handle().run(initial_states, n_steps, gamma, record=record)
+        h = self._rollout_handle(need_values=controller == "lookahead")
+        return h.run(initial_states, n_steps, gamma, record=record, controller=controller)
+
+    def lookahead(self, states: np.ndarray, gamma: float | None = None, q: bool = False):
+        """One-step lookahead on this object's value function at `states` (n, D), not clamped or wrapped: for every
+        action, Q = r + gamma * V(x') with x', r from this plugin's `step_dynamics` and V(x') the multilinear
+        interpolation the improvement pass computes (0 when the step terminates), and the action that maximises it
+        under the improvement's rule (INTEGRATION.md §2e).  At a non-absorbing grid node this is the action
+        policy_improvement() would choose there.  V is the live engine's (through download()) or, after run() /
+        load(), the host `value_function`; `gamma=None` is float32(config.gamma).  Returns (index int32 (n,),
+        action float32 (n,)), plus Q float32 (n, A) when `q`."""
+        if gamma is None:
+            gamma = float(np.float32(self.config.gamma))
+        pts = np.ascontiguousarray(np.atleast_2d(states), dtype=np.float32)
+        if pts.ndim != 2 or pts.shape[1] != self.N_DIMS:
+            raise ValueError(f"states must have {self.N_DIMS} columns, got {pts.shape}")
+        return self._rollout_handle(need_values=True).lookahead(pts, gamma, q=q)
 
     def simulate_step(self, states: np.ndarray, actions: np.ndarray):
         """One step of this plugin's `step_dynamics` per (states[i], actions[i]) on the device ->

@@ -19,7 +19,9 @@ With `--rollout` it also runs what evaluate() runs — the policy in closed loop
 `--episodes` episodes of up to `--steps` steps from the same seeded uniform start states, simulated
 with the plugin's own float32 `step_dynamics` (the model the DP solved, not gymnasium;
 include/dpb200.h: pi_rollout_*), discounted with the runner's gamma, and prints one summary line:
-mean return, mean discounted return, mean length, fraction of episodes that terminated.
+mean return, mean discounted return, mean length, fraction of episodes that terminated.  `--rollout-controller
+lookahead` acts with the one-step lookahead on the value function instead of the interpolated grid policy
+(engine.lookahead); the summary line then names the controller.
 
 With `--warm-start-bins B` a training run first solves the same runner with the same config at `B` bins and starts
 the `--bins` solve from that value function (engine.warm_start); `--warm-start-from PATH` starts it from a saved
@@ -64,6 +66,9 @@ def build_parser(runner: str) -> argparse.ArgumentParser:
     p.add_argument("--steps", type=int, default=1000, help="Steps per episode with --rollout (else accepted for compatibility)")
     p.add_argument("--rollout", action="store_true",
                    help="Also run --episodes closed-loop episodes of --steps steps on the GPU with the plugin's dynamics")
+    p.add_argument("--rollout-controller", choices=("policy", "lookahead"), default="policy",
+                   help="What acts in --rollout episodes: the interpolated grid policy (default) or the one-step "
+                        "lookahead on the value function")
     p.add_argument("--bins", type=int, default=spec.default_bins, help=f"Bins per dimension (default: {spec.default_bins})")
     p.add_argument("--seed", type=int, default=42, help="Random seed of the queried states (default: 42)")
     p.add_argument("--no-plot", action="store_true", help="Accepted for compatibility (plots are never produced)")
@@ -136,16 +141,20 @@ def summarize(pi, n_queries: int, seed: int) -> dict:
     return out
 
 
-def rollout_summary(pi, episodes: int, steps: int, seed: int, gamma: float) -> dict:
+def rollout_summary(pi, episodes: int, steps: int, seed: int, gamma: float, controller: str = "policy") -> dict:
     """--rollout: closed-loop episodes from start_states() under the plugin's dynamics (pi.rollout)."""
-    res = pi.rollout(start_states(pi, episodes, seed), steps, gamma=gamma)
-    return {"episodes": episodes, "steps": steps, "mean_return": float(res.total_reward.mean()),
-            "mean_discounted_return": float(res.discounted_return.mean()), "mean_length": float(res.length.mean()),
-            "terminated": float(res.terminated.mean())}
+    res = pi.rollout(start_states(pi, episodes, seed), steps, gamma=gamma, controller=controller)
+    out = {"episodes": episodes, "steps": steps, "mean_return": float(res.total_reward.mean()),
+           "mean_discounted_return": float(res.discounted_return.mean()), "mean_length": float(res.length.mean()),
+           "terminated": float(res.terminated.mean())}
+    if controller != "policy":
+        out["controller"] = controller
+    return out
 
 
 def format_rollout(r: dict) -> str:
-    return (f"[=] rollout {r['episodes']} episodes x {r['steps']} steps | mean return {r['mean_return']:.6f} | "
+    who = f" ({r['controller']} controller)" if "controller" in r else ""
+    return (f"[=] rollout{who} {r['episodes']} episodes x {r['steps']} steps | mean return {r['mean_return']:.6f} | "
             f"mean discounted return {r['mean_discounted_return']:.6f} | mean length {r['mean_length']:.2f} | "
             f"terminated {r['terminated']:.4f}")
 
@@ -186,7 +195,7 @@ def main(argv: list[str] | None = None) -> int:
     if args.rollout and args.episodes > 0:
         # the runner's gamma: a loaded policy carries the default CudaPIConfig, not the one it was trained with
         gamma = float(np.float32(spec.config().gamma))
-        print(format_rollout(rollout_summary(pi, args.episodes, args.steps, args.seed, gamma)))
+        print(format_rollout(rollout_summary(pi, args.episodes, args.steps, args.seed, gamma, args.rollout_controller)))
     return 0
 
 

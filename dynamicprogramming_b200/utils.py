@@ -13,7 +13,10 @@ summation order of the float32 dot product.  There is no CPU fallback.
 
 PolicyRollout runs what the reference's evaluate() loops over on the CPU — get_optimal_action, then one environment
 step — for a batch of episodes on the device, with the plugin's own `step_dynamics` as the simulator
-(pi_rollout_create / pi_rollout_run / pi_rollout_step).
+(pi_rollout_create / pi_rollout_run / pi_rollout_step).  With a value table set (`set_values`) it also answers the
+one-step lookahead on V — Q(x, a) = r(x, a) + gamma * V(x') under the plugin's model, and the action that maximises it —
+at any batch of states, and runs episodes with that lookahead as the controller (pi_rollout_lookahead,
+pi_rollout_run_lookahead; INTEGRATION.md §2e).
 """
 from __future__ import annotations
 
@@ -89,6 +92,9 @@ class RolloutResult:
     rewards: np.ndarray | None = None   # (n, T) float32: r_t
 
 
+CONTROLLERS = ("policy", "lookahead")
+
+
 class PolicyRollout:
     """Closed-loop rollouts of a policy table under the plugin's own dynamics (include/dpb200.h: pi_rollout_*): the
     loop of the reference's evaluate() — get_optimal_action, then one environment step — for a whole batch of episodes,
@@ -100,6 +106,8 @@ class PolicyRollout:
         lib = _ffi.lib()
         grid, pol, act = _policy_table(policy, action_space, bounds_low, bounds_high, grid_shape)
         self.n_dims = grid.n_dims
+        self.n_states = pol.size
+        self.action_space = act.copy()
         handle = C.c_void_p()
         _ffi.check(lib.pi_rollout_create(C.byref(grid), _ffi.ptr(pol), _ffi.ptr(act), len(act), dynamics_src.encode(),
                                          int(device), C.byref(handle)))
@@ -111,9 +119,36 @@ class PolicyRollout:
             raise ValueError(f"states must have {self.n_dims} columns, got {pts.shape}")
         return pts
 
-    def run(self, initial_states: np.ndarray, n_steps: int, gamma: float, record: bool = False) -> RolloutResult:
+    def set_values(self, values: np.ndarray) -> None:
+        """The value table the lookahead reads: n_states float32 in reference order (a saved policy's
+        `value_function`); replaces the one set before."""
+        v = np.ascontiguousarray(values, dtype=np.float32).ravel()
+        if v.size != self.n_states:
+            raise ValueError(f"values has {v.size} entries, the grid has {self.n_states} states")
+        _ffi.check(_ffi.lib().pi_rollout_set_values(self._h, _ffi.ptr(v)))
+
+    def lookahead(self, points: np.ndarray, gamma: float, q: bool = False):
+        """One-step lookahead on the values of set_values() at `points` (n, D), not clamped or wrapped: for every action
+        a, Q[a] = fmaf(gamma, V(x'), r) with x', r from the plugin's step_dynamics (V(x') = 0 when it terminates), and the
+        improvement's winner (lowest index on ties, NaN never wins).  Returns (index int32 (n,), action float32 (n,)),
+        plus Q float32 (n, A) when `q`."""
+        x = self._states(points)
+        n = len(x)
+        idx = np.empty(n, np.int32)
+        qm = np.empty((n, len(self.action_space)), np.float32) if q else None
+        _ffi.check(_ffi.lib().pi_rollout_lookahead(self._h, _ffi.ptr(x), n, float(np.float32(gamma)), _ffi.ptr(idx),
+                                                   _ffi.ptr(qm) if q else None))
+        act = self.action_space[idx]
+        return (idx, act, qm) if q else (idx, act)
+
+    def run(self, initial_states: np.ndarray, n_steps: int, gamma: float, record: bool = False,
+            controller: str = "policy") -> RolloutResult:
         """Episodes from `initial_states` (n, D) for up to `n_steps` steps each; `record` also returns the states,
-        actions and rewards of every step."""
+        actions and rewards of every step.  `controller` chooses the action: "policy" interpolates the grid policy
+        (get_optimal_action), "lookahead" takes the lookahead's winner on the values of set_values() with Q under
+        float32(gamma)."""
+        if controller not in CONTROLLERS:
+            raise ValueError(f"controller must be one of {CONTROLLERS}, got {controller!r}")
         x0 = self._states(initial_states)
         n, D, T = len(x0), self.n_dims, int(n_steps)
         res = RolloutResult(np.empty(n, np.float64), np.empty(n, np.float64), np.empty(n, np.int32),
@@ -124,9 +159,10 @@ class PolicyRollout:
             res.actions = np.empty((n, max(T, 0)), np.float32)
             res.rewards = np.empty((n, max(T, 0)), np.float32)
             traj = [_ffi.ptr(res.states), _ffi.ptr(res.actions), _ffi.ptr(res.rewards)]
-        _ffi.check(_ffi.lib().pi_rollout_run(self._h, _ffi.ptr(x0), n, T, float(gamma), _ffi.ptr(res.total_reward),
-                                             _ffi.ptr(res.discounted_return), _ffi.ptr(res.length),
-                                             _ffi.ptr(res.terminated), _ffi.ptr(res.final_states), *traj))
+        fn = _ffi.lib().pi_rollout_run if controller == "policy" else _ffi.lib().pi_rollout_run_lookahead
+        _ffi.check(fn(self._h, _ffi.ptr(x0), n, T, float(gamma), _ffi.ptr(res.total_reward),
+                      _ffi.ptr(res.discounted_return), _ffi.ptr(res.length), _ffi.ptr(res.terminated),
+                      _ffi.ptr(res.final_states), *traj))
         res.terminated = res.terminated.astype(bool)
         return res
 

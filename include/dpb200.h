@@ -351,6 +351,30 @@ void pi_rollout_destroy(pi_rollout* r);
 /* Compile-only check of a plugin's dynamics source against the rollout kernels (NVRTC, sm_100a); needs no GPU. */
 int pi_rollout_compile_check(const char* dynamics_src, int32_t n_dims, int64_t* cubin_bytes);
 
+/* N8: one-step lookahead on a value table (csrc/lookahead_src.cuh).  For a query point x (not clamped or wrapped) and
+ * each action index a = 0..A-1:
+ *   step_dynamics(x, actions[a], &x', &r, &term);
+ *   ev = term ? 0 : the multilinear interpolation of V at x' with the table builder's cell search and the
+ *        improvement's corner order and fmaf chain (csrc/row_value_src.cuh: expected_value);
+ *   Q[a] = fmaf(gamma, ev, r)   (float32).
+ * The chosen action is the improvement's winner: ascending a, strict '>' from -1e30f, lowest index on ties, NaN never
+ * wins, action 0 when nothing beats -1e30f.  The terminal mask is not consulted.  At a non-absorbing grid node, with the
+ * values the improvement pass reads, the winner is the action pi_improve writes there.
+ *
+ * pi_rollout_set_values: the value table V, n_states float32 in reference order (a saved .npz's value_function),
+ * uploaded once and replaced by each call; every bit pattern is accepted. */
+int pi_rollout_set_values(pi_rollout* r, const float* values);
+/* Host buffers: points n x D float32; best_action n int32 and q n x n_actions float32 (row-major), either may be NULL.
+ * n == 0 is valid.  PI_ERR_INVALID for a null handle or points, n < 0, or before pi_rollout_set_values. */
+int pi_rollout_lookahead(pi_rollout* r, const float* points, int64_t n, float gamma, int32_t* best_action, float* q);
+/* pi_rollout_run with the lookahead as the controller: a_t = actions[winner at x_t] with Q under (float)gamma; the
+ * step, the returns (discounted with gamma), the buffers and the error rules are those of pi_rollout_run, and it is
+ * PI_ERR_INVALID before pi_rollout_set_values. */
+int pi_rollout_run_lookahead(pi_rollout* r, const float* initial_states, int64_t n_episodes, int32_t n_steps,
+                             double gamma, double* total_reward, double* discounted_return, int32_t* length,
+                             uint8_t* terminated, float* final_states, float* traj_states, float* traj_actions,
+                             float* traj_rewards);
+
 #ifdef __cplusplus
 }
 #endif
