@@ -533,223 +533,6 @@ __global__ void __launch_bounds__(kPBlock) eval_persistent_kernel(const PersistP
     }
 }
 
-// ---------------------------------------------------------------------------
-// Evaluation sweep, TWO consecutive states per thread along the fastest-stored
-// dimension (logical dimension F, istride[F] == 1).
-//
-// When the two states' successor cells are neighbours along F (base_1 == base_0 + 1
-// — the common case once the layout probe has put a well-behaved dimension
-// fastest), the 2^D corners of both states live in 2^(D-1) three-element windows
-// V[a], V[a+1], V[a+2]: state 0 uses (a, a+1), state 1 uses (a+1, a+2).  Each window
-// is fetched with two aligned 64-bit loads, so the pair needs 2^D 64-bit requests
-// instead of 2*2^D 32-bit ones, and the L1 data-pipe wavefronts (the binding unit
-// of the scalar kernel, see DESIGN.md §5) drop by almost 2x.  Rows of the two
-// states are one 256-bit load per 16-byte plane.  The fma chain of each state is
-// still evaluated in ascending corner order with individually rounded weights, so
-// the result is bit-identical to eval_sweep_kernel.  Any other pair (sentinel rows,
-// clamped / non-adjacent successors) takes the scalar path.
-// ---------------------------------------------------------------------------
-__device__ __forceinline__ void ld_stream32(const void* p, unsigned (&r)[8]) {
-    asm volatile("ld.global.nc.L1::no_allocate.v8.u32 {%0,%1,%2,%3,%4,%5,%6,%7}, [%8];"
-                 : "=r"(r[0]), "=r"(r[1]), "=r"(r[2]), "=r"(r[3]), "=r"(r[4]), "=r"(r[5]), "=r"(r[6]), "=r"(r[7])
-                 : "l"(p));
-}
-
-// rows of local states s0 (even) and s0 + 1
-template <int D>
-__device__ __forceinline__ void load_row2(const unsigned char* __restrict__ tab, long long n_pad, long long s0,
-                                          unsigned (&w0)[Row<D>::W], unsigned (&w1)[Row<D>::W]) {
-    using R = Row<D>;
-#pragma unroll
-    for (int p = 0; p < R::N4; ++p) {
-        unsigned r[8];
-        ld_stream32(tab + (size_t)p * 16u * (size_t)n_pad + (size_t)s0 * 16u, r);
-#pragma unroll
-        for (int k = 0; k < 4; ++k) { w0[4 * p + k] = r[k]; w1[4 * p + k] = r[4 + k]; }
-    }
-    if constexpr (R::N2 != 0) {
-        uint4 v = ld_stream16(tab + (size_t)R::N4 * 16u * (size_t)n_pad + (size_t)s0 * 8u);
-        w0[4 * R::N4] = v.x; w0[4 * R::N4 + 1] = v.y; w1[4 * R::N4] = v.z; w1[4 * R::N4 + 1] = v.w;
-    }
-    if constexpr (R::N1 != 0) {
-        uint2 v = ld_stream8(tab + ((size_t)R::N4 * 16u + (size_t)R::N2 * 8u) * (size_t)n_pad + (size_t)s0 * 4u);
-        w0[R::W - 1] = v.x; w1[R::W - 1] = v.y;
-    }
-}
-
-// bit position of logical dimension d inside a corner number (see corner_bit)
-template <int D>
-__host__ __device__ constexpr int corner_pos(int d) { return D == 2 ? 1 - d : d; }
-
-// prefix products over dims 0..D-2 (2^(D-1) values), reference multiplication order
-template <int D>
-__device__ __forceinline__ void prefix_weights(const float (&frac)[D], float (&pre)[(1 << D) / 2]) {
-    if constexpr (D >= 3) {
-        pre[0] = 1.0f - frac[0];
-        pre[1] = frac[0];
-#pragma unroll
-        for (int d = 1; d < D - 1; ++d) {
-            const float g = 1.0f - frac[d];
-#pragma unroll
-            for (int c = (1 << d) - 1; c >= 0; --c) {
-                const float q = pre[c];
-                pre[c + (1 << d)] = q * frac[d];
-                pre[c] = q * g;
-            }
-        }
-    } else {
-        pre[0] = 0.0f;  // unused for D <= 2
-    }
-}
-template <int D>
-__device__ __forceinline__ float corner_weight(const float (&frac)[D], const float (&pre)[(1 << D) / 2], int c) {
-    if constexpr (D == 1) {
-        return c ? frac[0] : 1.0f - frac[0];
-    } else if constexpr (D == 2) {
-        const float a = corner_bit<2>(c, 0) ? frac[0] : 1.0f - frac[0];
-        const float b = corner_bit<2>(c, 1) ? frac[1] : 1.0f - frac[1];
-        return a * b;
-    } else {
-        constexpr int H = (1 << D) / 2;
-        return pre[c & (H - 1)] * ((c & H) ? frac[D - 1] : 1.0f - frac[D - 1]);
-    }
-}
-
-template <int D, int F>
-__global__ void __launch_bounds__(kBlock) eval_sweep_pair_kernel(const EvalParams p) {
-    constexpr int W = Row<D>::W;
-    constexpr int C = 1 << D;
-    constexpr int P = corner_pos<D>(F);     // bit position of the fast dimension in a corner number
-    constexpr int NLO = 1 << P;             // row-combos below the fast bit
-    constexpr int NHI = C >> (P + 1);       // row-combos above it
-    const Ctl* __restrict__ ctl = p.ctl;
-    if (ctl->done) return;
-    const int par = (ctl->base + p.j + ctl->parity0) & 1;
-    const float* __restrict__ Vin = par ? p.V1 : p.V0;
-    float* __restrict__ Vout = par ? p.V0 : p.V1;
-
-    const long long s0 = 2 * ((long long)blockIdx.x * kBlock + threadIdx.x);
-    float res = 0.0f;
-    if (s0 < p.n_local) {
-        const bool has1 = s0 + 1 < p.n_local;
-        unsigned w0[W], w1[W];
-        load_row2<D>(p.rows, p.n_pad, s0, w0, w1);
-        const int b0 = (int)w0[0], b1 = (int)w1[0];
-        const long long g0 = p.s_begin + s0;
-        float vold0, vold1 = 0.0f;
-        if ((g0 & 1) == 0) {
-            const float2 t = *reinterpret_cast<const float2*>(Vin + g0);  // V buffers are padded, s0+1 is readable
-            vold0 = t.x; vold1 = t.y;
-        } else {
-            vold0 = Vin[g0];
-            if (has1) vold1 = Vin[g0 + 1];
-        }
-        float vnew0, vnew1 = 0.0f;
-        int stride[D];
-#pragma unroll
-        for (int d = 0; d < D; ++d) stride[d] = p.stride[d];
-
-        // Effective bases: a sentinel row (terminated / absorbing / padding) borrows its partner's
-        // cell so that its (discarded) loads stay in range; delta = distance between the two
-        // successor cells along the fast dimension.  delta == 1: neighbours; delta == 0: same cell
-        // (clamped at a grid edge, or one row is a sentinel).  Anything else -> scalar path.
-        const bool sen0 = b0 < 0, sen1 = !has1 || b1 < 0;
-        const int e0 = sen0 ? (sen1 ? 0 : b1) : b0;
-        const int e1 = sen1 ? e0 : b1;
-        const int delta = e1 - e0;
-        if (delta == 0 || delta == 1) {
-            float f0[D], f1[D];
-#pragma unroll
-            for (int d = 0; d < D; ++d) { f0[d] = __uint_as_float(w0[1 + d]); f1[d] = __uint_as_float(w1[1 + d]); }
-            float pre0[C / 2], pre1[C / 2];
-            prefix_weights<D>(f0, pre0);
-            prefix_weights<D>(f1, pre1);
-            float ev0 = 0.0f, ev1 = 0.0f;
-#pragma unroll
-            for (int hi = 0; hi < NHI; ++hi) {
-                float x[NLO][3];
-#pragma unroll
-                for (int lo = 0; lo < NLO; ++lo) {
-                    const int c = (hi << (P + 1)) | lo;  // corner with the fast bit clear
-                    int off = 0;
-#pragma unroll
-                    for (int d = 0; d < D; ++d)
-                        if (d != F && corner_bit<D>(c, d)) off += stride[d];
-                    const int a = e0 + off;
-                    const float2* q = reinterpret_cast<const float2*>(Vin + (a & ~1));
-                    const float2 r01 = q[0], r23 = q[1];
-                    const bool odd = a & 1;
-                    x[lo][0] = odd ? r01.y : r01.x;
-                    x[lo][1] = odd ? r23.x : r01.y;
-                    x[lo][2] = odd ? r23.y : r23.x;
-                }
-#pragma unroll
-                for (int fb = 0; fb < 2; ++fb) {
-#pragma unroll
-                    for (int lo = 0; lo < NLO; ++lo) {
-                        const int c = (hi << (P + 1)) | (fb << P) | lo;
-                        ev0 = fmaf(corner_weight<D>(f0, pre0, c), x[lo][fb], ev0);
-                        ev1 = fmaf(corner_weight<D>(f1, pre1, c), delta ? x[lo][fb + 1] : x[lo][fb], ev1);
-                    }
-                }
-            }
-            // sentinel rows: terminated -> sum := 0 (:231-232); absorbing -> new_V := V (:221)
-            vnew0 = b0 == PI_ROW_ABSORBING ? vold0 : fmaf(p.gamma, sen0 ? 0.0f : ev0, __uint_as_float(w0[D + 1]));
-            vnew1 = b1 == PI_ROW_ABSORBING ? vold1 : fmaf(p.gamma, sen1 ? 0.0f : ev1, __uint_as_float(w1[D + 1]));
-        } else {
-            // scalar path, one state at a time (identical to eval_sweep_kernel)
-            if (b0 == PI_ROW_ABSORBING) {
-                vnew0 = vold0;
-            } else {
-                float ev = 0.0f;
-                if (b0 >= 0) {
-                    float fr[D];
-#pragma unroll
-                    for (int d = 0; d < D; ++d) fr[d] = __uint_as_float(w0[1 + d]);
-                    ev = expected_value<D>(Vin, b0, fr, stride);
-                }
-                vnew0 = fmaf(p.gamma, ev, __uint_as_float(w0[D + 1]));
-            }
-            if (has1) {
-                if (b1 == PI_ROW_ABSORBING) {
-                    vnew1 = vold1;
-                } else {
-                    float ev = 0.0f;
-                    if (b1 >= 0) {
-                        float fr[D];
-#pragma unroll
-                        for (int d = 0; d < D; ++d) fr[d] = __uint_as_float(w1[1 + d]);
-                        ev = expected_value<D>(Vin, b1, fr, stride);
-                    }
-                    vnew1 = fmaf(p.gamma, ev, __uint_as_float(w1[D + 1]));
-                }
-            }
-        }
-        if ((g0 & 1) == 0 && has1) {
-            *reinterpret_cast<float2*>(Vout + g0) = make_float2(vnew0, vnew1);
-        } else {
-            Vout[g0] = vnew0;
-            if (has1) Vout[g0 + 1] = vnew1;
-        }
-        if (p.peers.n) {
-            store_peers(p.peers, par != 0, g0, vnew0);
-            if (has1) store_peers(p.peers, par != 0, g0 + 1, vnew1);
-        }
-        res = fabsf(vnew0 - vold0);
-        if (has1) res = fmaxf(res, fabsf(vnew1 - vold1));
-    }
-    if (!p.check) return;
-    __shared__ float s_red[kBlock / 32];
-    res = warp_max(res);
-    if ((threadIdx.x & 31) == 0) s_red[threadIdx.x >> 5] = res;
-    __syncthreads();
-    if (threadIdx.x < 32) {
-        float r = threadIdx.x < kBlock / 32 ? s_red[threadIdx.x] : 0.0f;
-        r = warp_max(r);
-        if (threadIdx.x == 0) p.partial[blockIdx.x] = r;
-    }
-}
-
 // End of a batch of k sweeps: advance the sweep counter; if the last sweep was a
 // check sweep, reduce the per-block residuals; if `decide`, apply the sync-point
 // test of policy_evaluation (:325-331).  When sharded the residual is all-reduced

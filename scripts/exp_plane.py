@@ -26,7 +26,7 @@ d, ms = eng.sweeps(25)
 print("engine sweeps: %.4f ms/sweep" % (ms / 25), flush=True)
 out = []
 for cfg in cfgs:
-    # "cfg@K=V,K=V": environment knobs read when the sweep is compiled (e.g. DPB200_PLANE_ROWPF)
+    # "cfg@K=V;K=V": environment variables set while this configuration is compiled and timed
     spec, _, envs_ = cfg.partition("@")
     for kv in filter(None, envs_.split(";")):
         k, _, v = kv.partition("=")

@@ -3,7 +3,7 @@
 (scripts/data/k5_policy16.npz, captured by scripts/k5_policies.py; falls back to the bench policy).
 Every variant must produce the same V bits.
 
-    python scripts/exp_variants.py "DPB200_EVAL_VARIANT=0" "DPB200_EVAL_VARIANT=1" "DPB200_EVAL_VARIANT=1 DPB200_LOOKAHEAD=0" ...
+    python scripts/exp_variants.py "DPB200_EVAL_VARIANT=0" "DPB200_EVAL_VARIANT=1" "DPB200_EVAL_VARIANT=64" ...
 """
 import hashlib, os, sys, time
 from pathlib import Path
